@@ -2,6 +2,7 @@
 """bench.py -- headline measurement of the zipc hot path on B200 (contract: DESIGN.md "Measurement").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload deflate|inflate|crc32] [--level L] [--impl reference]
+                  [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one batch of synthetic input (SURVEY.md 8d):
   deflate (default; BASELINE.json configs[3], the first item of its metric): batch deflate + CRC-32 of 10,000
@@ -16,6 +17,13 @@ independent units, no data-path collective); rank 0 prints the aggregate.  "also
 workloads and levels (fewer steps), the compression ratio against the reference's (`ratio_vs_ref`), and for N > 1 a
 STRONG-scaling leg: ONE member set / ONE buffer driven over all N GPUs through the library's box-wide entry points
 (zipc_b200_multi_*), results gathered to the host and CRCs combined inside the timed region.
+
+--dump-outputs DIR writes what the headline call handed back in its last timed step as DIR/<name>.npy (float64 for
+statuses, sizes and CRC-32s, float32 for bytes; rank 0 only).  Inputs are seeded, so two builds run with the same
+arguments can be compared output for output:
+  deflate / inflate: status, crc32, compressed_size / decompressed_size of every member, and the output bytes of a fixed
+                     seeded sample of members (sample_members, sample_compressed_bytes / sample_decompressed_bytes)
+  crc32:             crc32 of the buffer
 
 --impl reference times the reference's algorithm on the host cores.  The reference is OCaml and this image has no
 OCaml toolchain, so it is the C restatement in oracle/ ("port").  That arm never loads libzipc_b200.so.
@@ -223,6 +231,28 @@ class Harness:
 
 P = lambda a, t: a.ctypes.data_as(C.POINTER(t))
 
+DUMP_LIMIT = 64 << 20
+DUMP_MEMBERS = 48   # members whose bytes --dump-outputs writes: 48 x (256 KiB + deflate overhead) as float32 < 51 MB
+
+
+def member_outputs(size_name, bytes_name, dbuf, offs, lens, ck, st):
+    """What a batch call hands back: status, CRC-32 and output size of every member, and the output bytes of a fixed
+    seeded sample of members, as float64 / float32 (exact: sizes < 2**53, CRC-32 < 2**32, bytes < 2**8)."""
+    pick = np.sort(np.random.default_rng(0).choice(len(lens), min(len(lens), DUMP_MEMBERS), replace=False))
+    sample = [dbuf[int(offs[i]):int(offs[i]) + int(lens[i])].cpu().numpy() for i in pick]
+    return {"status": st.astype(np.float64), "crc32": ck.astype(np.float64), size_name: lens.astype(np.float64),
+            "sample_members": pick.astype(np.float64),
+            bytes_name: np.concatenate(sample).astype(np.float32) if sample else np.zeros(0, dtype=np.float32)}
+
+
+def write_outputs(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes, more than {DUMP_LIMIT >> 20} MB (use fewer --members)")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
 
 def _pack_device(h: Harness, items, pin=True):
     """concatenate (16-byte aligned) into one (pinned) host buffer + device copy; returns offsets"""
@@ -242,7 +272,7 @@ def _pack_device(h: Harness, items, pin=True):
 # ---------------------------------------------------------------------------------------------------
 # workloads (GPU arm)
 # ---------------------------------------------------------------------------------------------------
-def run_crc32(h: Harness, steps, warmup, rank, adler=True):
+def run_crc32(h: Harness, steps, warmup, rank, adler=True, dump=False):
     from zipc_b200 import synth
     n = GiB
     host = h.pinned(synth.rand_v1(2 + rank, n), keep=True)  # also the strong-scaling leg's buffer
@@ -253,6 +283,7 @@ def run_crc32(h: Harness, steps, warmup, rank, adler=True):
     total_ms = h.timed(fn, steps, warmup)
     launches = (h.ctx.launches - l0) // (steps + warmup) * steps
     got = int(dcrc[0].item()) & 0xFFFFFFFF
+    outputs = {"crc32": np.array([got], dtype=np.float64)} if dump else None
     kms = h.kernel_ms(fn, min(steps, 10))
     out = C.c_uint32()
     e2e_fn = lambda: h.L.zipc_b200_crc32(h.ctx.h, host.ctypes.data, n, C.byref(out))
@@ -280,10 +311,10 @@ def run_crc32(h: Harness, steps, warmup, rank, adler=True):
                         "roofline_frac_per_call": round(n / dt / 1e9 / measured_peak_gbs()[0], 4), "chunk_kernel_ms": round(akms, 4) if akms else None}
         assert int(ad["rfc1950"]["value"], 16) == zlib.adler32(host), ad
     return dict(units=n, total_ms=total_ms, steps=steps, launches=launches, kernel_ms=kms, algo_bytes=n, e2e_s=e2e_s,
-                h2d=n, d2h=4, host=host, kernel="crc32_tiles_kernel", extra={"crc32": "%08x" % got, "adler32": ad})
+                h2d=n, d2h=4, host=host, kernel="crc32_tiles_kernel", extra={"crc32": "%08x" % got, "adler32": ad}, outputs=outputs)
 
 
-def run_deflate(h: Harness, datas, level, steps, warmup, e2e=True, keep_streams=False):
+def run_deflate(h: Harness, datas, level, steps, warmup, e2e=True, keep_streams=False, dump=False):
     from zipc_b200 import _lib
     lvl = LEVELS[level]
     n = len(datas)
@@ -303,6 +334,7 @@ def run_deflate(h: Harness, datas, level, steps, warmup, e2e=True, keep_streams=
     total_ms = h.timed(fn, steps, warmup)
     launches = (h.ctx.launches - l0) // (steps + warmup) * steps
     assert (st == 0).all(), "deflate status"
+    outputs = member_outputs("compressed_size", "sample_compressed_bytes", ddst, doff, dl, ck, st) if dump else None
     Cb = int(dl.sum())
     sizes = dl.copy()
     # parity spot check inside the bench: CRC-32 of the input and a zlib round trip of a sample straight from the device
@@ -312,7 +344,7 @@ def run_deflate(h: Harness, datas, level, steps, warmup, e2e=True, keep_streams=
         assert zlib.decompress(cs, -15) == datas[i].tobytes(), "round trip lost in bench"
     kms = h.kernel_ms(fn, min(steps, 3))
     r = dict(units=U, total_ms=total_ms, steps=steps, launches=launches, kernel_ms=kms, algo_bytes=U + Cb, kernel="deflate_kernel",
-             sizes=sizes, h2d=U, d2h=Cb, e2e_s=None,
+             sizes=sizes, h2d=U, d2h=Cb, e2e_s=None, outputs=outputs,
              extra={"uncompressed_bytes": U, "compressed_bytes": Cb, "ratio": round(Cb / U, 4)})
     if e2e:
         e_ptrs = (C.c_void_p * n)(*[hsrc.ctypes.data + int(o) for o in soff])
@@ -334,7 +366,7 @@ def run_deflate(h: Harness, datas, level, steps, warmup, e2e=True, keep_streams=
     return r
 
 
-def run_inflate(h: Harness, datas, streams, steps, warmup, e2e=True):
+def run_inflate(h: Harness, datas, streams, steps, warmup, e2e=True, dump=False):
     n = len(datas)
     U = int(sum(d.size for d in datas)); Cb = int(sum(len(s) for s in streams))
     hcs, dcs, coff, clen = _pack_device(h, streams)
@@ -352,13 +384,14 @@ def run_inflate(h: Harness, datas, streams, steps, warmup, e2e=True):
     total_ms = h.timed(fn, steps, warmup)
     launches = (h.ctx.launches - l0) // (steps + warmup) * steps
     assert (st == 0).all() and (dl == slen).all(), "inflate status"
+    outputs = member_outputs("decompressed_size", "sample_decompressed_bytes", ddst, soff, dl, ck, st) if dump else None
     for i in list(range(0, n, max(1, n // 200)))[:200]:
         assert int(ck[i]) == zlib.crc32(datas[i]), "crc parity lost in bench"
     i = n // 3
     assert ddst[int(soff[i]):int(soff[i]) + int(slen[i])].cpu().numpy().tobytes() == datas[i].tobytes()
     kms = h.kernel_ms(fn, min(steps, 3))
     r = dict(units=U, total_ms=total_ms, steps=steps, launches=launches, kernel_ms=kms, algo_bytes=U + Cb, kernel="inflate_kernel<false>",
-             h2d=Cb, d2h=U, e2e_s=None, extra={"uncompressed_bytes": U, "compressed_bytes": Cb, "ratio": round(Cb / U, 4)})
+             h2d=Cb, d2h=U, e2e_s=None, outputs=outputs, extra={"uncompressed_bytes": U, "compressed_bytes": Cb, "ratio": round(Cb / U, 4)})
     if e2e:  # compressed members inside one pinned host buffer (an in-memory archive), pinned output arena
         e_ptrs = (C.c_void_p * n)(*[hcs.ctypes.data + int(o) for o in coff])
         e_arena = h.pinned(np.zeros(int(((slen + np.uint64(15)) & ~np.uint64(15)).sum()) + 64, dtype=np.uint8))
@@ -848,9 +881,14 @@ def main():
     ap.add_argument("--no-also", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--members", type=int, default=10000)
     ap.add_argument("--level", choices=["fast", "default", "best"], default="default", help="deflate level of the codec workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the headline call returned in its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.workload == "crc32" else 5
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path: it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return reference_arm(args)
@@ -929,17 +967,21 @@ def main():
         return streams
 
     # ---- headline ---------------------------------------------------------------------------------------------------
+    dump = bool(args.dump_outputs) and rank == 0
     if which == "deflate":
-        r = measured(lambda: run_deflate(h, datas, args.level, args.steps, args.warmup, keep_streams=True))
+        r = measured(lambda: run_deflate(h, datas, args.level, args.steps, args.warmup, keep_streams=True, dump=dump))
         streams = r.pop("streams", None)
         single_e2e["deflate"] = r["e2e_s"]
     elif which == "inflate":
         get_streams()
-        r = measured(lambda: run_inflate(h, datas, streams, args.steps, args.warmup))
+        r = measured(lambda: run_inflate(h, datas, streams, args.steps, args.warmup, dump=dump))
         single_e2e["inflate"] = r["e2e_s"]
     else:
-        r = measured(lambda: run_crc32(h, args.steps, args.warmup, rank))
+        r = measured(lambda: run_crc32(h, args.steps, args.warmup, rank, dump=dump))
         single_e2e["crc32"] = r["e2e_s"]
+    outputs = r.pop("outputs")
+    if dump:
+        write_outputs(args.dump_outputs, outputs)
     line = {"metric": METRIC[which], "value": round(r["value"], 2), "unit": "GB/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": round(r["ms_per_step"], 4), "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic",

@@ -1,24 +1,22 @@
-"""Regenerates tests/golden/* from the read-only reference checkout.
+"""Regenerates tests/golden/* from a checkout of the reference (zipc):
+    python tests/golden/make_golden.py <zipc checkout>/test/test.ml
 
-Run in the build container only (/root/reference does not exist on the GPU box):
-    python tests/golden/make_golden.py
-
-zip-docs.zip is the fixture embedded as an OCaml string literal in
-/root/reference/test/test.ml:131-3294 (Info-ZIP made; 1 dir + 2 deflate members).  The literal
+zip-docs.zip is the fixture embedded as an OCaml string literal in the reference's
+test/test.ml:131-3294 (Info-ZIP made; 1 dir + 2 deflate members).  The literal
 consists only of \\xHH escapes and line continuations; it is decoded here and its fingerprint
 checked against SURVEY.md section 8c (56,924 bytes, CRC-32 0a88d91b, md5 d2076f2e...).
 """
 import hashlib
 import os
 import re
+import sys
 import zlib
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_TEST = "/root/reference/test/test.ml"
 
 
-def extract_fixture() -> bytes:
-    src = open(REF_TEST, "rb").read().decode("latin-1")
+def extract_fixture(ref_test: str) -> bytes:
+    src = open(ref_test, "rb").read().decode("latin-1")
     start = src.index("zip_docs_zip :=")
     lit_start = src.index('"', start) + 1
     lit_end = src.index('"', lit_start)
@@ -29,7 +27,9 @@ def extract_fixture() -> bytes:
 
 
 def main():
-    data = extract_fixture()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    data = extract_fixture(sys.argv[1])
     assert len(data) == 56924, len(data)
     assert zlib.crc32(data) == 0x0A88D91B, hex(zlib.crc32(data))
     assert hashlib.md5(data).hexdigest() == "d2076f2e591c1af277938f79485fe0d7"
