@@ -159,7 +159,11 @@ void zipc_b200_inflate_plan(size_t n, const size_t *src_len, size_t lanes, char 
 int zipc_b200_fetch(zipc_b200_ctx *ctx, void *dst, size_t dst_cap);
 /* Device-resident form: streams live in one device buffer d_src at src_off[i]; outputs are
  * written to d_dst at dst_off[i] (given by the caller, capacity max_out[i] each, which must be
- * known).  Per-stream results are copied back to the host arrays. */
+ * known: ZIPC_SIZE_UNKNOWN is ZIPC_ERR_INVALID_ARG).  Per-stream results are copied back to the host arrays.
+ * src_off and dst_off need no alignment.  Stream i is read from [src_off[i], src_off[i] + src_len[i]) only: the bytes
+ * after it, whatever they are, never change its result.  Output i is written inside [dst_off[i], dst_off[i] + dst_len[i])
+ * on success and inside [dst_off[i], dst_off[i] + max_out[i]) otherwise, never outside, so slots may sit back to back.
+ * The device bytes may change between calls (each call reads them afresh). */
 int zipc_b200_inflate_batch_dev(zipc_b200_ctx *ctx, int checksum_kind, int adler_mode, size_t n,
                                 const void *d_src, const size_t *src_off, const size_t *src_len,
                                 void *d_dst, const size_t *dst_off, const size_t *max_out,
@@ -188,6 +192,13 @@ int zipc_b200_deflate_batch(zipc_b200_ctx *ctx, int level, int checksum_kind, in
                             size_t n, const void *const *src, const size_t *src_len,
                             void *dst, size_t dst_cap, size_t *dst_need,
                             size_t *dst_off, size_t *dst_len, uint32_t *checksum, int *status);
+/* Device-resident form: input i is [src_off[i], src_off[i] + src_len[i]) of d_src (any alignment; the bytes around it are
+ * never read into the result), output i goes to the caller's slot at dst_off[i] of d_dst, which must be 4-byte aligned
+ * (ZIPC_ERR_INVALID_ARG otherwise, before anything runs), with capacity dst_cap_each[i] (zipc_b200_deflate_bound(src_len[i])
+ * always suffices).  A member is compressed by one CTA whatever its size (no primed segments).  On success exactly
+ * [dst_off[i], dst_off[i] + dst_len[i]) is written; bytes of the slot after dst_len[i] keep their contents.  A slot that is
+ * too small gives status[i] = ZIPC_ERR_DST_TOO_SMALL and dst_len[i] = 0, and only bytes inside
+ * [dst_off[i], dst_off[i] + dst_cap_each[i]) may have been written; the other members are not affected. */
 int zipc_b200_deflate_batch_dev(zipc_b200_ctx *ctx, int level, int checksum_kind, int adler_mode,
                                 size_t n, const void *d_src, const size_t *src_off,
                                 const size_t *src_len, void *d_dst, const size_t *dst_off,
