@@ -379,7 +379,7 @@ int adler32_launch_buffer(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len
   // the result is one word: the last thread of the fold / reduction stores it straight into mapped host memory (a posted write
   // over PCIe) -- no copy operation, and no staging of a 4-byte copy into the caller's pageable word -- and the host reads it
   // once the stream is through
-  if (!ctx->h_word) ZB_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_word), 64, cudaHostAllocMapped));
+  if (int st = map_host_word(ctx)) return st;
   uint32_t *d_out = ctx->h_word;
   if (mode == ZIPC_ADLER_RFC1950) {
     // exact arithmetic: an ordered reduction over all SMs' worth of threads

@@ -36,6 +36,17 @@ cudaError_t stream_sync(zipc_b200_ctx *ctx, cudaStream_t s) {
   return cudaEventSynchronize(ctx->ev_block);
 }
 
+int map_host_word(zipc_b200_ctx *ctx) {
+  if (!ctx->h_word) ZB_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_word), 64, cudaHostAllocMapped));
+  return ZIPC_OK;
+}
+
+int crc32_to_host_word(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len) {
+  if (int st = map_host_word(ctx)) return st;
+  return crc32_launch_buffer(ctx, d_src, len, ctx->h_word + 1);
+}
+uint32_t host_word_crc32(const zipc_b200_ctx *ctx) { return reinterpret_cast<const volatile uint32_t *>(ctx->h_word)[1]; }
+
 int DevBuf::reserve(size_t bytes) {
   if (bytes <= cap) return ZIPC_OK;
   if (p) { cudaFree(p); p = nullptr; cap = 0; }
@@ -65,77 +76,99 @@ static bool is_pinned(const void *p) {
   return a.type == cudaMemoryTypeHost;
 }
 
-static constexpr size_t kStageChunk = 16u << 20;
+// A copy of pinned host memory, or of no more than 64 KiB, is one DMA; anything else goes through the staging ring.
+static bool copy_direct(const void *h, size_t bytes) { return bytes <= (1u << 16) || is_pinned(h); }
 
-// host -> device.  Pinned sources are DMA'd directly; pageable ones go through a double-buffered
-// pinned staging ring so that the CPU copy of chunk k+1 overlaps the DMA of chunk k.
-int h2d(zipc_b200_ctx *ctx, void *d, const void *h, size_t bytes) {
-  if (!bytes) return ZIPC_OK;
-  if (is_pinned(h)) {
-    ZB_CUDA(ctx, cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+// Staging of pageable host memory: two pinned buffers of kStageChunk bytes (ctx->h_stage), used in turn, so that the CPU
+// copy into or out of one overlaps the DMA of the other.  The last DMA of buffer i is behind ctx->ev_stage[i]; after a
+// download its bytes still have to go on to the host address `to[i]`.  A ring is drained when it goes out of scope, so no
+// DMA into or out of the staging buffers outlives the call, whichever way it returns.
+static constexpr size_t kStageChunk = 16u << 20;
+class StageRing {
+  zipc_b200_ctx *c;
+  int k = 0;  // the buffer to use next
+  bool busy[2] = {false, false};
+  uint8_t *to[2] = {nullptr, nullptr};
+  size_t to_len[2] = {0, 0};
+  uint8_t *buf(int i) const { return c->h_stage.as<uint8_t>() + (size_t)i * kStageChunk; }
+  int wait(int i) {
+    if (!busy[i]) return ZIPC_OK;
+    busy[i] = false;
+    ZB_CUDA(c, cudaEventSynchronize(c->ev_stage[i]));
+    if (to_len[i]) std::memcpy(to[i], buf(i), to_len[i]);
+    to_len[i] = 0;
     return ZIPC_OK;
   }
-  if (bytes <= (1u << 16)) {
-    ZB_CUDA(ctx, cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    return ZIPC_OK;
-  }
-  if (int st = ctx->h_stage.reserve(2 * kStageChunk)) return st;
-  cudaEvent_t ev[2];
-  ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming));
-  ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming));
-  size_t off = 0;
-  int k = 0;
-  bool used[2] = {false, false};
-  int rc = ZIPC_OK;
-  while (off < bytes) {
-    size_t m = std::min(kStageChunk, bytes - off);
-    uint8_t *s = ctx->h_stage.as<uint8_t>() + (size_t)k * kStageChunk;
-    if (used[k]) cudaEventSynchronize(ev[k]);
-    std::memcpy(s, static_cast<const uint8_t *>(h) + off, m);
-    cudaError_t e = cudaMemcpyAsync(static_cast<uint8_t *>(d) + off, s, m, cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { rc = set_cuda_error(ctx, e, "h2d staging"); break; }
-    cudaEventRecord(ev[k], ctx->stream);
-    used[k] = true;
-    off += m;
+  int dma(void *dst, const void *src, size_t bytes, cudaMemcpyKind kind) {
+    ZB_CUDA(c, cudaMemcpyAsync(dst, src, bytes, kind, c->stream));
+    busy[k] = true;
+    ZB_CUDA(c, cudaEventRecord(c->ev_stage[k], c->stream));
     k ^= 1;
+    return ZIPC_OK;
   }
-  for (int i = 0; i < 2; i++) { if (used[i]) cudaEventSynchronize(ev[i]); cudaEventDestroy(ev[i]); }
-  return rc;
+
+ public:
+  explicit StageRing(zipc_b200_ctx *ctx) : c(ctx) {}
+  ~StageRing() { drain(); }
+  int open() {
+    if (int st = c->h_stage.reserve(2 * kStageChunk)) return st;
+    for (cudaEvent_t &e : c->ev_stage)
+      if (!e) ZB_CUDA(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    return ZIPC_OK;
+  }
+  // the next buffer, once its last DMA is through
+  int next(uint8_t **b) {
+    if (int st = wait(k)) return st;
+    *b = buf(k);
+    return ZIPC_OK;
+  }
+  // DMA of the first `bytes` of that buffer to device address d
+  int upload(void *d, size_t bytes) { return dma(d, buf(k), bytes, cudaMemcpyHostToDevice); }
+  // DMA of `bytes` from device address d into the next buffer; they reach host address h once it is needed again
+  int download(void *h, const void *d, size_t bytes) {
+    if (int st = wait(k)) return st;
+    to[k] = static_cast<uint8_t *>(h);
+    to_len[k] = bytes;
+    return dma(buf(k), d, bytes, cudaMemcpyDeviceToHost);
+  }
+  // waits for both buffers, the older first
+  int drain() {
+    const int a = wait(k), b = wait(k ^ 1);
+    return a ? a : b;
+  }
+};
+
+// host -> device, enqueued on the context's stream (a pageable source has been read when this returns)
+int h2d(zipc_b200_ctx *ctx, void *d, const void *h, size_t bytes) {
+  if (copy_direct(h, bytes)) {
+    if (bytes) ZB_CUDA(ctx, cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    return ZIPC_OK;
+  }
+  StageRing ring(ctx);
+  if (int st = ring.open()) return st;
+  for (size_t off = 0; off < bytes; off += kStageChunk) {
+    const size_t m = std::min(kStageChunk, bytes - off);
+    uint8_t *s;
+    if (int st = ring.next(&s)) return st;
+    std::memcpy(s, static_cast<const uint8_t *>(h) + off, m);
+    if (int st = ring.upload(static_cast<uint8_t *>(d) + off, m)) return st;
+  }
+  return ring.drain();
 }
 
-// device -> host, same idea in the other direction.  Synchronous on return.
+// device -> host.  Synchronous on return: the context's stream is through.
 int d2h(zipc_b200_ctx *ctx, void *h, const void *d, size_t bytes) {
-  if (!bytes) return ZIPC_OK;
-  if (is_pinned(h) || bytes <= (1u << 16)) {
-    ZB_CUDA(ctx, cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (copy_direct(h, bytes)) {
+    if (bytes) ZB_CUDA(ctx, cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
     return ZIPC_OK;
   }
-  if (int st = ctx->h_stage.reserve(2 * kStageChunk)) return st;
-  cudaEvent_t ev[2];
-  ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming));
-  ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming));
-  size_t off = 0, pend_off[2] = {0, 0}, pend_len[2] = {0, 0};
-  int k = 0, rc = ZIPC_OK;
-  while (off < bytes || pend_len[0] || pend_len[1]) {
-    if (pend_len[k]) {  // drain the buffer we are about to reuse
-      cudaEventSynchronize(ev[k]);
-      std::memcpy(static_cast<uint8_t *>(h) + pend_off[k], ctx->h_stage.as<uint8_t>() + (size_t)k * kStageChunk, pend_len[k]);
-      pend_len[k] = 0;
-    }
-    if (off < bytes) {
-      size_t m = std::min(kStageChunk, bytes - off);
-      cudaError_t e = cudaMemcpyAsync(ctx->h_stage.as<uint8_t>() + (size_t)k * kStageChunk,
-                                      static_cast<const uint8_t *>(d) + off, m, cudaMemcpyDeviceToHost, ctx->stream);
-      if (e != cudaSuccess) { rc = set_cuda_error(ctx, e, "d2h staging"); break; }
-      cudaEventRecord(ev[k], ctx->stream);
-      pend_off[k] = off; pend_len[k] = m;
-      off += m;
-    }
-    k ^= 1;
-  }
-  cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]);
-  return rc;
+  StageRing ring(ctx);
+  if (int st = ring.open()) return st;
+  for (size_t off = 0; off < bytes; off += kStageChunk)
+    if (int st = ring.download(static_cast<uint8_t *>(h) + off, static_cast<const uint8_t *>(d) + off, std::min(kStageChunk, bytes - off)))
+      return st;
+  return ring.drain();
 }
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) & ~(a - 1); }
@@ -154,7 +187,7 @@ static uint64_t env_u64(const char *name, uint64_t dflt) {
 int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const size_t *len,
                   std::vector<const uint8_t *> &d_ptr, UploadSplit *split) {
   d_ptr.assign(n, nullptr);
-  if (split) split->parts = 0;
+  if (split) split->cut = 0;
   ctx->epoch++;  // new input bytes: plans made over the old ones are void
   // pipelined batches: wait for this group's turn on the bus; the next group may go once these bytes have arrived
   struct GatePass {
@@ -211,20 +244,15 @@ int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const si
     uint8_t *base = ctx->d_in.as<uint8_t>() + pre;
     for (size_t i = 0; i < n; i++) d_ptr[i] = len[i] ? base + ((uintptr_t)src[i] - lo) : base;
     if (split && split->want && span >= (128u << 20) && !ctx->gate && is_pinned((const void *)lo)) {
-      // K parts (ZIPC_B200_UPLOAD_PARTS, default 2: measured 40.3 GB/s end to end on C3, 36-37 with 3 to 6 parts, whose
-      // size-ordered queues each end in a tail of large streams), cut at starts of ranges: the first on the context's stream (what follows on that stream may use it), the
-      // others one after the other on their own stream, each arrival announced through d_upflag
-      static const uint64_t want_parts = std::min<uint64_t>(env_u64("ZIPC_B200_UPLOAD_PARTS", 2), 8);
-      uint32_t K = 1;
-      for (uint32_t p = 1; p < want_parts; p++) {
-        const uintptr_t target = lo + span / want_parts * p;
-        uintptr_t cut = hi;
-        for (size_t i = 0; i < n; i++) { const uintptr_t a = (uintptr_t)src[i]; if (len[i] && a >= target && a < cut) cut = a; }
-        if (cut < hi && cut > (K > 1 ? split->cut[K - 1] : lo)) split->cut[K++] = cut;
-      }
-      if (K >= 2) {
+      // two parts (measured 40.3 GB/s end to end on C3, 36-37 with 3 to 6 parts, whose size-ordered queues each end in a tail
+      // of large streams), cut at the first start of a range in the second half of the span: the first part on the context's
+      // stream (what follows on that stream may use it), the second behind it on its own stream, its arrival announced
+      // through d_upflag
+      uintptr_t cut = hi;
+      for (size_t i = 0; i < n; i++) { const uintptr_t a = (uintptr_t)src[i]; if (len[i] && a >= lo + span / 2 && a < cut) cut = a; }
+      if (cut < hi && cut > lo) {
         if (!ctx->upload_stream) ZB_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->upload_stream, cudaStreamNonBlocking));
-        if (ctx->upload_split_live) {  // (a call that failed half way left its late parts behind: their flag words must not be rewritten under them)
+        if (ctx->upload_split_live) {  // (a call that failed half way left its second part behind: its flag word must not be rewritten under it)
           ZB_CUDA(ctx, cudaStreamSynchronize(ctx->upload_stream));
           ctx->upload_split_live = false;
         }
@@ -233,19 +261,16 @@ int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const si
           ZB_CUDA(ctx, cudaMalloc(reinterpret_cast<void **>(&ctx->d_upflag), 64));
           ZB_CUDA(ctx, cudaMemset(ctx->d_upflag, 0, 64));
         }
-        ctx->upload_serial += 16;  // counts of this upload: serial + 1 .. serial + K - 1
-        ZB_CUDA(ctx, cudaMemcpyAsync(base, (const void *)lo, split->cut[1] - lo, cudaMemcpyHostToDevice, ctx->stream));
+        ctx->upload_serial += 16;  // the count of this upload's second part: serial + 1
+        ZB_CUDA(ctx, cudaMemcpyAsync(base, (const void *)lo, cut - lo, cudaMemcpyHostToDevice, ctx->stream));
         if (!ctx->ev_half) ZB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_half, cudaEventDisableTiming));
         ZB_CUDA(ctx, cudaEventRecord(ctx->ev_half, ctx->stream));
         ZB_CUDA(ctx, cudaStreamWaitEvent(ctx->upload_stream, ctx->ev_half, 0));  // one part after the other: each gets the whole bus
-        for (uint32_t p = 1; p < K; p++) {
-          const uintptr_t a = split->cut[p], b = p + 1 < K ? split->cut[p + 1] : hi;
-          ctx->h_gflag[240 + p] = ctx->upload_serial + p;
-          ZB_CUDA(ctx, cudaMemcpyAsync(base + (a - lo), (const void *)a, b - a, cudaMemcpyHostToDevice, ctx->upload_stream));
-          ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_upflag, &ctx->h_gflag[240 + p], sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->upload_stream));
-        }
+        ctx->h_gflag[241] = ctx->upload_serial + 1;  // (above the group flags)
+        ZB_CUDA(ctx, cudaMemcpyAsync(base + (cut - lo), (const void *)cut, hi - cut, cudaMemcpyHostToDevice, ctx->upload_stream));
+        ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_upflag, &ctx->h_gflag[241], sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->upload_stream));
         ctx->upload_split_live = true;
-        split->parts = K;
+        split->cut = cut;
         return ZIPC_OK;
       }
     }
@@ -264,18 +289,14 @@ int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const si
   // pageable ranges: packed into pinned staging chunk by chunk (CPU copy of chunk k+1 overlaps the DMA of chunk k);
   // consecutive pageable ranges keep consecutive device offsets, so a staged run is one DMA
   if (pageable) {
-    if (int st = ctx->h_stage.reserve(2 * kStageChunk)) return st;
-    cudaEvent_t ev[2];
-    ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming));
-    ZB_CUDA(ctx, cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming));
-    bool used[2] = {false, false};
-    int k = 0, rc = ZIPC_OK;
+    StageRing ring(ctx);
+    if (int st = ring.open()) return st;
     size_t i = 0, done_in_i = 0;  // next range / bytes of it already staged
-    while (rc == ZIPC_OK) {
+    for (;;) {
       while (i < n && (!len[i] || pin[i])) { i++; done_in_i = 0; }
       if (i >= n) break;
-      uint8_t *s = ctx->h_stage.as<uint8_t>() + (size_t)k * kStageChunk;
-      if (used[k]) cudaEventSynchronize(ev[k]);
+      uint8_t *s;
+      if (int st = ring.next(&s)) return st;
       // fill this staging buffer with a run of device-contiguous pageable bytes
       const size_t dev_start = off[i] + done_in_i;
       size_t fill = 0;
@@ -291,19 +312,23 @@ int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const si
           if (padto == align_up(len[i], 16) - len[i]) { fill += padto; i++; done_in_i = 0; } else break;
         }
       }
-      cudaError_t e = cudaMemcpyAsync(dbase + dev_start, s, fill, cudaMemcpyHostToDevice, ctx->stream);
-      if (e != cudaSuccess) { rc = set_cuda_error(ctx, e, "upload_ranges staging"); break; }
-      cudaEventRecord(ev[k], ctx->stream);
-      used[k] = true;
-      k ^= 1;
+      if (int st = ring.upload(dbase + dev_start, fill)) return st;
     }
-    for (int j = 0; j < 2; j++) { if (used[j]) cudaEventSynchronize(ev[j]); cudaEventDestroy(ev[j]); }
-    if (rc) return rc;
+    if (int st = ring.drain()) return st;
   }
   for (size_t i = 0; i < n; i++)
     if (len[i] && pin[i]) ZB_CUDA(ctx, cudaMemcpyAsync(dbase + off[i], src[i], len[i], cudaMemcpyHostToDevice, ctx->stream));
   for (size_t i = 0; i < n; i++) d_ptr[i] = dbase + off[i];
   return ZIPC_OK;
+}
+
+int upload_buffer(zipc_b200_ctx *ctx, const void *src, size_t len, const uint8_t **d) {
+  ctx->epoch++;  // new input bytes: plans made over the old ones are void
+  const size_t pre = (uintptr_t)src & 15;  // keep the host alignment so 16-byte paths stay aligned
+  if (int st = ctx->d_in.reserve(pre + len + 64)) return st;
+  uint8_t *p = ctx->d_in.as<uint8_t>() + pre;
+  *d = p;
+  return h2d(ctx, p, src, len);
 }
 
 static __global__ void make_crc_segs_kernel(const InflateTask *tasks, const InflateResult *res, uint32_t n, CrcSeg *segs) {
@@ -676,11 +701,10 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
         if (ok && checksum) {
           checksum[i] = 0;
           if (ck == ZIPC_CK_CRC32) {
-            // (the result word through mapped host memory: a 4-byte copy into the caller's pageable array would hold up every lane)
-            if (!c->h_word) ZB_CUDA(c, cudaHostAlloc(reinterpret_cast<void **>(&c->h_word), 64, cudaHostAllocMapped));
-            if (int st = crc32_launch_buffer(c, d_dst[i], total, c->h_word + 1)) return st;
+            // (a 4-byte copy into the caller's pageable array would hold up every lane)
+            if (int st = crc32_to_host_word(c, d_dst[i], total)) return st;
             ZB_CUDA(c, stream_sync(c, c->stream));
-            checksum[i] = reinterpret_cast<volatile uint32_t *>(c->h_word)[1];
+            checksum[i] = host_word_crc32(c);
           } else if (ck == ZIPC_CK_ADLER32) {
             // folded block by block, each block on its own 5552-byte grid with the state re-packed in between, as the reference
             // does while it decodes (zipc_deflate.ml:682-690): the chunks reported the lengths of their blocks
@@ -773,11 +797,10 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
 }
 
 // ---- progressive download ---------------------------------------------------------------------------------------------------
-// ZIPC_B200_DOWNLOAD_GROUPS: groups of a progressive download (default 32; 0 or 1 = one copy after the kernel).
-static uint64_t download_groups() { static const uint64_t v = std::min<uint64_t>(env_u64("ZIPC_B200_DOWNLOAD_GROUPS", 32), 200); return v; }
+static constexpr uint32_t kDownloadGroups = 32;
 
 bool progressive_ok(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *src_len, const char *grouped, void *dst, size_t dst_cap) {
-  if (download_groups() < 2 || !dst || ctx->is_sub) return false;
+  if (!dst || ctx->is_sub) return false;
   size_t sum = 0, ng = 0;
   for (size_t i = 0; i < n; i++) {
     if (cap[i] == ZIPC_SIZE_UNKNOWN) return false;
@@ -787,8 +810,8 @@ bool progressive_ok(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_
   return ng >= 1024 && sum >= (64ull << 20) && dst_cap >= sum && is_pinned(dst);
 }
 
-int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *src_len, const char *grouped, const char *late, void *dst,
-               size_t dst_cap, std::vector<size_t> &off, size_t &total, DownloadPlan &plan) {
+int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const void *const *src, const size_t *src_len, const char *grouped,
+               const UploadSplit &split, void *dst, size_t dst_cap, std::vector<size_t> &off, size_t &total, DownloadPlan &plan) {
   off.assign(n, 0);
   plan = DownloadPlan{};
   if (!progressive_ok(ctx, n, cap, src_len, grouped, dst, dst_cap)) {
@@ -798,14 +821,15 @@ int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *sr
     return ZIPC_OK;
   }
   // grouped streams: in the order in which the parts of the upload arrive, then by ascending output size; equal counts per group
+  std::vector<char> late(n);
+  for (size_t i = 0; i < n; i++) late[i] = src_len[i] && split.late(src[i]);
   std::vector<uint32_t> idx;
   for (size_t i = 0; i < n; i++) if (grouped[i]) idx.push_back((uint32_t)i);
   std::sort(idx.begin(), idx.end(), [&](uint32_t a, uint32_t b) {
-    const int la = late ? late[a] : 0, lb = late ? late[b] : 0;
-    return la != lb ? la < lb : cap[a] != cap[b] ? cap[a] < cap[b] : a < b; });
-  const uint32_t G = (uint32_t)download_groups();
+    return late[a] != late[b] ? late[a] < late[b] : cap[a] != cap[b] ? cap[a] < cap[b] : a < b; });
+  const uint32_t G = kDownloadGroups;
   plan.ngroups = G; plan.group_of.assign(n, 0); plan.goff.assign(G, 0); plan.gbytes.assign(G, 0); plan.dst = static_cast<uint8_t *>(dst);
-  if (late) plan.late.assign(late, late + n);
+  if (split.cut) plan.late = late;
   size_t t = 0;
   for (size_t r = 0; r < idx.size(); r++) {
     const uint32_t i = idx[r], g = (uint32_t)(r * G / idx.size());
@@ -822,25 +846,22 @@ int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *sr
   return ZIPC_OK;
 }
 
-// the grouped ranges are on their way (inflate_core); copy the rest and wait for all of it
-int finish_download(zipc_b200_ctx *ctx, const DownloadPlan &plan) {
-  if (plan.tail_bytes)
-    ZB_CUDA(ctx, cudaMemcpyAsync(plan.dst + plan.tail_off, ctx->d_out.as<uint8_t>() + plan.tail_off, plan.tail_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+int finish_to_host(zipc_b200_ctx *ctx, const std::vector<size_t> &off, size_t total, void *dst, size_t dst_cap, size_t *dst_off,
+                   size_t *dst_need, const DownloadPlan *plan) {
+  ctx->last_total = total;
+  if (dst_off) std::copy(off.begin(), off.end(), dst_off);
+  if (dst_need) *dst_need = total;
+  if (!dst || dst_cap < total) {
+    ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
+    return ZIPC_ERR_DST_TOO_SMALL;
+  }
+  if (!plan || !plan->ngroups) return d2h(ctx, dst, ctx->d_out.p, total);
+  // the groups are on their way (inflate_core): copy the rest and wait for all of it
+  if (plan->tail_bytes)
+    ZB_CUDA(ctx, cudaMemcpyAsync(plan->dst + plan->tail_off, ctx->d_out.as<uint8_t>() + plan->tail_off, plan->tail_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   ZB_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
   ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
   return ZIPC_OK;
-}
-
-// Shared tail of the host-pointer batch calls: lay out the arena, run, copy back.
-static int finish_to_host(zipc_b200_ctx *ctx, size_t n, const std::vector<size_t> &off, const size_t *len, size_t total,
-                   void *dst, size_t dst_cap, size_t *dst_need, size_t *dst_off) {
-  ctx->last_off = off;
-  ctx->last_len.assign(len, len + n);
-  ctx->last_total = total;
-  for (size_t i = 0; i < n; i++) dst_off[i] = off[i];
-  if (dst_need) *dst_need = total;
-  if (!dst || dst_cap < total) return ZIPC_ERR_DST_TOO_SMALL;
-  return d2h(ctx, dst, ctx->d_out.p, total);
 }
 
 void pipe_mark(const zipc_b200_ctx *ctx, const char *stage) {
@@ -928,6 +949,7 @@ void zipc_b200_ctx_destroy(zipc_b200_ctx *ctx) {
   if (ctx->hi_stream) cudaStreamDestroy(ctx->hi_stream);
   if (ctx->d_upflag) cudaFree(ctx->d_upflag);
   if (ctx->ev_half) cudaEventDestroy(ctx->ev_half);
+  for (cudaEvent_t e : ctx->ev_stage) if (e) cudaEventDestroy(e);
   if (ctx->ev_block) cudaEventDestroy(ctx->ev_block);
   if (ctx->h_gflag) cudaFreeHost(ctx->h_gflag);
   if (ctx->h_word) cudaFreeHost(ctx->h_word);
@@ -1007,21 +1029,17 @@ int zipc_b200_crc32_dev_async(zipc_b200_ctx *ctx, const void *d_src, size_t len,
 int zipc_b200_crc32_dev(zipc_b200_ctx *ctx, const void *d_src, size_t len, uint32_t *crc) {
   if (!ctx || !crc || (!d_src && len)) return ZIPC_ERR_INVALID_ARG;
   DeviceGuard g(ctx->device);
-  // the combine kernel's last thread stores the one-word result straight into mapped host memory (as adler32_launch_buffer does)
-  if (!ctx->h_word) ZB_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_word), 64, cudaHostAllocMapped));
-  if (int st = crc32_launch_buffer(ctx, static_cast<const uint8_t *>(d_src), len, ctx->h_word + 1)) return st;
+  if (int st = crc32_to_host_word(ctx, static_cast<const uint8_t *>(d_src), len)) return st;
   ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
-  *crc = reinterpret_cast<volatile uint32_t *>(ctx->h_word)[1];
+  *crc = host_word_crc32(ctx);
   return ZIPC_OK;
 }
 
 int zipc_b200_crc32(zipc_b200_ctx *ctx, const void *src, size_t len, uint32_t *crc) {
   if (!ctx || !crc || (!src && len)) return ZIPC_ERR_INVALID_ARG;
   DeviceGuard g(ctx->device);
-  size_t pre = (uintptr_t)src & 15;
-  if (int st = ctx->d_in.reserve(pre + len + 64)) return st;
-  uint8_t *d = ctx->d_in.as<uint8_t>() + pre;
-  if (int st = h2d(ctx, d, src, len)) return st;
+  const uint8_t *d;
+  if (int st = upload_buffer(ctx, src, len, &d)) return st;
   return zipc_b200_crc32_dev(ctx, d, len, crc);
 }
 
@@ -1035,10 +1053,8 @@ int zipc_b200_adler32_dev(zipc_b200_ctx *ctx, const void *d_src, size_t len, int
 int zipc_b200_adler32(zipc_b200_ctx *ctx, const void *src, size_t len, int mode, uint32_t *adler) {
   if (!ctx || !adler || (!src && len)) return ZIPC_ERR_INVALID_ARG;
   DeviceGuard g(ctx->device);
-  size_t pre = (uintptr_t)src & 15;
-  if (int st = ctx->d_in.reserve(pre + len + 64)) return st;
-  uint8_t *d = ctx->d_in.as<uint8_t>() + pre;
-  if (int st = h2d(ctx, d, src, len)) return st;
+  const uint8_t *d;
+  if (int st = upload_buffer(ctx, src, len, &d)) return st;
   return zipc_b200_adler32_dev(ctx, d, len, mode, adler);
 }
 
@@ -1052,7 +1068,7 @@ int zipc_b200_crc32_batch(zipc_b200_ctx *ctx, size_t n, const void *const *src, 
   if (int st = ctx->d_desc.reserve(n * sizeof(CrcSeg))) return st;
   if (int st = ctx->d_res.reserve(n * sizeof(uint32_t))) return st;
   CrcSeg *hs = ctx->h_desc.as<CrcSeg>();
-  for (size_t i = 0; i < n; i++) { hs[i].ptr = dp[i]; hs[i].len = len[i]; hs[i].init = 0xFFFFFFFFu; hs[i]._pad = 0; }
+  for (size_t i = 0; i < n; i++) hs[i] = crc_seg(dp[i], len[i]);
   ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc.p, hs, n * sizeof(CrcSeg), cudaMemcpyHostToDevice, ctx->stream));
   if (int st = crc32_launch_segments(ctx, ctx->d_desc.as<CrcSeg>(), (uint32_t)n, ctx->d_res.as<uint32_t>())) return st;
   ZB_CUDA(ctx, cudaMemcpyAsync(crc, ctx->d_res.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1096,11 +1112,7 @@ int zipc_b200_inflate_batch(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n
   std::vector<size_t> off;
   size_t total = 0;
   DownloadPlan plan;
-  {
-    std::vector<char> late;
-    if (split.parts) { late.resize(n); for (size_t i = 0; i < n; i++) late[i] = src_len[i] ? (char)split.part_of(src[i]) : 0; }
-    if (int st = plan_arena(ctx, n, cap.data(), src_len, all.data(), split.parts ? late.data() : nullptr, dst, dst_cap, off, total, plan)) return st;
-  }
+  if (int st = plan_arena(ctx, n, cap.data(), src, src_len, all.data(), split, dst, dst_cap, off, total, plan)) return st;
   if (int st = ctx->d_out.reserve(total + 64)) return st;
   for (size_t i = 0; i < n; i++) d_dst[i] = ctx->d_out.as<uint8_t>() + off[i];
   if (int st = inflate_core(ctx, ck, adler_mode, n, d_src, src_len, d_dst, cap, false, dst_len, checksum, status, 0, &plan)) {
@@ -1110,20 +1122,13 @@ int zipc_b200_inflate_batch(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n
   // a stream of unknown size that failed while being sized keeps that (uncapped) verdict
   for (size_t i = 0; i < n; i++)
     if (was_unknown[i] && cs[i] != ZIPC_OK) { status[i] = cs[i]; dst_len[i] = 0; if (checksum) checksum[i] = 0; }
-  if (plan.ngroups) {
-    ctx->last_off = off; ctx->last_len.assign(dst_len, dst_len + n); ctx->last_total = total;
-    for (size_t i = 0; i < n; i++) dst_off[i] = off[i];
-    if (dst_need) *dst_need = total;
-    return finish_download(ctx, plan);
-  }
-  return finish_to_host(ctx, n, off, dst_len, total, dst, dst_cap, dst_need, dst_off);
+  return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need, &plan);
 }
 
 int zipc_b200_fetch(zipc_b200_ctx *ctx, void *dst, size_t dst_cap) {
   if (!ctx || !dst) return ZIPC_ERR_INVALID_ARG;
-  if (dst_cap < ctx->last_total) return ZIPC_ERR_DST_TOO_SMALL;
   DeviceGuard g(ctx->device);
-  return d2h(ctx, dst, ctx->d_out.p, ctx->last_total);
+  return finish_to_host(ctx, {}, ctx->last_total, dst, dst_cap, nullptr, nullptr);
 }
 
 int zipc_b200_inflate_batch_dev(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const void *d_src_v,

@@ -73,6 +73,14 @@ struct CrcSeg {       // one CRC-32 work item: state after running `len` bytes f
   uint32_t init;
   uint32_t _pad;
 };
+inline CrcSeg crc_seg(const uint8_t *ptr, uint64_t len) {  // a whole range, from the standard initial state
+  CrcSeg s;
+  s.ptr = ptr;
+  s.len = len;
+  s.init = 0xFFFFFFFFu;
+  s._pad = 0;
+  return s;
+}
 
 struct AdlerSeg {     // one Adler-32 work item: sums over [ptr, ptr+len)
   const uint8_t *ptr;
@@ -153,8 +161,9 @@ struct zipc_b200_ctx {
   uint32_t upload_serial = 0;
   cudaEvent_t ev_block = nullptr;      // stream_sync of a sub-context
   cudaEvent_t ev_half = nullptr;       // first half of a split upload is through
+  cudaEvent_t ev_stage[2] = {nullptr, nullptr};  // the last DMA of each buffer of h_stage (api.cu StageRing)
   bool upload_split_live = false;      // the late half of the current upload is still on its way
-  uint32_t *h_word = nullptr;          // mapped host memory: the one-word result of a whole-buffer Adler-32, written by the kernel
+  uint32_t *h_word = nullptr;          // mapped host memory: one-word results written by kernels (map_host_word)
   uint32_t *h_gflag = nullptr;         // mapped host memory: group-complete flags written by inflate_kernel
 
   // intra-stream parallel inflate: the plan of the last large stream decoded speculatively (a count-only pass is followed by
@@ -184,9 +193,7 @@ struct zipc_b200_ctx {
   uint32_t sm_share = 0;                       // a lane: the SMs its speculative decode spreads over (0 = all)
   cudaEvent_t ev_lanes = nullptr;              // "everything queued on `stream` so far" for the lanes' streams to wait on
 
-  // results of the last batch call kept for zipc_b200_fetch()
-  std::vector<size_t> last_off, last_len;
-  size_t last_total = 0;
+  size_t last_total = 0;   // bytes of d_out the last host-pointer call left for zipc_b200_fetch()
 };
 
 namespace zb {
@@ -242,17 +249,25 @@ int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaS
 // api.cu helpers shared with zip_api.cu
 int h2d(zipc_b200_ctx *ctx, void *d, const void *h, size_t bytes);
 int d2h(zipc_b200_ctx *ctx, void *h, const void *d, size_t bytes);
+// One whole host buffer into ctx->d_in at the host's 16-byte phase; *d: where its bytes begin.  Voids the plans made over the
+// old input bytes (ctx->epoch).
+int upload_buffer(zipc_b200_ctx *ctx, const void *src, size_t len, const uint8_t **d);
+// Allocates ctx->h_word on first use: kernels store one-word results there (word 0: Adler-32, word 1: CRC-32), so that no
+// 4-byte copy into a caller's pageable word stalls the host.  The host reads a word after its next wait for the stream.
+int map_host_word(zipc_b200_ctx *ctx);
+// enqueues the CRC-32 of a device buffer into h_word[1]; host_word_crc32 reads it
+int crc32_to_host_word(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len);
+uint32_t host_word_crc32(const zipc_b200_ctx *ctx);
 // cudaStreamSynchronize; the threads of a pipelined batch (sub-contexts) sleep on a blocking event instead of spinning: there
 // are up to 24 of them per process, and a box runs one process per GPU
 cudaError_t stream_sync(zipc_b200_ctx *ctx, cudaStream_t s);
-// A split upload (api.cu upload_ranges): the first part of a large pinned span goes out on the context's stream, the others
-// one after the other on upload_stream, each followed by a count (ctx->upload_serial + part) into ctx->d_upflag; a stream
-// whose bytes lie in part p >= 1 is decoded only after the kernel has seen that count.
+// A split upload (api.cu upload_ranges): the first part of a large pinned span goes out on the context's stream, the second
+// behind it on upload_stream, followed by a count (ctx->upload_serial + 1) into ctx->d_upflag; a stream whose bytes lie in
+// the second part is decoded only after the kernel has seen that count.
 struct UploadSplit {
-  bool want = false;        // in: the caller can deal with a split
-  uint32_t parts = 0;       // out: number of parts (0: the upload was not split)
-  uintptr_t cut[8] = {0};   // out: host address where part p begins (p = 1 .. parts - 1)
-  uint32_t part_of(const void *p) const { uint32_t k = 0; for (uint32_t j = 1; j < parts; j++) if ((uintptr_t)p >= cut[j]) k = j; return k; }
+  bool want = false;   // in: the caller can deal with a split
+  uintptr_t cut = 0;   // out: host address where the second part begins (0: the upload was not split)
+  bool late(const void *p) const { return cut && (uintptr_t)p >= cut; }
 };
 int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const size_t *len,
                   std::vector<const uint8_t *> &d_ptr, UploadSplit *split = nullptr);
@@ -265,7 +280,7 @@ struct DownloadPlan {
   std::vector<size_t> goff, gbytes;     // arena range of each group
   uint8_t *dst = nullptr;               // the caller's (pinned) arena
   size_t tail_off = 0, tail_bytes = 0;  // arena range of everything that is not a grouped stream (copied at the end)
-  std::vector<char> late;               // per stream handed to inflate_core: the part of a split upload that carries its input (0: the first)
+  std::vector<char> late;               // per stream handed to inflate_core: 1 if the second part of a split upload carries its input
 };
 int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
                  const size_t *src_len, const std::vector<uint8_t *> &d_dst, const std::vector<size_t> &cap,
@@ -273,11 +288,15 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
                  const DownloadPlan *plan = nullptr);
 // Lay out the output arena of n members (cap[i] bytes each, 16-byte aligned slots).  grouped[i] != 0 marks the streams that
 // go through the inflate kernel.  Fills off / total, and plan when the batch qualifies for a progressive download.
-// late[i] (may be null): the part of a split upload that carries the stream's input; later parts form later groups.
+// The streams whose input the second part of a split upload carries (src: their host addresses) form the later groups.
 bool progressive_ok(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *src_len, const char *grouped, void *dst, size_t dst_cap);
-int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const size_t *src_len, const char *grouped, const char *late, void *dst,
-               size_t dst_cap, std::vector<size_t> &off, size_t &total, DownloadPlan &plan);
-int finish_download(zipc_b200_ctx *ctx, const DownloadPlan &plan);
+int plan_arena(zipc_b200_ctx *ctx, size_t n, const size_t *cap, const void *const *src, const size_t *src_len, const char *grouped,
+               const UploadSplit &split, void *dst, size_t dst_cap, std::vector<size_t> &off, size_t &total, DownloadPlan &plan);
+// Tail of every host-pointer call that leaves its output in ctx->d_out: keeps `total` for zipc_b200_fetch, reports the layout
+// (dst_off, dst_need: may be null) and copies the output into the caller's arena, progressively when `plan` has groups.  Without
+// an arena, or with one too small, it returns ZIPC_ERR_DST_TOO_SMALL.  Either way the stream is through when it returns.
+int finish_to_host(zipc_b200_ctx *ctx, const std::vector<size_t> &off, size_t total, void *dst, size_t dst_cap, size_t *dst_off,
+                   size_t *dst_need, const DownloadPlan *plan = nullptr);
 // ZIPC_B200_PIPE_DEBUG=1: time stamps of the stages of a pipelined batch on stderr (group ticket, stage, ms)
 void pipe_mark(const zipc_b200_ctx *ctx, const char *stage);
 // api.cu / multi.cc: copy / compute pipelining of large host-pointer batches on one device

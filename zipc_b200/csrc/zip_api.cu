@@ -101,7 +101,7 @@ int deflate_run(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n,
   if (want_crc) {
     if (int st = ctx->d_desc2.reserve(n * (sizeof(CrcSeg) + sizeof(uint32_t)))) return st;
     CrcSeg *hs = reinterpret_cast<CrcSeg *>(ht + n);
-    for (size_t i = 0; i < n; i++) { hs[i].ptr = d_src[i]; hs[i].len = src_len[i]; hs[i].init = 0xFFFFFFFFu; hs[i]._pad = 0; }
+    for (size_t i = 0; i < n; i++) hs[i] = crc_seg(d_src[i], src_len[i]);
     CrcSeg *ds = ctx->d_desc2.as<CrcSeg>();
     dc = reinterpret_cast<uint32_t *>(ds + n);
     ZB_CUDA(ctx, cudaMemcpyAsync(ds, hs, n * sizeof(CrcSeg), cudaMemcpyHostToDevice, ctx->stream));
@@ -323,11 +323,9 @@ int deflate_batch_layout(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, 
   size_t total = 0;
   for (size_t i = 0; i < n; i++) { off[i] = total + (gap ? gap[i] : 0); total = off[i] + align_up(dst_len[i], align); }
   if (int st = compact_pieces(ctx, pc, off, total)) return st;
-  ctx->last_off = off; ctx->last_len.assign(dst_len, dst_len + n); ctx->last_total = total;
-  for (size_t i = 0; i < n; i++) dst_off[i] = off[i];
-  if (dst_need) *dst_need = total;
-  if (!dst || dst_cap < total) { ZB_CUDA(ctx, stream_sync(ctx, ctx->stream)); pipe_mark(ctx, "compacted"); return ZIPC_ERR_DST_TOO_SMALL; }
-  return d2h(ctx, dst, ctx->d_out.p, total);
+  const int rc = finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
+  pipe_mark(ctx, "compacted");
+  return rc;
 }
 
 }  // namespace zb
@@ -416,12 +414,8 @@ int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode,
     ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, h, (2 * n + np) * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
     if (int st = gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)(2 * n + np))) return st;
   }
-  for (size_t i = 0; i < n; i++) dst_off[i] = off[i];
-  ctx->last_off = off; ctx->last_len = flen; ctx->last_total = total;
   for (size_t i = 0; i < n; i++) { dst_len[i] = flen[i]; if (adler) adler[i] = ad[i]; }
-  if (dst_need) *dst_need = total;
-  if (!dst || dst_cap < total) { ZB_CUDA(ctx, stream_sync(ctx, ctx->stream)); return ZIPC_ERR_DST_TOO_SMALL; }
-  return d2h(ctx, dst, ctx->d_out.p, total);
+  return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
 }
 
 // ---- segmented single stream -----------------------------------------------------------------------------
@@ -436,10 +430,8 @@ static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size
   *nseg_out = nseg;
   if (index && index_cap_pairs < nseg + 1) return ZIPC_ERR_INVALID_ARG;
   // input to the device (one copy), segments are slices of it
-  const size_t pre = (uintptr_t)src & 15;
-  if (int st = ctx->d_in.reserve(pre + len + 64)) return st;
-  uint8_t *d_base = ctx->d_in.as<uint8_t>() + pre;
-  if (int st = h2d(ctx, d_base, src, len)) return st;
+  const uint8_t *d_base;
+  if (int st = upload_buffer(ctx, src, len, &d_base)) return st;
   std::vector<const uint8_t *> d_src(nseg);
   std::vector<size_t> slen(nseg);
   std::vector<uint32_t> flags(nseg, kDeflateNotFinal);
@@ -456,12 +448,8 @@ static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size
   if (int st = make_slots(ctx, nseg, slen.data(), d_slot, cap)) return st;
   if (int st = deflate_run(ctx, level, ZIPC_CK_NONE, 0, nseg, d_src, slen.data(), d_slot, cap, clen.data(), nullptr, st_m.data(), &flags)) return st;
   for (size_t i = 0; i < nseg; i++) if (st_m[i]) return st_m[i];
-  if (crc32) {
-    if (int st = ctx->d_small.reserve(256)) return st;
-    uint32_t *d_crc = ctx->d_small.as<uint32_t>() + 32;
-    if (int st = crc32_launch_buffer(ctx, d_base, len, d_crc)) return st;
-    ZB_CUDA(ctx, cudaMemcpyAsync(crc32, d_crc, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  }
+  if (crc32)
+    if (int st = crc32_to_host_word(ctx, d_base, len)) return st;
   // the pieces are byte aligned: concatenate without gaps
   std::vector<size_t> off(nseg);
   size_t total = 0;
@@ -471,10 +459,9 @@ static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size
     index[2 * nseg] = total; index[2 * nseg + 1] = len;
   }
   if (int st = compact(ctx, nseg, d_slot, clen.data(), off, total)) return st;
-  ctx->last_off = off; ctx->last_len = clen; ctx->last_total = total;
-  *dst_len = total;
-  if (!dst || dst_cap < total) { ZB_CUDA(ctx, stream_sync(ctx, ctx->stream)); return ZIPC_ERR_DST_TOO_SMALL; }
-  return d2h(ctx, dst, ctx->d_out.p, total);
+  const int rc = finish_to_host(ctx, off, total, dst, dst_cap, nullptr, dst_len);
+  if (crc32 && (rc == ZIPC_OK || rc == ZIPC_ERR_DST_TOO_SMALL)) *crc32 = host_word_crc32(ctx);
+  return rc;
 }
 
 int zipc_b200_deflate_segmented(zipc_b200_ctx *ctx, int level, const void *src, size_t len, size_t segment_size,
@@ -498,10 +485,8 @@ int zipc_b200_inflate_segmented(zipc_b200_ctx *ctx, const void *src, size_t len,
   for (size_t i = 0; i < nseg; i++)
     if (index[2 * i] > index[2 * i + 2] || index[2 * i + 1] > index[2 * i + 3]) return ZIPC_ERR_INVALID_ARG;
   *dst_len = utotal;
-  const size_t pre = (uintptr_t)src & 15;
-  if (int st = ctx->d_in.reserve(pre + len + 64)) return st;
-  uint8_t *d_base = ctx->d_in.as<uint8_t>() + pre;
-  if (int st = h2d(ctx, d_base, src, len)) return st;
+  const uint8_t *d_base;
+  if (int st = upload_buffer(ctx, src, len, &d_base)) return st;
   if (int st = ctx->d_out.reserve(utotal + 64)) return st;
   std::vector<const uint8_t *> d_src(nseg);
   std::vector<uint8_t *> d_dst(nseg);
@@ -517,15 +502,11 @@ int zipc_b200_inflate_segmented(zipc_b200_ctx *ctx, const void *src, size_t len,
     if (st_m[i]) { *status = st_m[i]; break; }
     if (ol[i] != cap[i]) { *status = ZIPC_ERR_CORRUPTED; break; }  // the index promised more bytes
   }
-  if (crc32) {
-    if (int st = ctx->d_small.reserve(256)) return st;
-    uint32_t *d_crc = ctx->d_small.as<uint32_t>() + 32;
-    if (int st = crc32_launch_buffer(ctx, ctx->d_out.as<uint8_t>(), utotal, d_crc)) return st;
-    ZB_CUDA(ctx, cudaMemcpyAsync(crc32, d_crc, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  }
-  ctx->last_off.assign(1, 0); ctx->last_len.assign(1, (size_t)utotal); ctx->last_total = utotal;
-  if (!dst || dst_cap < utotal) { ZB_CUDA(ctx, stream_sync(ctx, ctx->stream)); return ZIPC_ERR_DST_TOO_SMALL; }
-  return d2h(ctx, dst, ctx->d_out.p, utotal);
+  if (crc32)
+    if (int st = crc32_to_host_word(ctx, ctx->d_out.as<uint8_t>(), utotal)) return st;
+  const int rc = finish_to_host(ctx, {}, utotal, dst, dst_cap, nullptr, nullptr);
+  if (crc32 && (rc == ZIPC_OK || rc == ZIPC_ERR_DST_TOO_SMALL)) *crc32 = host_word_crc32(ctx);
+  return rc;
 }
 
 // ---- archive layer ---------------------------------------------------------------------------------------
@@ -562,11 +543,7 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
   std::vector<size_t> off;
   size_t total = 0;
   DownloadPlan plan;
-  {
-    std::vector<char> late;
-    if (split.parts) { late.resize(n); for (size_t i = 0; i < n; i++) late[i] = slen[i] ? (char)split.part_of(src[i]) : 0; }
-    if (int st = plan_arena(ctx, n, cap.data(), slen.data(), grouped.data(), split.parts ? late.data() : nullptr, dst, dst_cap, off, total, plan)) return st;
-  }
+  if (int st = plan_arena(ctx, n, cap.data(), src.data(), slen.data(), grouped.data(), split, dst, dst_cap, off, total, plan)) return st;
   // whatever way this call ends, no progressive copy into the caller's arena outlives it
   struct CopyFence {
     zipc_b200_ctx *c;
@@ -611,7 +588,7 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
     for (size_t j = 0; j < k; j++) {
       size_t i = idx[j];
       hc[j] = CopyDesc{d_src[i], ctx->d_out.as<uint8_t>() + off[i], slen[i]};
-      hs[j].ptr = d_src[i]; hs[j].len = slen[i]; hs[j].init = 0xFFFFFFFFu; hs[j]._pad = 0;
+      hs[j] = crc_seg(d_src[i], slen[i]);
     }
     CopyDesc *dc = ctx->d_desc2.as<CopyDesc>();
     CrcSeg *ds = reinterpret_cast<CrcSeg *>(dc + k);
@@ -630,12 +607,7 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
       if (c != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
     }
   }
-  ctx->last_off = off; ctx->last_len.assign(dst_len, dst_len + n); ctx->last_total = total;
-  for (size_t i = 0; i < n; i++) dst_off[i] = off[i];
-  if (dst_need) *dst_need = total;
-  if (!dst || dst_cap < total) return ZIPC_ERR_DST_TOO_SMALL;
-  if (plan.ngroups) return finish_download(ctx, plan);
-  return d2h(ctx, dst, ctx->d_out.p, total);
+  return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need, &plan);
 }
 
 int zipc_b200_zip_deflate_archive(zipc_b200_ctx *ctx, int level, size_t n, const char *const *paths,
