@@ -176,6 +176,17 @@ int zipc_b200_zlib_decompress_batch(zipc_b200_ctx *ctx, int adler_mode, size_t n
                                     const size_t *max_out, void *dst, size_t dst_cap,
                                     size_t *dst_need, size_t *dst_off, size_t *dst_len,
                                     uint32_t *expect, uint32_t *found, int *status);
+/* Device-resident Zipc_deflate.zlib_decompress (src/zipc_deflate.mli:104-118, zipc_deflate.ml:720-740): arguments and output
+ * contract of zipc_b200_inflate_batch_dev (any src_off / dst_off; stream i is read from [src_off[i], src_off[i] + src_len[i])
+ * only, so its 4-byte trailer is the last 4 bytes of that range; output inside [dst_off[i], dst_off[i] + max_out[i]);
+ * ZIPC_SIZE_UNKNOWN is ZIPC_ERR_INVALID_ARG), results of zipc_b200_zlib_decompress_batch for the same bytes (status, dst_len,
+ * expect / found, found = the method on ZIPC_ERR_ZLIB_METHOD; the body is [2, src_len - 2) as in the reference,
+ * zipc_deflate.ml:732).  The headers are checked on the device, in the reference's order; a stream whose header is
+ * rejected is not decoded and its slot is not written.  adler_mode is ZIPC_ADLER_*. */
+int zipc_b200_zlib_decompress_batch_dev(zipc_b200_ctx *ctx, int adler_mode, size_t n,
+                                        const void *d_src, const size_t *src_off, const size_t *src_len,
+                                        void *d_dst, const size_t *dst_off, const size_t *max_out,
+                                        size_t *dst_len, uint32_t *expect, uint32_t *found, int *status);
 
 /* ---- deflate ------------------------------------------------------------------------------- */
 /* Zipc_deflate.deflate / crc_32_and_deflate / adler_32_and_deflate for n independent inputs
@@ -212,6 +223,21 @@ int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode,
                                   const void *const *src, const size_t *src_len,
                                   void *dst, size_t dst_cap, size_t *dst_need,
                                   size_t *dst_off, size_t *dst_len, uint32_t *adler, int *status);
+/* Device-resident Zipc_deflate.zlib_compress (src/zipc_deflate.mli:151-162, zipc_deflate.ml:1262-1277): input i is
+ * [src_off[i], src_off[i] + src_len[i]) of d_src (any alignment), stream i goes to the caller's slot at dst_off[i] of d_dst
+ * (any alignment, unlike zipc_b200_deflate_batch_dev) with capacity dst_cap_each[i]; zipc_b200_zlib_bound(src_len[i])
+ * always suffices.  Members are compressed as by zipc_b200_zlib_compress_batch, large ones as primed segments over many
+ * CTAs, and the streams and adler[] are byte for byte those it returns for the same batch.  On success exactly
+ * [dst_off[i], dst_off[i] + dst_len[i]) is written.  A stream that does not fit its slot gives status[i] =
+ * ZIPC_ERR_DST_TOO_SMALL, dst_len[i] = 0, adler[i] = 0, and nothing of its slot is written; the other members are not
+ * affected.  adler_mode is ZIPC_ADLER_*; adler may be NULL. */
+int zipc_b200_zlib_compress_batch_dev(zipc_b200_ctx *ctx, int level, int adler_mode, size_t n,
+                                      const void *d_src, const size_t *src_off, const size_t *src_len,
+                                      void *d_dst, const size_t *dst_off, const size_t *dst_cap_each,
+                                      size_t *dst_len, uint32_t *adler, int *status);
+/* Upper bound of a zlib stream of zipc_b200_zlib_compress_batch(_dev) for an input of src_len bytes, whatever segments the
+ * library cuts the input into (slot sizing). */
+size_t zipc_b200_zlib_bound(size_t src_len);
 
 /* ---- one large stream as independent segments (BASELINE.json configs 1 and 5) ----------------------- */
 /* Zipc_deflate.crc_32_and_deflate for ONE large input, parallel inside the stream: the input is cut into

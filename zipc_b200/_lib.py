@@ -32,7 +32,8 @@ EXPORTS = [
     "zipc_b200_adler32_dev", "zipc_b200_crc32_batch", "zipc_b200_crc32_combine", "zipc_b200_adler32_combine",
     "zipc_b200_inflate_batch", "zipc_b200_fetch", "zipc_b200_inflate_batch_dev", "zipc_b200_zlib_decompress_batch",
     "zipc_b200_deflate_batch", "zipc_b200_deflate_batch_dev", "zipc_b200_deflate_bound",
-    "zipc_b200_zlib_compress_batch", "zipc_b200_deflate_segmented", "zipc_b200_deflate_primed", "zipc_b200_inflate_segmented", "zipc_b200_ptime_to_dos", "zipc_b200_ptime_of_dos", "zipc_b200_zip_parse",
+    "zipc_b200_zlib_compress_batch", "zipc_b200_zlib_decompress_batch_dev", "zipc_b200_zlib_compress_batch_dev",
+    "zipc_b200_zlib_bound", "zipc_b200_deflate_segmented", "zipc_b200_deflate_primed", "zipc_b200_inflate_segmented", "zipc_b200_ptime_to_dos", "zipc_b200_ptime_of_dos", "zipc_b200_zip_parse",
     "zipc_b200_zip_encoding_size", "zipc_b200_zip_assemble", "zipc_b200_zip_extract_batch",
     "zipc_b200_zip_parse_ex", "zipc_b200_zip_encoding_size_ex", "zipc_b200_zip_assemble_ex", "zipc_b200_inflate_plan", "zipc_b200_zip_deflate_archive_ex",
     "zipc_b200_zip_deflate_archive", "zipc_b200_free", "zipc_b200_synth_text", "zipc_b200_synth_rand",
@@ -90,6 +91,9 @@ def _declare(L):
         "zipc_b200_deflate_batch_dev": (i32, [vp, i32, i32, i32, sz, vp, szp, szp, vp, szp, szp, szp, u32p, ip]),
         "zipc_b200_deflate_bound": (sz, [sz]),
         "zipc_b200_zlib_compress_batch": (i32, [vp, i32, i32, sz, vpp, szp, vp, sz, szp, szp, szp, u32p, ip]),
+        "zipc_b200_zlib_decompress_batch_dev": (i32, [vp, i32, sz, vp, szp, szp, vp, szp, szp, szp, u32p, u32p, ip]),
+        "zipc_b200_zlib_compress_batch_dev": (i32, [vp, i32, i32, sz, vp, szp, szp, vp, szp, szp, szp, u32p, ip]),
+        "zipc_b200_zlib_bound": (sz, [sz]),
         "zipc_b200_deflate_segmented": (i32, [vp, i32, vp, sz, sz, i32, vp, sz, szp, P(u64), sz, szp, u32p]),
         "zipc_b200_deflate_primed": (i32, [vp, i32, vp, sz, sz, i32, vp, sz, szp, P(u64), sz, szp, u32p]),
         "zipc_b200_inflate_segmented": (i32, [vp, vp, sz, P(u64), sz, vp, sz, szp, u32p, ip]),

@@ -345,6 +345,16 @@ static __global__ void xor_ffffffff_kernel(uint32_t *v, uint32_t n) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) v[i] ^= 0xFFFFFFFFu;
 }
+// one thread per zlib stream in device memory: header status, method and trailer (byte loads: any offset)
+static __global__ void zlib_frames_kernel(ZlibFrame *f, uint32_t n) {
+  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  ZlibFrame z = f[i];
+  z.method = 0;
+  z.status = (uint32_t)zlib_header_status(z.src, z.len, &z.method);
+  z.expect = z.status == ZIPC_OK ? zlib_trailer(z.src, z.len) : 0u;
+  f[i] = z;
+}
 
 // One warp per stream (inflate.cu).  All pointers in d_src / d_dst are device addresses.
 static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
@@ -1168,13 +1178,11 @@ int zipc_b200_zlib_decompress_batch(zipc_b200_ctx *ctx, int adler_mode, size_t n
     size_t len = src_len[i];
     body[i] = s; blen[i] = 0;
     if (len && !s) return ZIPC_ERR_INVALID_ARG;
-    if (len < 6) { pre[i] = ZIPC_ERR_CORRUPTED; continue; }
-    unsigned cmf = s[0], flg = s[1];
-    if ((256 * cmf + flg) % 31 != 0) { pre[i] = ZIPC_ERR_CORRUPTED; continue; }
-    if ((cmf & 0x0F) != 8) { pre[i] = ZIPC_ERR_ZLIB_METHOD; if (found) found[i] = cmf & 0x0F; continue; }
-    if ((cmf >> 4) > 7) { pre[i] = ZIPC_ERR_ZLIB_WINDOW; continue; }
-    if (flg & 0x20) { pre[i] = ZIPC_ERR_ZLIB_DICT; continue; }
-    exp[i] = (uint32_t)s[len - 4] << 24 | (uint32_t)s[len - 3] << 16 | (uint32_t)s[len - 2] << 8 | s[len - 1];
+    uint32_t method = 0;
+    pre[i] = zlib_header_status(s, len, &method);
+    if (pre[i] == ZIPC_ERR_ZLIB_METHOD && found) found[i] = method;
+    if (pre[i]) continue;
+    exp[i] = zlib_trailer(s, len);
     body[i] = s + 2;
     blen[i] = len - 4;  // as the reference: two bytes into the trailer (zipc_deflate.ml:732)
   }
@@ -1193,6 +1201,67 @@ int zipc_b200_zlib_decompress_batch(zipc_b200_ctx *ctx, int adler_mode, size_t n
     }
   }
   return rc;
+}
+
+int zipc_b200_zlib_decompress_batch_dev(zipc_b200_ctx *ctx, int adler_mode, size_t n, const void *d_src_v, const size_t *src_off,
+                                        const size_t *src_len, void *d_dst_v, const size_t *dst_off, const size_t *max_out,
+                                        size_t *dst_len, uint32_t *expect, uint32_t *found, int *status) {
+  if (!ctx || (adler_mode != ZIPC_ADLER_REF_COMPAT && adler_mode != ZIPC_ADLER_RFC1950) ||
+      (n && (!d_src_v || !src_off || !src_len || !d_dst_v || !dst_off || !max_out || !dst_len || !status)))
+    return ZIPC_ERR_INVALID_ARG;
+  if (!n) return ZIPC_OK;
+  if (n > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
+  for (size_t i = 0; i < n; i++) if (max_out[i] == ZIPC_SIZE_UNKNOWN) return ZIPC_ERR_INVALID_ARG;
+  DeviceGuard g(ctx->device);
+  ctx->epoch++;  // the caller's device bytes may have changed since the last call
+  // headers and trailers are read on the device, by one thread per stream, and come back in one copy
+  if (int st = ctx->h_res.reserve(n * sizeof(ZlibFrame))) return st;
+  if (int st = ctx->d_desc2.reserve(n * sizeof(ZlibFrame))) return st;
+  ZlibFrame *hf = ctx->h_res.as<ZlibFrame>(), *df = ctx->d_desc2.as<ZlibFrame>();
+  for (size_t i = 0; i < n; i++) hf[i] = ZlibFrame{static_cast<const uint8_t *>(d_src_v) + src_off[i], src_len[i], 0, 0, 0, 0};
+  ZB_CUDA(ctx, cudaMemcpyAsync(df, hf, n * sizeof(ZlibFrame), cudaMemcpyHostToDevice, ctx->stream));
+  zlib_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(df, (uint32_t)n);
+  ctx->launches++;
+  ZB_CUDA(ctx, cudaGetLastError());
+  ZB_CUDA(ctx, cudaMemcpyAsync(hf, df, n * sizeof(ZlibFrame), cudaMemcpyDeviceToHost, ctx->stream));
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
+  // streams with a bad header get their status here and are not decoded (their slots stay untouched); the others' bodies are
+  // [2, len - 2), as in the reference (zipc_deflate.ml:732)
+  std::vector<uint32_t> idx, exp;
+  std::vector<const uint8_t *> body;
+  std::vector<uint8_t *> d_dst;
+  std::vector<size_t> blen, cap;
+  for (size_t i = 0; i < n; i++) {
+    const ZlibFrame &f = hf[i];
+    if (f.status != ZIPC_OK) {
+      status[i] = (int)f.status;
+      dst_len[i] = 0;
+      if (f.status == ZIPC_ERR_ZLIB_METHOD && found) found[i] = f.method;
+      continue;
+    }
+    idx.push_back((uint32_t)i);
+    exp.push_back(f.expect);
+    body.push_back(f.src + 2);
+    blen.push_back((size_t)f.len - 4);
+    d_dst.push_back(static_cast<uint8_t *>(d_dst_v) + dst_off[i]);
+    cap.push_back(max_out[i]);
+  }
+  const size_t k = idx.size();
+  std::vector<size_t> ol(k);
+  std::vector<uint32_t> ad(k);
+  std::vector<int> st(k);
+  if (int rc = inflate_core(ctx, ZIPC_CK_ADLER32, adler_mode, k, body, blen.data(), d_dst, cap, false, ol.data(), ad.data(), st.data()))
+    return rc;
+  for (size_t j = 0; j < k; j++) {
+    const uint32_t i = idx[j];
+    status[i] = st[j];
+    dst_len[i] = ol[j];
+    if (st[j] != ZIPC_OK) continue;
+    if (expect) expect[i] = exp[j];
+    if (found) found[i] = ad[j];
+    if (ad[j] != exp[j]) status[i] = ZIPC_ERR_CHECKSUM;
+  }
+  return ZIPC_OK;
 }
 
 }  // extern "C"

@@ -135,6 +135,31 @@ struct CopyDesc {     // gather: len bytes from src to dst
   uint64_t len;
 };
 
+// ---- zlib framing (RFC 1950) -------------------------------------------------------------------
+// The header checks of zlib_decompress in the reference's order (zipc_deflate.ml:722-731): ZIPC_OK or the stream's status;
+// *method receives CM on ZIPC_ERR_ZLIB_METHOD (the "%d" of the message).  s holds len bytes (host or device memory).
+__host__ __device__ inline int zlib_header_status(const uint8_t *s, uint64_t len, uint32_t *method) {
+  if (len < 6) return ZIPC_ERR_CORRUPTED;
+  const uint32_t cmf = s[0], flg = s[1];
+  if ((256 * cmf + flg) % 31 != 0) return ZIPC_ERR_CORRUPTED;
+  if ((cmf & 0x0F) != 8) { *method = cmf & 0x0F; return ZIPC_ERR_ZLIB_METHOD; }
+  if ((cmf >> 4) > 7) return ZIPC_ERR_ZLIB_WINDOW;
+  if (flg & 0x20) return ZIPC_ERR_ZLIB_DICT;
+  return ZIPC_OK;
+}
+// the big-endian Adler-32 in the last 4 of len >= 4 bytes
+__host__ __device__ inline uint32_t zlib_trailer(const uint8_t *s, uint64_t len) {
+  return (uint32_t)s[len - 4] << 24 | (uint32_t)s[len - 3] << 16 | (uint32_t)s[len - 2] << 8 | s[len - 1];
+}
+struct ZlibFrame {    // one stream of zipc_b200_zlib_decompress_batch_dev: the host fills src / len, zlib_frames_kernel the rest
+  const uint8_t *src;
+  uint64_t len;
+  uint32_t status;    // zlib_header_status
+  uint32_t method;    // CM when status is ZIPC_ERR_ZLIB_METHOD
+  uint32_t expect;    // the trailer when status is ZIPC_OK
+  uint32_t _pad;
+};
+
 }  // namespace zb
 
 // ---- the context -------------------------------------------------------------------------------

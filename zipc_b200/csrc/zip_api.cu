@@ -3,7 +3,7 @@
 //
 //   zipc_b200_deflate_batch        <- Zipc_deflate.deflate / crc_32_and_deflate / adler_32_and_deflate
 //                                     (reference src/zipc_deflate.ml:1247-1259)
-//   zipc_b200_zlib_compress_batch  <- Zipc_deflate.zlib_compress (:1262-1277)
+//   zipc_b200_zlib_compress_batch  <- Zipc_deflate.zlib_compress (:1262-1277); _dev: inputs and outputs in device memory
 //   zipc_b200_zip_extract_batch    <- Zipc.File.to_binary_string over parsed members (src/zipc.ml:205-225)
 //   zipc_b200_zip_deflate_archive  <- Zipc.File.deflate_of_binary_string + Zipc.to_binary_string
 //                                     (src/zipc.ml:179-185, 570-588)
@@ -294,6 +294,36 @@ int compact_pieces(zipc_b200_ctx *ctx, const Pieces &pc, const std::vector<size_
   return compact(ctx, poff.size(), pc.d_slot, pc.len.data(), poff, total);
 }
 
+// zlib framing of the members deflate_members compressed into pc (reference :1264-1277): 2 header bytes at to[i], the body's
+// pieces behind them, the big-endian Adler-32 behind the body_len[i] bytes of body.  Header, pieces and trailer are placed
+// by one device gather (one descriptor table, one launch) at any alignment of to[i]; a member whose to[i] is null is left out.
+int place_zlib(zipc_b200_ctx *ctx, int level, size_t n, const Pieces &pc, const size_t *body_len, const uint32_t *adler,
+               const std::vector<uint8_t *> &to) {
+  const size_t np = pc.member.size();
+  const unsigned cmf = 0x78, hdr = (cmf << 8) | ((unsigned)level << 6), flg = (hdr + 31 - hdr % 31) & 0xFF;
+  if (int st = ctx->h_res.reserve(n * 8)) return st;
+  if (int st = ctx->d_res.reserve(n * 8)) return st;
+  if (int st = ctx->h_desc.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
+  if (int st = ctx->d_desc2.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
+  uint8_t *hb = ctx->h_res.as<uint8_t>();
+  uint8_t *db = ctx->d_res.as<uint8_t>();
+  CopyDesc *h = ctx->h_desc.as<CopyDesc>();
+  size_t nd = 0;
+  for (size_t i = 0; i < n; i++) {
+    if (!to[i]) continue;
+    hb[8 * i] = (uint8_t)cmf; hb[8 * i + 1] = (uint8_t)flg;
+    hb[8 * i + 2] = (uint8_t)(adler[i] >> 24); hb[8 * i + 3] = (uint8_t)(adler[i] >> 16);
+    hb[8 * i + 4] = (uint8_t)(adler[i] >> 8); hb[8 * i + 5] = (uint8_t)adler[i];
+    h[nd++] = CopyDesc{db + 8 * i, to[i], 2};
+    h[nd++] = CopyDesc{db + 8 * i + 2, to[i] + 2 + body_len[i], 4};
+  }
+  for (size_t k = 0; k < np; k++)
+    if (to[pc.member[k]]) h[nd++] = CopyDesc{pc.d_slot[k], to[pc.member[k]] + 2 + pc.rel[k], pc.len[k]};
+  ZB_CUDA(ctx, cudaMemcpyAsync(db, hb, n * 8, cudaMemcpyHostToDevice, ctx->stream));
+  ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, h, nd * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
+  return gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)nd);
+}
+
 }  // namespace
 
 int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaStream_t stream) {
@@ -386,37 +416,55 @@ int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode,
   std::vector<uint32_t> ad(n);
   Pieces pc;  // (a large payload is compressed as primed segments, one CTA each: several pieces per stream)
   if (int st = deflate_members(ctx, level, ZIPC_CK_ADLER32, adler_mode, n, d_src, src_len, dst_len, ad.data(), status, pc)) return st;
-  const size_t np = pc.member.size();
-  // framing: 2 header bytes, body, big-endian Adler-32 (reference :1264-1277).  Header and trailer bytes are placed
-  // by the same device gather as the bodies (one descriptor table, one launch), so fetch() sees complete streams.
+  // framed streams in ctx->d_out, so that fetch() sees complete streams
   std::vector<size_t> off(n), flen(n);
   size_t total = 0;
   for (size_t i = 0; i < n; i++) { off[i] = total; flen[i] = dst_len[i] + 6; total += align_up(flen[i], 16); }
   if (int st = ctx->d_out.reserve(total + 64)) return st;
-  {
-    const unsigned cmf = 0x78, hdr = (cmf << 8) | ((unsigned)level << 6), flg = (hdr + 31 - hdr % 31) & 0xFF;
-    if (int st = ctx->h_res.reserve(n * 8)) return st;
-    if (int st = ctx->d_res.reserve(n * 8)) return st;
-    if (int st = ctx->h_desc.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
-    if (int st = ctx->d_desc2.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
-    uint8_t *hb = ctx->h_res.as<uint8_t>();
-    uint8_t *db = ctx->d_res.as<uint8_t>(), *dout = ctx->d_out.as<uint8_t>();
-    CopyDesc *h = ctx->h_desc.as<CopyDesc>();
-    for (size_t i = 0; i < n; i++) {
-      hb[8 * i] = (uint8_t)cmf; hb[8 * i + 1] = (uint8_t)flg;
-      hb[8 * i + 2] = (uint8_t)(ad[i] >> 24); hb[8 * i + 3] = (uint8_t)(ad[i] >> 16);
-      hb[8 * i + 4] = (uint8_t)(ad[i] >> 8); hb[8 * i + 5] = (uint8_t)ad[i];
-      h[2 * i] = CopyDesc{db + 8 * i, dout + off[i], 2};
-      h[2 * i + 1] = CopyDesc{db + 8 * i + 2, dout + off[i] + 2 + dst_len[i], 4};
-    }
-    for (size_t k = 0; k < np; k++) h[2 * n + k] = CopyDesc{pc.d_slot[k], dout + off[pc.member[k]] + 2 + pc.rel[k], pc.len[k]};
-    ZB_CUDA(ctx, cudaMemcpyAsync(db, hb, n * 8, cudaMemcpyHostToDevice, ctx->stream));
-    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, h, (2 * n + np) * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
-    if (int st = gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)(2 * n + np))) return st;
-  }
+  std::vector<uint8_t *> to(n);
+  for (size_t i = 0; i < n; i++) to[i] = ctx->d_out.as<uint8_t>() + off[i];
+  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), to)) return st;
   for (size_t i = 0; i < n; i++) { dst_len[i] = flen[i]; if (adler) adler[i] = ad[i]; }
   return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
 }
+
+int zipc_b200_zlib_compress_batch_dev(zipc_b200_ctx *ctx, int level, int adler_mode, size_t n, const void *d_src_v,
+                                      const size_t *src_off, const size_t *src_len, void *d_dst_v, const size_t *dst_off,
+                                      const size_t *dst_cap_each, size_t *dst_len, uint32_t *adler, int *status) {
+  if (!ctx || level < 0 || level > 3 || (adler_mode != ZIPC_ADLER_REF_COMPAT && adler_mode != ZIPC_ADLER_RFC1950) ||
+      (n && (!d_src_v || !src_off || !src_len || !d_dst_v || !dst_off || !dst_cap_each || !dst_len || !status)))
+    return ZIPC_ERR_INVALID_ARG;
+  if (!n) return ZIPC_OK;
+  DeviceGuard g(ctx->device);
+  std::vector<const uint8_t *> d_src(n);
+  for (size_t i = 0; i < n; i++) d_src[i] = static_cast<const uint8_t *>(d_src_v) + src_off[i];
+  std::vector<uint32_t> ad(n);
+  Pieces pc;  // compressed into the library's slots as by zipc_b200_zlib_compress_batch: same pieces, same bytes
+  if (int st = deflate_members(ctx, level, ZIPC_CK_ADLER32, adler_mode, n, d_src, src_len, dst_len, ad.data(), status, pc)) return st;
+  // a stream goes to its slot only if all of it fits: a slot too small is not written at all
+  std::vector<uint8_t *> to(n, nullptr);
+  for (size_t i = 0; i < n; i++) {
+    if (status[i] == ZIPC_OK && (dst_cap_each[i] < 6 || dst_len[i] > dst_cap_each[i] - 6)) status[i] = ZIPC_ERR_DST_TOO_SMALL;
+    if (status[i] == ZIPC_OK) to[i] = static_cast<uint8_t *>(d_dst_v) + dst_off[i];
+  }
+  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), to)) return st;
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (the gather reads the pinned descriptor table: it must be through before the next call)
+  for (size_t i = 0; i < n; i++) {
+    dst_len[i] = to[i] ? dst_len[i] + 6 : 0;
+    if (adler) adler[i] = to[i] ? ad[i] : 0u;
+  }
+  return ZIPC_OK;
+}
+
+// A member below the split threshold is one deflate stream of at most zipc_b200_deflate_bound(L) bytes.  A split member
+// (deflate_members) is cut into nseg <= L / 65536 + 1 segments: every segment but the last has at least kSplitSegmentMin =
+// 64 KiB.  The encoder closes a block every 61440 source bytes of a segment and never emits a block larger than its stored
+// form (3 header bits, at most 7 padding bits, LEN / NLEN, the bytes: 42 bits over the source), and every segment but the
+// last ends with an empty stored block (at most 42 bits).  A segment of l bytes has at most l / 61440 + 1 blocks, so all
+// segments together have at most L / 61440 + nseg blocks and nseg - 1 empty stored blocks, and the body is at most
+//   L + 6 (L / 61440 + 2 nseg) + 1  <=  L + 6 (L / 61440 + 2) + 12 (L / 65536) + 1  <=  deflate_bound(L) + 12 (L / 65536)
+// bytes, 2 + 4 framing bytes around it.  (Level none is never split: stored blocks of 65534 bytes, within deflate_bound.)
+size_t zipc_b200_zlib_bound(size_t src_len) { return zipc_b200_deflate_bound(src_len) + 12 * (src_len / kSplitSegmentMin) + 6; }
 
 // ---- segmented single stream -----------------------------------------------------------------------------
 static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size_t len, size_t segment_size,
