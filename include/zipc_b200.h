@@ -320,6 +320,29 @@ int zipc_b200_zip_assemble_ex(const zipc_b200_member *members, size_t n, const c
 int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *members, size_t n,
                                 void *dst, size_t dst_cap, size_t *dst_need,
                                 size_t *dst_off, size_t *dst_len, uint32_t *found, int *status);
+/* Device-resident Zipc.of_binary_string (zipc.ml:400-438): the archive is the len bytes at d_bytes in device memory.
+ * Returns what zipc_b200_zip_parse_ex returns for the same bytes and flags: the same status, the same members in the same
+ * order (sorted by path, a later duplicate winning) and the same field values, with two differences:
+ *   - compressed_bytes is d_bytes, a DEVICE pointer: the payload of a member is at compressed_bytes + start on the device;
+ *   - path points into a host copy of the central directory.
+ * That copy and the member array are one allocation: free both with one zipc_b200_free(*members).  The call copies only the
+ * last 65,577 bytes (EOCD search), the ZIP64 end record if there is one, and the central directory to the host, and reads
+ * all local headers with one kernel, however many members there are.  len < 22: ZIPC_ERR_ZIP_SHORT, nothing is read.
+ * Members from this call go to zipc_b200_zip_extract_batch_dev only, never to the host-pointer calls. */
+int zipc_b200_zip_parse_dev(zipc_b200_ctx *ctx, const void *d_bytes, size_t len, unsigned flags,
+                            zipc_b200_member **members, size_t *n);
+/* Device-resident Zipc.File.to_binary_string (zipc.ml:205-225) over parsed members: members[i].compressed_bytes + start must
+ * be device memory on the ctx's device (members of zipc_b200_zip_parse_dev, or built by the caller, from one archive or
+ * several); a member whose compressed_bytes is not (host members passed by mistake) makes the call return
+ * ZIPC_ERR_INVALID_ARG before anything runs.  Output i goes to d_dst + dst_off[i], any alignment; its slot holds
+ * decompressed_size bytes for a deflate member and compressed_size bytes for a stored one.  Nothing is written for
+ * directories, encrypted members and unsupported methods.  status / dst_len / found are those of zipc_b200_zip_extract_batch
+ * for the same members (found may be NULL).  Output contract of zipc_b200_inflate_batch_dev: on success exactly
+ * [dst_off[i], dst_off[i] + dst_len[i]) is written, on failure writes stay inside the slot, so slots may sit back to back.
+ * The device bytes are read anew by every call.  Stored members are copied and checksummed in one pass over their bytes,
+ * large ones by many warps. */
+int zipc_b200_zip_extract_batch_dev(zipc_b200_ctx *ctx, const zipc_b200_member *members, size_t n,
+                                    void *d_dst, const size_t *dst_off, size_t *dst_len, uint32_t *found, int *status);
 /* Batch form of Zipc.File.deflate_of_binary_string (zipc.ml:179-185) followed by
  * Zipc.to_binary_string: compress n payloads on the GPU at `level` and emit one archive.
  * paths are normalised as Member.make does (zipc.ml:244-255); mode / mtime may be NULL

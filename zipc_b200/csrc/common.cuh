@@ -82,6 +82,18 @@ inline CrcSeg crc_seg(const uint8_t *ptr, uint64_t len) {  // a whole range, fro
   return s;
 }
 
+// One tile of a stored ZIP member for stored_copy_crc (crc32.cu): a member of L bytes is cut into tiles of kStoredTile bytes
+// (the last one shorter; a member of 0 bytes is one empty tile).
+constexpr uint64_t kStoredTile = 256u << 10;
+struct StoredTile {
+  const uint8_t *src;
+  uint8_t *dst;
+  uint64_t len;
+  uint64_t after;     // bytes of the member after this tile
+  uint32_t member;    // index of the member's CRC word
+  uint32_t init;      // 0xFFFFFFFF for the member's first tile, 0 for the others
+};
+
 struct AdlerSeg {     // one Adler-32 work item: sums over [ptr, ptr+len)
   const uint8_t *ptr;
   uint32_t len;       // <= 5552
@@ -159,6 +171,27 @@ struct ZlibFrame {    // one stream of zipc_b200_zlib_decompress_batch_dev: the 
   uint32_t expect;    // the trailer when status is ZIPC_OK
   uint32_t _pad;
 };
+
+// ---- ZIP archives ------------------------------------------------------------------------------
+// The four fields of a local file header (APPNOTE 4.3.7) the parser checks; off comes from the central directory.
+struct ZipLfh {
+  uint64_t off;
+  uint32_t sig, crc, name_len, extra_len;
+};
+// h: the 30 bytes of a local header (host or device memory, any alignment)
+__host__ __device__ inline void zip_lfh_fields(const uint8_t *h, ZipLfh &f) {
+  f.sig = (uint32_t)h[0] | (uint32_t)h[1] << 8 | (uint32_t)h[2] << 16 | (uint32_t)h[3] << 24;
+  f.crc = (uint32_t)h[14] | (uint32_t)h[15] << 8 | (uint32_t)h[16] << 16 | (uint32_t)h[17] << 24;
+  f.name_len = (uint32_t)h[26] | (uint32_t)h[27] << 8;
+  f.extra_len = (uint32_t)h[28] | (uint32_t)h[29] << 8;
+}
+struct ZipEnd {       // what the end records say
+  uint64_t count, cd_size, cd_start;
+  uint64_t rec64;     // offset of the ZIP64 end record still to read (~0: none)
+};
+// bytes at the end of an archive that zip_find_end may read: the EOCD (22 bytes + a comment of up to 65,535), the ZIP64
+// locator in front of it (20)
+constexpr uint64_t kZipTailWindow = 65535 + 22 + 20;
 
 }  // namespace zb
 
@@ -251,6 +284,11 @@ int crc_tables_upload(zipc_b200_ctx *ctx);
 int crc32_launch_segments(zipc_b200_ctx *ctx, const CrcSeg *d_segs, uint32_t nseg, uint32_t *d_states);
 // whole-buffer CRC-32 (final value, init/xorout applied) into *d_crc
 int crc32_launch_buffer(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len, uint32_t *d_crc);
+// Stored ZIP members: copies len[i] bytes from src[i] to dst[i] (device addresses, any alignment, no overlap) and returns
+// the CRC-32 of each (final value) in crc[i] on the host.  Every source byte is read once and written once, in one kernel
+// whose warps take tiles of kStoredTile bytes.  Exactly [dst[i], dst[i] + len[i]) is written.  The stream is through on return.
+int stored_copy_crc(zipc_b200_ctx *ctx, size_t n, const uint8_t *const *src, uint8_t *const *dst, const uint64_t *len,
+                    uint32_t *crc);
 // adler32.cu
 int adler32_launch_buffer(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len, int mode, uint32_t *h_out);
 // per-range Adler-32 for n ranges given as (ptr,len) on the host; results (final values) to h_out
@@ -334,6 +372,15 @@ int pipeline_deflate_gapped(zipc_b200_mctx *m, int level, size_t n, const void *
 int deflate_batch_layout(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n, const void *const *src, const size_t *src_len,
                          void *dst, size_t dst_cap, size_t *dst_need, size_t *dst_off, size_t *dst_len, uint32_t *checksum, int *status,
                          const uint32_t *gap, size_t align);
+// host_util.cc: the archive parser in pieces (zipc_b200_zip_parse_ex and zipc_b200_zip_parse_dev share them)
+int zip_find_end(const uint8_t *tail, uint64_t tail_at, uint64_t len, unsigned flags, ZipEnd &e);
+int zip_read_end64(const uint8_t *rec, uint64_t len, ZipEnd &e);
+int zip_check_cd_range(uint64_t len, const ZipEnd &e);
+int zip_walk_cd(const uint8_t *cd, uint64_t len, unsigned flags, const ZipEnd &e, std::vector<zipc_b200_member> &ms,
+                std::vector<ZipLfh> &lfh);
+int zip_parse_finish(std::vector<zipc_b200_member> &ms, const std::vector<ZipLfh> &lfh, int cd_status, uint64_t len,
+                     const uint8_t *bytes, const uint8_t *cd, uint64_t cd_size, bool cd_copy, zipc_b200_member **members,
+                     size_t *n_out);
 // host_util.cc
 int zip_assemble_impl(const zipc_b200_member *ms, size_t n, const char *first, void *out_v, size_t out_cap,
                       size_t *out_len, bool copy_payload, uint64_t *payload_off, unsigned flags = 0 /* ZIPC_ZIP_* */);

@@ -21,6 +21,11 @@
 //     multiplication with x^(128*d), d in [0,31], and XOR-reduced over the warp.
 //   * Large buffers: one tile per warp; tile states are merged by a small second kernel with a
 //     Horner + tree scheme over x^(8*L) (crc32_combine_tiles).
+//   * Stored ZIP members (stored_copy_crc_kernel): the same warp loop also writes every 16-byte word it
+//     loaded to the member's output slot, so a payload is read once and written once (2N bytes) while
+//     its CRC-32 is computed.  Members are cut into tiles of kStoredTile bytes, one warp each; every warp
+//     advances its tile's state over the bytes of the member that follow the tile and XORs it into the
+//     member's word.
 //
 // Algorithmic bytes per launch: N (every input byte is read exactly once, nothing is written
 // but 4 bytes per segment).  Roofline: HBM.
@@ -52,7 +57,8 @@ uint32_t gf_xpow8(uint64_t nbytes) {  // x^(8*nbytes) mod P
 //   [0    .. 1023]  strided slice tables  TS[k][b] = T0[b] * x^(8*(k+508))
 //   [1024 .. 2047]  ordinary slice tables T[k][b]  = T0[b] * x^(8*k)
 //   [2048 .. 2079]  XP[m] = x^(128*m)   (advance a state by 16*m bytes)
-constexpr int kTabWords = 1024 + 1024 + 32;
+//   [2080 .. 2143]  X2N[k] = x^(2^k)     (advance a state by any number of bytes: stored_copy_crc_kernel)
+constexpr int kTabWords = 1024 + 1024 + 32 + 64;
 constexpr int kStride = 512;
 
 int crc_tables_upload(zipc_b200_ctx *ctx) {
@@ -71,6 +77,8 @@ int crc_tables_upload(zipc_b200_ctx *ctx) {
     }
   }
   for (int m = 0; m < 32; m++) t[2048 + m] = gf_xpow8(16ull * m);
+  x2n_init();
+  for (int k = 0; k < 64; k++) t[2080 + k] = g_x2n[k];
   ZB_CUDA(ctx, cudaMalloc(&ctx->d_crc_tabs, kTabWords * sizeof(uint32_t)));
   ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_crc_tabs, t.data(), kTabWords * sizeof(uint32_t),
                                cudaMemcpyHostToDevice, ctx->stream));
@@ -120,23 +128,92 @@ __device__ __forceinline__ uint32_t step_byte(const uint32_t *__restrict__ st, u
   return (c >> 8) ^ st[(c ^ b) & 0xffu];
 }
 
-// State after running seg.len bytes from seg.init; result valid in lane 0.
+// What crc_segment_warp does with the bytes it reads besides the CRC: nothing (NoStore), or write them to a destination
+// (CopyStore).  Bytes outside the 16-byte-aligned body go through byte(); the body comes row by row through row(), called by
+// the whole warp in row order, with valid = false for the lanes that have no block in the row.
+struct NoStore {
+  static constexpr bool kStores = false;
+  static constexpr int kRows = 8;   // rows requested together by the main loop
+  __device__ __forceinline__ void begin(uint32_t, uint64_t) {}
+  __device__ __forceinline__ void byte(uint64_t, uint32_t) {}
+  __device__ __forceinline__ void row(const uint4 &, uint64_t, int, bool) {}
+};
+
+__device__ __forceinline__ void st_v4(uint8_t *p, const uint4 &v) { *reinterpret_cast<uint4 *>(p) = v; }
+// bytes [from, to) of v to p[from, to)
+__device__ __forceinline__ void st_bytes(uint8_t *p, const uint4 &v, uint32_t from, uint32_t to) {
+  for (uint32_t i = from; i < to; i++) {
+    const uint32_t w = i < 4 ? v.x : i < 8 ? v.y : i < 12 ? v.z : v.w;
+    p[i] = (uint8_t)(w >> (8 * (i & 3)));
+  }
+}
+
+// The body's blocks land at dst + head + 16 b, i.e. at phase p of the destination's 16-byte words: aligned word b (at
+// dbase + 16 b) holds the last p bytes of block b - 1 and the first 16 - p bytes of block b.  Lane l takes block b - 1 from
+// lane l - 1 by shuffle, lane 0 from the previous row's lane 31 (the carry), and stores word b whole; word 0 and word nblk
+// are the partial ends of the body.  Every store lies inside [dst, dst + len): no byte outside the slot is written.
+struct CopyStore {
+  static constexpr bool kStores = true;
+  static constexpr int kRows = 4;   // (8 rows of loads in flight and the row being joined do not fit 64 registers)
+  uint8_t *dst;       // destination of the segment's byte 0
+  uint8_t *dbase;     // 16-byte aligned: dst + head - p
+  uint64_t nblk;
+  uint32_t p, q, sh;  // phase; the shift 16 - p as whole words (q) and bits (sh)
+  uint4 carry;
+  __device__ __forceinline__ explicit CopyStore(uint8_t *d) : dst(d) {}
+  __device__ __forceinline__ void begin(uint32_t head, uint64_t nb) {
+    p = (uint32_t)((uintptr_t)(dst + head) & 15);
+    dbase = dst + head - p;
+    nblk = nb;
+    q = ((16 - p) >> 2) & 3;
+    sh = ((16 - p) & 3) * 8;
+    carry = make_uint4(0, 0, 0, 0);
+  }
+  __device__ __forceinline__ void byte(uint64_t i, uint32_t v) { dst[i] = (uint8_t)v; }
+  // bytes 16 - p .. 15 of a, then bytes 0 .. 15 - p of b
+  __device__ __forceinline__ uint4 join(const uint4 &a, const uint4 &b) const {
+    uint32_t a0 = a.x, a1 = a.y, a2 = a.z, a3 = a.w, a4 = b.x, a5 = b.y, a6 = b.z, a7 = b.w;
+    if (q & 2) { a0 = a2; a1 = a3; a2 = a4; a3 = a5; a4 = a6; a5 = a7; }
+    if (q & 1) { a0 = a1; a1 = a2; a2 = a3; a3 = a4; a4 = a5; }
+    return make_uint4(__funnelshift_r(a0, a1, sh), __funnelshift_r(a1, a2, sh), __funnelshift_r(a2, a3, sh),
+                      __funnelshift_r(a3, a4, sh));
+  }
+  __device__ __forceinline__ void row(const uint4 &cur, uint64_t r, int lane, bool valid) {
+    const int from = (lane + 31) & 31;
+    uint4 prev = make_uint4(__shfl_sync(0xffffffffu, cur.x, from), __shfl_sync(0xffffffffu, cur.y, from),
+                            __shfl_sync(0xffffffffu, cur.z, from), __shfl_sync(0xffffffffu, cur.w, from));
+    const uint4 t = prev;
+    if (lane == 0) prev = carry;
+    carry = t;
+    if (!valid) return;
+    const uint64_t b = 32 * r + (uint64_t)lane;
+    uint8_t *w = dbase + 16 * b;
+    if (p == 0) { st_v4(w, cur); return; }
+    const uint4 o = join(prev, cur);
+    if (b) st_v4(w, o);
+    else st_bytes(w, o, p, 16);
+    if (b + 1 == nblk) st_bytes(w + 16, join(cur, cur), 0, p);
+  }
+};
+
+// State after running seg.len bytes from seg.init; result valid in lane 0.  The sink sees every byte once (see NoStore).
+template <class Sink>
 __device__ uint32_t crc_segment_warp(const CrcSeg seg, int lane, const uint32_t *__restrict__ rep,
-                                     const uint32_t *__restrict__ st, const uint32_t *__restrict__ xp) {
+                                     const uint32_t *__restrict__ st, const uint32_t *__restrict__ xp, Sink &sink) {
   const uint8_t *ptr = seg.ptr;
   uint64_t len = seg.len;
   const uint32_t lane4 = (uint32_t)lane * 4u;
   if (len < 64) {  // tiny: one lane, bytewise
     uint32_t c = seg.init;
     if (lane == 0)
-      for (uint32_t i = 0; i < (uint32_t)len; i++) c = step_byte(st, c, ptr[i]);
+      for (uint32_t i = 0; i < (uint32_t)len; i++) { const uint32_t v = ptr[i]; c = step_byte(st, c, v); sink.byte(i, v); }
     return c;
   }
   uint32_t head = (uint32_t)((16 - ((uintptr_t)ptr & 15)) & 15);
   uint32_t c0 = 0, c1 = 0, c2 = 0, c3 = 0;
   if (lane == 0) {  // unaligned head, then the running state is folded into the first body word
     uint32_t c = seg.init;
-    for (uint32_t i = 0; i < head; i++) c = step_byte(st, c, ptr[i]);
+    for (uint32_t i = 0; i < head; i++) { const uint32_t v = ptr[i]; c = step_byte(st, c, v); sink.byte(i, v); }
     c0 = c;
   }
   const uint8_t *body = ptr + head;
@@ -146,22 +223,25 @@ __device__ uint32_t crc_segment_warp(const CrcSeg seg, int lane, const uint32_t 
   uint64_t rows = nblk >> 5;
   int k = (int)(nblk & 31);                // lanes < k own one more block
   const uint4 *p = reinterpret_cast<const uint4 *>(body) + lane;
+  sink.begin(head, nblk);
 
   // rows [0, rows-1): nobody's last block -> strided tables for every lane
   // 8 rows (4 KiB per warp) are requested together, then consumed; with 32 warps per SM out of phase this keeps
   // enough loads in flight (a software-pipelined variant measured the same: the LDS pipe, ~75 % busy, is the
   // next limiter after HBM, not load latency).
   uint64_t R = rows > 0 ? rows - 1 : 0, r = 0;
-  for (; r + 8 <= R; r += 8) {
-    uint4 w[8];
+  constexpr int G = Sink::kRows;
+  for (; r + G <= R; r += G) {
+    uint4 w[G];
 #pragma unroll
-    for (int j = 0; j < 8; j++) w[j] = ldg_stream(p + 32 * (r + j));
+    for (int j = 0; j < G; j++) w[j] = ldg_stream(p + 32 * (r + j));
 #pragma unroll
-    for (int j = 0; j < 8; j++) {
+    for (int j = 0; j < G; j++) {
       c0 = step_rep(rep, lane4, c0 ^ w[j].x);
       c1 = step_rep(rep, lane4, c1 ^ w[j].y);
       c2 = step_rep(rep, lane4, c2 ^ w[j].z);
       c3 = step_rep(rep, lane4, c3 ^ w[j].w);
+      sink.row(w[j], r + j, lane, true);
     }
   }
   for (; r < R; r++) {
@@ -170,11 +250,13 @@ __device__ uint32_t crc_segment_warp(const CrcSeg seg, int lane, const uint32_t 
     c1 = step_rep(rep, lane4, c1 ^ w.y);
     c2 = step_rep(rep, lane4, c2 ^ w.z);
     c3 = step_rep(rep, lane4, c3 ^ w.w);
+    sink.row(w, r, lane, true);
   }
   bool has = false;
   if (rows >= 1) {  // row rows-1: last block of lanes >= k
     uint4 w = ldg_stream(p + 32 * (rows - 1));
     has = true;
+    sink.row(w, rows - 1, lane, true);
     if (lane < k) {
       c0 = step_rep(rep, lane4, c0 ^ w.x); c1 = step_rep(rep, lane4, c1 ^ w.y);
       c2 = step_rep(rep, lane4, c2 ^ w.z); c3 = step_rep(rep, lane4, c3 ^ w.w);
@@ -183,7 +265,17 @@ __device__ uint32_t crc_segment_warp(const CrcSeg seg, int lane, const uint32_t 
       c2 = step_std(st, c2 ^ w.z); c3 = step_std(st, c3 ^ w.w);
     }
   }
-  if (lane < k) {  // partial row: last block of lanes < k
+  if constexpr (Sink::kStores) {
+    if (k) {  // partial row: last block of lanes < k (the whole warp takes part in the sink's shuffle)
+      const uint4 w = lane < k ? ldg_stream(p + 32 * rows) : make_uint4(0, 0, 0, 0);
+      sink.row(w, rows, lane, lane < k);
+      if (lane < k) {
+        has = true;
+        c0 = step_std(st, c0 ^ w.x); c1 = step_std(st, c1 ^ w.y);
+        c2 = step_std(st, c2 ^ w.z); c3 = step_std(st, c3 ^ w.w);
+      }
+    }
+  } else if (lane < k) {  // partial row: last block of lanes < k
     uint4 w = ldg_stream(p + 32 * rows);
     has = true;
     c0 = step_std(st, c0 ^ w.x); c1 = step_std(st, c1 ^ w.y);
@@ -203,7 +295,7 @@ __device__ uint32_t crc_segment_warp(const CrcSeg seg, int lane, const uint32_t 
   for (int o = 16; o > 0; o >>= 1) s ^= __shfl_xor_sync(0xffffffffu, s, o);
   if (lane == 0) {
     const uint8_t *t = body + (nblk << 4);
-    for (uint32_t i = 0; i < tail; i++) s = step_byte(st, s, t[i]);
+    for (uint32_t i = 0; i < tail; i++) { const uint32_t v = t[i]; s = step_byte(st, s, v); sink.byte(head + (nblk << 4) + i, v); }
   }
   return s;
 }
@@ -238,7 +330,8 @@ crc32_segments_kernel(const CrcSeg *__restrict__ segs, uint32_t nseg, const uint
     if (lane == 0) s = atomicAdd(queue, 1u);
     s = __shfl_sync(0xffffffffu, s, 0);
     if (s >= nseg) break;
-    uint32_t c = crc_segment_warp(segs[s], lane, rep, st, xp);
+    NoStore none;
+    uint32_t c = crc_segment_warp(segs[s], lane, rep, st, xp, none);
     if (lane == 0) states[s] = c;
   }
 }
@@ -258,7 +351,8 @@ crc32_tiles_kernel(const uint8_t *__restrict__ src, uint64_t len, uint64_t tile,
     seg.ptr = src + off;
     seg.len = len - off < tile ? len - off : tile;
     seg.init = t == 0 ? 0xFFFFFFFFu : 0u;
-    uint32_t c = crc_segment_warp(seg, lane, rep, st, xp);
+    NoStore none;
+    uint32_t c = crc_segment_warp(seg, lane, rep, st, xp, none);
     if (lane == 0) states[t] = c;
   }
 }
@@ -296,6 +390,37 @@ crc32_combine_tiles_kernel(const uint32_t *__restrict__ states, uint32_t F, uint
   if (q == 0) *out = (gf_mul(v[0], xl) ^ states[F]) ^ 0xFFFFFFFFu;
 }
 
+// Stored members: tile t of the launch copies tiles[t].len bytes from src to dst and XORs its state, advanced over the
+// tiles[t].after bytes of its member that follow it, into acc[tiles[t].member] (zeroed before the launch).  A member's first
+// tile starts from the CRC init value, so acc ends as the member's state before the final XOR.  Tiles pulled from a queue.
+constexpr size_t kCopySmemBytes = kSmemBytes + 64 * sizeof(uint32_t);
+__global__ void __launch_bounds__(kThreads, 1)
+stored_copy_crc_kernel(const StoredTile *__restrict__ tiles, uint32_t ntiles, const uint32_t *__restrict__ g_tabs,
+                       uint32_t *__restrict__ acc, unsigned int *__restrict__ queue) {
+  extern __shared__ __align__(16) uint32_t smem[];
+  if (threadIdx.x < 64) smem[kRepWords + 1024 + 32 + threadIdx.x] = g_tabs[2080 + threadIdx.x];  // (load_tables syncs)
+  load_tables(g_tabs, smem);
+  const int lane = threadIdx.x & 31;
+  const uint32_t *rep = smem, *st = smem + kRepWords, *xp = st + 1024, *x2n = xp + 32;
+  for (;;) {
+    unsigned int t = 0;
+    if (lane == 0) t = atomicAdd(queue, 1u);
+    t = __shfl_sync(0xffffffffu, t, 0);
+    if (t >= ntiles) break;
+    const StoredTile d = tiles[t];
+    CopyStore sink(d.dst);
+    uint32_t c = crc_segment_warp(CrcSeg{d.src, d.len, d.init, 0}, lane, rep, st, xp, sink);
+    if (d.after) {  // times x^(8 after): bit i of `after` contributes x^(2^(i+3)); lane l takes bits l and l + 32
+      uint32_t f = (d.after >> lane) & 1 ? x2n[lane + 3] : 0x80000000u;
+      if (d.after >> 32 && lane < 29 && (d.after >> (lane + 32)) & 1) f = gf_mul(f, x2n[lane + 35]);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) f = gf_mul(f, __shfl_xor_sync(0xffffffffu, f, o));
+      c = gf_mul(c, f);
+    }
+    if (lane == 0) atomicXor(acc + d.member, c);
+  }
+}
+
 unsigned long long g_attr_devs = 0;  // bit d: attributes set on device d (function attributes are per device)
 int ensure_attrs(zipc_b200_ctx *ctx) {
   if (g_attr_devs >> (ctx->device & 63) & 1ull) return ZIPC_OK;
@@ -303,6 +428,8 @@ int ensure_attrs(zipc_b200_ctx *ctx) {
                                     (int)kSmemBytes));
   ZB_CUDA(ctx, cudaFuncSetAttribute(crc32_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)kSmemBytes));
+  ZB_CUDA(ctx, cudaFuncSetAttribute(stored_copy_crc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)kCopySmemBytes));
   g_attr_devs |= 1ull << (ctx->device & 63);
   return ZIPC_OK;
 }
@@ -354,6 +481,49 @@ int crc32_launch_buffer(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t len, 
   crc32_combine_tiles_kernel<<<1, kCombThreads, 0, ctx->stream>>>(d_states, F, G, gf_xpow8(last_len), cc, d_crc);
   ctx->launches++;
   ZB_CUDA(ctx, cudaGetLastError());
+  return ZIPC_OK;
+}
+
+int stored_copy_crc(zipc_b200_ctx *ctx, size_t n, const uint8_t *const *src, uint8_t *const *dst, const uint64_t *len,
+                    uint32_t *crc) {
+  if (!n) return ZIPC_OK;
+  if (n > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
+  size_t ntiles = 0;
+  for (size_t i = 0; i < n; i++) ntiles += len[i] ? (len[i] + kStoredTile - 1) / kStoredTile : 1;
+  if (ntiles > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
+  if (int st = ensure_attrs(ctx)) return st;
+  const size_t tile_bytes = ntiles * sizeof(StoredTile);
+  if (int st = ctx->h_desc.reserve(tile_bytes + n * sizeof(uint32_t))) return st;
+  if (int st = ctx->d_desc2.reserve(tile_bytes + n * sizeof(uint32_t))) return st;
+  if (int st = ctx->d_small.reserve(256)) return st;
+  StoredTile *ht = ctx->h_desc.as<StoredTile>();
+  size_t t = 0;
+  for (size_t i = 0; i < n; i++) {  // (a zero-length member is one empty tile: its word ends as the init value)
+    uint64_t off = 0;
+    do {
+      const uint64_t l = len[i] - off < kStoredTile ? len[i] - off : kStoredTile;
+      ht[t++] = StoredTile{src[i] + off, dst[i] + off, l, len[i] - off - l, (uint32_t)i, off ? 0u : 0xFFFFFFFFu};
+      off += l;
+    } while (off < len[i]);
+  }
+  StoredTile *dt = ctx->d_desc2.as<StoredTile>();
+  uint32_t *d_acc = reinterpret_cast<uint32_t *>(ctx->d_desc2.as<uint8_t>() + tile_bytes);
+  unsigned int *queue = ctx->d_small.as<unsigned int>();
+  ZB_CUDA(ctx, cudaMemcpyAsync(dt, ht, tile_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  ZB_CUDA(ctx, cudaMemsetAsync(d_acc, 0, n * sizeof(uint32_t), ctx->stream));
+  ZB_CUDA(ctx, cudaMemsetAsync(queue, 0, sizeof(unsigned int), ctx->stream));
+  uint32_t grid = (uint32_t)((ntiles + kWarps - 1) / kWarps);
+  if (grid > (uint32_t)ctx->sm_count) grid = (uint32_t)ctx->sm_count;
+  {
+    KernelTimer kt(ctx);
+    stored_copy_crc_kernel<<<grid, kThreads, kCopySmemBytes, ctx->stream>>>(dt, (uint32_t)ntiles, ctx->d_crc_tabs, d_acc, queue);
+  }
+  ctx->launches++;
+  ZB_CUDA(ctx, cudaGetLastError());
+  uint32_t *h_acc = reinterpret_cast<uint32_t *>(ctx->h_desc.as<uint8_t>() + tile_bytes);
+  ZB_CUDA(ctx, cudaMemcpyAsync(h_acc, d_acc, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
+  for (size_t i = 0; i < n; i++) crc[i] = h_acc[i] ^ 0xFFFFFFFFu;
   return ZIPC_OK;
 }
 

@@ -9,10 +9,9 @@
 #include <string>
 #include <vector>
 
-#include "../../include/zipc_b200.h"
+#include "common.cuh"
 
 namespace zb {
-uint32_t gf_xpow8(uint64_t nbytes);
 uint32_t gf_mul_host(uint32_t a, uint32_t b);
 }  // namespace zb
 
@@ -156,49 +155,74 @@ static bool zip64_cd_extra(const uint8_t *x, size_t xlen, uint64_t &usize, uint6
 }
 
 // ---- Zipc.of_binary_string (zipc.ml:400-438) ------------------------------------------------------
-int zipc_b200_zip_parse(const void *bytes, size_t len, zipc_b200_member **members, size_t *n_out) {
-  return zipc_b200_zip_parse_ex(bytes, len, ZIPC_ZIP_REFERENCE, members, n_out);
-}
+// One parser for host and device bytes.  It looks at an archive through the few pieces it needs: the window at the end
+// where the EOCD is searched, the ZIP64 end record, the central directory, and four fields of each member's local header.
+// zipc_b200_zip_parse_ex finds them all in host memory; zipc_b200_zip_parse_dev (zip_api.cu) copies the first three from
+// device memory and reads the local headers with one kernel.  The checks are made in the sequential parser's order: member
+// k's local header is checked before member k + 1's directory entry.
+}  // extern "C"
 
-// flags = ZIPC_ZIP_REFERENCE: the reference's behaviour (ZIP64 rejected, zipc.ml:404).  ZIPC_ZIP_ALLOW_ZIP64 (SURVEY.md
-// 8f-4, beyond the reference): a ZIP64 end of central directory locator in front of the EOCD is followed, and central
-// directory entries take their 64-bit sizes / offsets from the ZIP64 extra field.
-int zipc_b200_zip_parse_ex(const void *bytes, size_t len, unsigned flags, zipc_b200_member **members, size_t *n_out) {
-  if (!members || !n_out || (!bytes && len)) return ZIPC_ERR_INVALID_ARG;
+namespace zb {
+
+// The end of central directory record, searched in tail = bytes [tail_at, len) (zipc.ml:415-425).  tail_at must be at most
+// len - kZipTailWindow (or 0).  A ZIP64 end record to read next is reported in e.rec64 (else ~0).
+int zip_find_end(const uint8_t *tail, uint64_t tail_at, uint64_t len, unsigned flags, ZipEnd &e) {
   const bool z64 = (flags & ZIPC_ZIP_ALLOW_ZIP64) != 0;
-  *members = nullptr;
-  *n_out = 0;
-  const uint8_t *s = static_cast<const uint8_t *>(bytes);
-  // end of central directory: first signature hit scanning backwards (zipc.ml:415-425)
   if (len < 22) return ZIPC_ERR_ZIP_SHORT;
+  auto r16 = [&](uint64_t o) { return rd16(tail, (size_t)(o - tail_at)); };   // (only offsets >= tail_at are read)
+  auto r32 = [&](uint64_t o) { return rd32(tail, (size_t)(o - tail_at)); };
   int64_t at = (int64_t)len - 22, lowest = (int64_t)len - 65535 - 22;
   for (;; at--) {
     if (at < lowest || at < 0) return ZIPC_ERR_ZIP_NO_EOCD;
-    if (rd32(s, (size_t)at) == 0x06054b50u) break;
+    if (r32((uint64_t)at) == 0x06054b50u) break;
   }
-  const size_t e = (size_t)at;
-  size_t count = rd16(s, e + 10);
-  uint64_t cd_size = rd32(s, e + 12), cd_start = rd32(s, e + 16);
-  if (z64 && e >= 20 && rd32(s, e - 20) == 0x07064b50u) {            // ZIP64 EOCD locator (APPNOTE 4.3.15)
-    if (rd32(s, e - 16) != 0 || rd32(s, e - 4) > 1) return ZIPC_ERR_ZIP_MULTIPART;
-    const uint64_t r = rd64(s, e - 12);
-    if (r > len || len - r < 56 || rd32(s, (size_t)r) != 0x06064b50u) return ZIPC_ERR_ZIP_EOCD;
-    if (rd32(s, (size_t)r + 16) != 0 || rd32(s, (size_t)r + 20) != 0) return ZIPC_ERR_ZIP_MULTIPART;
-    if (rd64(s, (size_t)r + 24) != rd64(s, (size_t)r + 32)) return ZIPC_ERR_ZIP_MULTIPART;
-    count = (size_t)rd64(s, (size_t)r + 32);
-    cd_size = rd64(s, (size_t)r + 40);
-    cd_start = rd64(s, (size_t)r + 48);
-    if (cd_size > len || count > cd_size / 46) return ZIPC_ERR_ZIP_EOCD;  // (a count no directory of that size can hold)
-  } else {
-    if (rd16(s, e + 4) == 0xFFFF) return ZIPC_ERR_ZIP_ZIP64;         // zipc.ml:404
-    if (rd16(s, e + 4) != 0 || rd16(s, e + 6) != 0) return ZIPC_ERR_ZIP_MULTIPART;
+  const uint64_t o = (uint64_t)at;
+  e.count = r16(o + 10);
+  e.cd_size = r32(o + 12);
+  e.cd_start = r32(o + 16);
+  e.rec64 = ~0ull;
+  if (z64 && o >= 20 && r32(o - 20) == 0x07064b50u) {               // ZIP64 EOCD locator (APPNOTE 4.3.15)
+    if (r32(o - 16) != 0 || r32(o - 4) > 1) return ZIPC_ERR_ZIP_MULTIPART;
+    const uint64_t r = r32(o - 12) | (uint64_t)r32(o - 8) << 32;
+    if (r > len || len - r < 56) return ZIPC_ERR_ZIP_EOCD;
+    e.rec64 = r;
+    return ZIPC_OK;
   }
-  if (cd_start > len || cd_size > len - cd_start) return ZIPC_ERR_ZIP_EOCD;
-  const int64_t cd_max = (int64_t)(cd_start + cd_size) - 1;
+  if (r16(o + 4) == 0xFFFF) return ZIPC_ERR_ZIP_ZIP64;               // zipc.ml:404
+  if (r16(o + 4) != 0 || r16(o + 6) != 0) return ZIPC_ERR_ZIP_MULTIPART;
+  return zip_check_cd_range(len, e);
+}
 
-  std::vector<zipc_b200_member> ms(count);
-  int64_t i = (int64_t)cd_start;
-  for (size_t k = 0; k < count; k++) {
+// The 56 bytes of the ZIP64 end of central directory record at e.rec64 (APPNOTE 4.3.14).
+int zip_read_end64(const uint8_t *r, uint64_t len, ZipEnd &e) {
+  if (rd32(r, 0) != 0x06064b50u) return ZIPC_ERR_ZIP_EOCD;
+  if (rd32(r, 16) != 0 || rd32(r, 20) != 0) return ZIPC_ERR_ZIP_MULTIPART;
+  if (rd64(r, 24) != rd64(r, 32)) return ZIPC_ERR_ZIP_MULTIPART;
+  e.count = rd64(r, 32);
+  e.cd_size = rd64(r, 40);
+  e.cd_start = rd64(r, 48);
+  if (e.cd_size > len || e.count > e.cd_size / 46) return ZIPC_ERR_ZIP_EOCD;  // (a count no directory of that size can hold)
+  return zip_check_cd_range(len, e);
+}
+
+int zip_check_cd_range(uint64_t len, const ZipEnd &e) {
+  if (e.cd_start > len || e.cd_size > len - e.cd_start) return ZIPC_ERR_ZIP_EOCD;
+  return ZIPC_OK;
+}
+
+// The central directory (cd: its e.cd_size bytes) entry by entry, up to the first error, whose status is returned.  ms / lfh
+// receive the members before it (paths point into cd); lfh[k].off is member k's local header offset (directories: unused).
+int zip_walk_cd(const uint8_t *cd, uint64_t len, unsigned flags, const ZipEnd &e, std::vector<zipc_b200_member> &ms,
+                std::vector<ZipLfh> &lfh) {
+  const bool z64 = (flags & ZIPC_ZIP_ALLOW_ZIP64) != 0;
+  ms.clear();
+  lfh.clear();
+  ms.reserve((size_t)e.count);
+  lfh.reserve((size_t)e.count);
+  const uint8_t *s = cd;
+  const int64_t cd_max = (int64_t)e.cd_size - 1;
+  int64_t i = 0;
+  for (uint64_t k = 0; k < e.count; k++) {
     if (i > cd_max) return ZIPC_ERR_ZIP_TRUNC_CD;                     // zipc.ml:394
     if (i + 45 > cd_max || rd32(s, (size_t)i) != 0x02014b50u) return ZIPC_ERR_ZIP_CDFH;
     const size_t o = (size_t)i;
@@ -214,6 +238,8 @@ int zipc_b200_zip_parse_ex(const void *bytes, size_t len, unsigned flags, zipc_b
     if (hi) { m.is_dir = (hi & 070000) == 040000; m.mode = (int32_t)(hi & 07777); }
     else if (s[o + 38] & 0x10) { m.is_dir = 1; m.mode = 0755; }
     else { m.is_dir = 0; m.mode = 0644; }
+    ZipLfh f;
+    std::memset(&f, 0, sizeof f);
     if (!m.is_dir) {
       m.compression = (int32_t)rd16(s, o + 10);
       m.version_made_by = (int32_t)rd16(s, o + 4);
@@ -222,26 +248,82 @@ int zipc_b200_zip_parse_ex(const void *bytes, size_t len, unsigned flags, zipc_b
       m.compressed_size = rd32(s, o + 20);
       m.decompressed_size = rd32(s, o + 24);
       m.crc32 = rd32(s, o + 16);
-      uint64_t lfh = rd32(s, o + 42);
-      if (z64 && !zip64_cd_extra(s + o + 46 + plen, rd16(s, o + 30), m.decompressed_size, m.compressed_size, lfh)) return ZIPC_ERR_ZIP_CDFH;
-      if (lfh >= len) return ZIPC_ERR_ZIP_CDFH;                       // zipc.ml:380
-      if (lfh + 30 > len || rd32(s, (size_t)lfh) != 0x04034b50u) return ZIPC_ERR_ZIP_LFH;
-      const uint64_t data = lfh + 30 + rd16(s, (size_t)lfh + 26) + rd16(s, (size_t)lfh + 28);
-      if (data > len || m.compressed_size > len - data) return ZIPC_ERR_ZIP_LFH;  // zipc.ml:335
-      if (m.crc32 == 0) m.crc32 = rd32(s, (size_t)lfh + 14);          // zipc.ml:382-385
-      m.compressed_bytes = s;
-      m.start = data;
+      uint64_t off = rd32(s, o + 42);
+      if (z64 && !zip64_cd_extra(s + o + 46 + plen, rd16(s, o + 30), m.decompressed_size, m.compressed_size, off)) return ZIPC_ERR_ZIP_CDFH;
+      if (off >= len) return ZIPC_ERR_ZIP_CDFH;                       // zipc.ml:380
+      f.off = off;
     }
-    ms[k] = m;
+    ms.push_back(m);
+    lfh.push_back(f);
     i = next;
   }
+  return ZIPC_OK;
+}
+
+// The local header checks of the members zip_walk_cd returned, in order, then cd_status (the walk's); on success the members
+// sorted by path, a later duplicate winning, into one allocation.  lfh[k]'s fields are read when lfh[k].off + 30 <= len.
+// Payloads are at `bytes` + start.  With cd_copy, the directory's cd_size bytes are copied behind the members and the paths
+// point there (they pointed into cd).
+int zip_parse_finish(std::vector<zipc_b200_member> &ms, const std::vector<ZipLfh> &lfh, int cd_status, uint64_t len,
+                     const uint8_t *bytes, const uint8_t *cd, uint64_t cd_size, bool cd_copy, zipc_b200_member **members,
+                     size_t *n_out) {
+  for (size_t k = 0; k < ms.size(); k++) {
+    zipc_b200_member &m = ms[k];
+    if (m.is_dir) continue;
+    const ZipLfh &f = lfh[k];
+    if (f.off + 30 > len || f.sig != 0x04034b50u) return ZIPC_ERR_ZIP_LFH;
+    const uint64_t data = f.off + 30 + f.name_len + f.extra_len;
+    if (data > len || m.compressed_size > len - data) return ZIPC_ERR_ZIP_LFH;  // zipc.ml:335
+    if (m.crc32 == 0) m.crc32 = f.crc;                                // zipc.ml:382-385
+    m.compressed_bytes = bytes;
+    m.start = data;
+  }
+  if (cd_status) return cd_status;
   std::vector<size_t> ord = map_order(ms.data(), ms.size());
-  zipc_b200_member *res = static_cast<zipc_b200_member *>(std::malloc(sizeof(zipc_b200_member) * (ord.size() ? ord.size() : 1)));
+  const size_t head = sizeof(zipc_b200_member) * (ord.size() ? ord.size() : 1);
+  zipc_b200_member *res = static_cast<zipc_b200_member *>(std::malloc(head + (cd_copy ? (size_t)cd_size : 0)));
   if (!res) return ZIPC_ERR_NOMEM;
-  for (size_t k = 0; k < ord.size(); k++) res[k] = ms[ord[k]];
+  const char *names = reinterpret_cast<const char *>(cd);
+  if (cd_copy) {
+    char *copy = reinterpret_cast<char *>(res) + head;
+    if (cd_size) std::memcpy(copy, cd, (size_t)cd_size);
+    names = copy;
+  }
+  for (size_t k = 0; k < ord.size(); k++) {
+    res[k] = ms[ord[k]];
+    res[k].path = names + (res[k].path - reinterpret_cast<const char *>(cd));
+  }
   *members = res;
   *n_out = ord.size();
   return ZIPC_OK;
+}
+
+}  // namespace zb
+
+extern "C" {
+
+int zipc_b200_zip_parse(const void *bytes, size_t len, zipc_b200_member **members, size_t *n_out) {
+  return zipc_b200_zip_parse_ex(bytes, len, ZIPC_ZIP_REFERENCE, members, n_out);
+}
+
+// flags = ZIPC_ZIP_REFERENCE: the reference's behaviour (ZIP64 rejected, zipc.ml:404).  ZIPC_ZIP_ALLOW_ZIP64 (SURVEY.md
+// 8f-4, beyond the reference): a ZIP64 end of central directory locator in front of the EOCD is followed, and central
+// directory entries take their 64-bit sizes / offsets from the ZIP64 extra field.
+int zipc_b200_zip_parse_ex(const void *bytes, size_t len, unsigned flags, zipc_b200_member **members, size_t *n_out) {
+  if (!members || !n_out || (!bytes && len)) return ZIPC_ERR_INVALID_ARG;
+  *members = nullptr;
+  *n_out = 0;
+  const uint8_t *s = static_cast<const uint8_t *>(bytes);
+  zb::ZipEnd e;
+  if (int st = zb::zip_find_end(s, 0, len, flags, e)) return st;
+  if (e.rec64 != ~0ull)
+    if (int st = zb::zip_read_end64(s + e.rec64, len, e)) return st;
+  std::vector<zipc_b200_member> ms;
+  std::vector<zb::ZipLfh> lfh;
+  const int cd_status = zb::zip_walk_cd(s + e.cd_start, len, flags, e, ms, lfh);
+  for (size_t k = 0; k < ms.size(); k++)
+    if (!ms[k].is_dir && lfh[k].off + 30 <= len) zb::zip_lfh_fields(s + lfh[k].off, lfh[k]);
+  return zb::zip_parse_finish(ms, lfh, cd_status, len, s, s + e.cd_start, e.cd_size, false, members, n_out);
 }
 
 // ---- Zipc.encoding_size / to_binary_string (zipc.ml:447-588) -----------------------------------------

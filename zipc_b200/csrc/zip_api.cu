@@ -4,7 +4,9 @@
 //   zipc_b200_deflate_batch        <- Zipc_deflate.deflate / crc_32_and_deflate / adler_32_and_deflate
 //                                     (reference src/zipc_deflate.ml:1247-1259)
 //   zipc_b200_zlib_compress_batch  <- Zipc_deflate.zlib_compress (:1262-1277); _dev: inputs and outputs in device memory
-//   zipc_b200_zip_extract_batch    <- Zipc.File.to_binary_string over parsed members (src/zipc.ml:205-225)
+//   zipc_b200_zip_extract_batch    <- Zipc.File.to_binary_string over parsed members (src/zipc.ml:205-225); _dev: members
+//                                     and outputs in device memory
+//   zipc_b200_zip_parse_dev        <- Zipc.of_binary_string (src/zipc.ml:400-438) of an archive in device memory
 //   zipc_b200_zip_deflate_archive  <- Zipc.File.deflate_of_binary_string + Zipc.to_binary_string
 //                                     (src/zipc.ml:179-185, 570-588)
 #include <algorithm>
@@ -50,6 +52,45 @@ __global__ void __launch_bounds__(256) gather_kernel(const CopyDesc *__restrict_
       for (uint64_t i = head + (nw << 2) + threadIdx.x; i < d.len; i += blockDim.x) d.dst[i] = d.src[i];
     }
   }
+}
+
+// one thread per member of an archive in device memory: the fields of its local header (byte loads: any offset).  The host
+// hands in only headers that lie inside the archive (off + 30 <= len).
+__global__ void zip_lfh_kernel(const uint8_t *__restrict__ archive, ZipLfh *f, uint32_t n) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  ZipLfh h = f[i];
+  zip_lfh_fields(archive + h.off, h);
+  f[i] = h;
+}
+
+// File.to_binary_string's dispatch (zipc.ml:205-217): 1 stored, 2 deflate, 0 nothing to extract (a directory, or a member
+// whose status this sets: encrypted, unsupported method)
+int member_kind(const zipc_b200_member &m, int *status) {
+  *status = ZIPC_OK;
+  if (m.is_dir) return 0;
+  if (m.gp_flags & 1) { *status = ZIPC_ERR_ZIP_ENCRYPTED; return 0; }
+  if (m.compression != 0 && m.compression != 8) { *status = ZIPC_ERR_ZIP_FORMAT; return 0; }
+  return m.compression == 0 ? 1 : 2;
+}
+
+// Stored members idx[j]: payload src[j] (device) to dst[j], CRC-32 compared with the directory's (one kernel, stored_copy_crc)
+int extract_stored(zipc_b200_ctx *ctx, const zipc_b200_member *ms, const std::vector<uint32_t> &idx,
+                   const std::vector<const uint8_t *> &src, const std::vector<uint8_t *> &dst, size_t *dst_len, uint32_t *found,
+                   int *status) {
+  const size_t k = idx.size();
+  if (!k) return ZIPC_OK;
+  std::vector<uint64_t> len(k);
+  std::vector<uint32_t> ck(k);
+  for (size_t j = 0; j < k; j++) len[j] = ms[idx[j]].compressed_size;
+  if (int st = stored_copy_crc(ctx, k, src.data(), dst.data(), len.data(), ck.data())) return st;
+  for (size_t j = 0; j < k; j++) {
+    const size_t i = idx[j];
+    dst_len[i] = (size_t)len[j];
+    if (found) found[i] = ck[j];
+    if (ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
+  }
+  return ZIPC_OK;
 }
 
 // Runs the encoder over n device-resident inputs.  Output of member i lands in a private slot
@@ -570,13 +611,11 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
   std::vector<int> kind(n, 0);  // 0 skip, 1 stored, 2 deflate
   for (size_t i = 0; i < n; i++) {
     const zipc_b200_member &m = ms[i];
-    status[i] = ZIPC_OK; dst_len[i] = 0;
+    dst_len[i] = 0;
     if (found) found[i] = 0;
-    if (m.is_dir) continue;
-    if (m.gp_flags & 1) { status[i] = ZIPC_ERR_ZIP_ENCRYPTED; continue; }
-    if (m.compression != 0 && m.compression != 8) { status[i] = ZIPC_ERR_ZIP_FORMAT; continue; }
+    kind[i] = member_kind(m, &status[i]);
+    if (!kind[i]) continue;
     if (m.compressed_size && !m.compressed_bytes) return ZIPC_ERR_INVALID_ARG;
-    kind[i] = m.compression == 0 ? 1 : 2;
     src[i] = m.compressed_bytes + m.start;
     slen[i] = (size_t)m.compressed_size;
     cap[i] = kind[i] == 1 ? (size_t)m.compressed_size : (size_t)m.decompressed_size;
@@ -624,38 +663,125 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
       if (st2[j] == ZIPC_OK && ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
     }
   }
-  // stored members: device copy + CRC-32
+  // stored members: one pass that copies and checksums
   idx.clear();
-  for (size_t i = 0; i < n; i++) if (kind[i] == 1) idx.push_back((uint32_t)i);
+  std::vector<const uint8_t *> s1;
+  std::vector<uint8_t *> d1;
+  for (size_t i = 0; i < n; i++)
+    if (kind[i] == 1) { idx.push_back((uint32_t)i); s1.push_back(d_src[i]); d1.push_back(ctx->d_out.as<uint8_t>() + off[i]); }
+  if (int st = extract_stored(ctx, ms, idx, s1, d1, dst_len, found, status)) return st;
+  return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need, &plan);
+}
+
+// The parser of zipc_b200_zip_parse_ex (host_util.cc) over an archive in device memory.  Copies, whatever the member count:
+// the tail window the EOCD search needs, the ZIP64 end record if there is one, the central directory (unless the tail
+// window holds it already), and the local header fields of all members through one kernel and one copy back.
+int zipc_b200_zip_parse_dev(zipc_b200_ctx *ctx, const void *d_bytes, size_t len, unsigned flags, zipc_b200_member **members,
+                            size_t *n_out) {
+  if (!ctx || !members || !n_out || (!d_bytes && len)) return ZIPC_ERR_INVALID_ARG;
+  *members = nullptr;
+  *n_out = 0;
+  if (len < 22) return ZIPC_ERR_ZIP_SHORT;
+  DeviceGuard g(ctx->device);
+  const uint8_t *d = static_cast<const uint8_t *>(d_bytes);
+  const uint64_t tail_at = len > kZipTailWindow ? len - kZipTailWindow : 0;
+  std::vector<uint8_t> tail(len - tail_at);
+  if (int st = d2h(ctx, tail.data(), d + tail_at, tail.size())) return st;
+  ZipEnd e;
+  if (int st = zip_find_end(tail.data(), tail_at, len, flags, e)) return st;
+  if (e.rec64 != ~0ull) {
+    uint8_t rec[56];
+    if (int st = d2h(ctx, rec, d + e.rec64, sizeof rec)) return st;
+    if (int st = zip_read_end64(rec, len, e)) return st;
+  }
+  std::vector<uint8_t> cd_copy;  // (a directory inside the tail window is read from there)
+  const uint8_t *cd;
+  if (e.cd_start >= tail_at) {
+    cd = tail.data() + (e.cd_start - tail_at);
+  } else {
+    cd_copy.resize((size_t)e.cd_size);
+    if (int st = d2h(ctx, cd_copy.data(), d + e.cd_start, cd_copy.size())) return st;
+    cd = cd_copy.data();
+  }
+  std::vector<zipc_b200_member> ms;
+  std::vector<ZipLfh> lfh;
+  const int cd_status = zip_walk_cd(cd, len, flags, e, ms, lfh);
+  std::vector<uint32_t> idx;
+  for (size_t k = 0; k < ms.size(); k++)
+    if (!ms[k].is_dir && lfh[k].off + 30 <= len) idx.push_back((uint32_t)k);
   if (!idx.empty()) {
-    size_t k = idx.size();
-    if (int st = ctx->h_desc.reserve(k * (sizeof(CopyDesc) + sizeof(CrcSeg)))) return st;
-    if (int st = ctx->d_desc2.reserve(k * (sizeof(CopyDesc) + sizeof(CrcSeg) + 4))) return st;
-    CopyDesc *hc = ctx->h_desc.as<CopyDesc>();
-    CrcSeg *hs = reinterpret_cast<CrcSeg *>(hc + k);
-    for (size_t j = 0; j < k; j++) {
-      size_t i = idx[j];
-      hc[j] = CopyDesc{d_src[i], ctx->d_out.as<uint8_t>() + off[i], slen[i]};
-      hs[j] = crc_seg(d_src[i], slen[i]);
-    }
-    CopyDesc *dc = ctx->d_desc2.as<CopyDesc>();
-    CrcSeg *ds = reinterpret_cast<CrcSeg *>(dc + k);
-    uint32_t *dck = reinterpret_cast<uint32_t *>(ds + k);
-    ZB_CUDA(ctx, cudaMemcpyAsync(dc, hc, k * (sizeof(CopyDesc) + sizeof(CrcSeg)), cudaMemcpyHostToDevice, ctx->stream));
-    if (int st = gather_launch(ctx, dc, (uint32_t)k)) return st;
-    if (int st = crc32_launch_segments(ctx, ds, (uint32_t)k, dck)) return st;
-    std::vector<uint32_t> ck(k);
-    ZB_CUDA(ctx, cudaMemcpyAsync(ck.data(), dck, k * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    const size_t m = idx.size();
+    if (int st = ctx->h_res.reserve(m * sizeof(ZipLfh))) return st;
+    if (int st = ctx->d_desc2.reserve(m * sizeof(ZipLfh))) return st;
+    ZipLfh *hf = ctx->h_res.as<ZipLfh>(), *df = ctx->d_desc2.as<ZipLfh>();
+    for (size_t j = 0; j < m; j++) hf[j] = lfh[idx[j]];
+    ZB_CUDA(ctx, cudaMemcpyAsync(df, hf, m * sizeof(ZipLfh), cudaMemcpyHostToDevice, ctx->stream));
+    zip_lfh_kernel<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream>>>(d, df, (uint32_t)m);
+    ctx->launches++;
+    ZB_CUDA(ctx, cudaGetLastError());
+    ZB_CUDA(ctx, cudaMemcpyAsync(hf, df, m * sizeof(ZipLfh), cudaMemcpyDeviceToHost, ctx->stream));
     ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
-    for (size_t j = 0; j < k; j++) {
-      size_t i = idx[j];
-      uint32_t c = ck[j] ^ 0xFFFFFFFFu;
-      dst_len[i] = slen[i];
-      if (found) found[i] = c;
-      if (c != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
+    for (size_t j = 0; j < m; j++) lfh[idx[j]] = hf[j];
+  }
+  return zip_parse_finish(ms, lfh, cd_status, len, d, cd, e.cd_size, true, members, n_out);
+}
+
+// Zipc.File.to_binary_string over members whose payloads are in device memory, into the caller's device slots.  Deflate
+// members go through the inflate core with CRC-32 (as zipc_b200_inflate_batch_dev), stored members through stored_copy_crc.
+int zipc_b200_zip_extract_batch_dev(zipc_b200_ctx *ctx, const zipc_b200_member *ms, size_t n, void *d_dst_v, const size_t *dst_off,
+                                    size_t *dst_len, uint32_t *found, int *status) {
+  if (!ctx || (n && (!ms || !d_dst_v || !dst_off || !dst_len || !status))) return ZIPC_ERR_INVALID_ARG;
+  if (!n) return ZIPC_OK;
+  if (n > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
+  DeviceGuard g(ctx->device);
+  // every payload pointer must be device memory of this ctx's device: host members (zipc_b200_zip_parse_ex) passed here by
+  // mistake are refused before anything runs.  One query per distinct pointer.
+  std::vector<const uint8_t *> seen;
+  for (size_t i = 0; i < n; i++) {
+    const zipc_b200_member &m = ms[i];
+    int st_i;
+    if (!member_kind(m, &st_i)) continue;
+    if (!m.compressed_bytes) {
+      if (m.compressed_size) return ZIPC_ERR_INVALID_ARG;
+      continue;
+    }
+    if (std::find(seen.begin(), seen.end(), m.compressed_bytes) != seen.end()) continue;
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, m.compressed_bytes) != cudaSuccess) { cudaGetLastError(); return ZIPC_ERR_INVALID_ARG; }
+    if (a.type != cudaMemoryTypeDevice || a.device != ctx->device) return ZIPC_ERR_INVALID_ARG;
+    seen.push_back(m.compressed_bytes);
+  }
+  ctx->epoch++;  // the caller's device bytes may have changed since the last call
+  uint8_t *d_dst = static_cast<uint8_t *>(d_dst_v);
+  std::vector<uint32_t> i2, i1;
+  std::vector<const uint8_t *> s2, s1;
+  std::vector<uint8_t *> d2, d1;
+  std::vector<size_t> l2, c2;
+  for (size_t i = 0; i < n; i++) {
+    const zipc_b200_member &m = ms[i];
+    dst_len[i] = 0;
+    if (found) found[i] = 0;
+    const int kind = member_kind(m, &status[i]);
+    if (kind == 1) { i1.push_back((uint32_t)i); s1.push_back(m.compressed_bytes + m.start); d1.push_back(d_dst + dst_off[i]); }
+    if (kind == 2) {
+      i2.push_back((uint32_t)i); s2.push_back(m.compressed_bytes + m.start); d2.push_back(d_dst + dst_off[i]);
+      l2.push_back((size_t)m.compressed_size); c2.push_back((size_t)m.decompressed_size);
     }
   }
-  return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need, &plan);
+  if (!i2.empty()) {
+    const size_t k = i2.size();
+    std::vector<size_t> ol(k);
+    std::vector<uint32_t> ck(k);
+    std::vector<int> st2(k);
+    if (int st = inflate_core(ctx, ZIPC_CK_CRC32, 0, k, s2, l2.data(), d2, c2, false, ol.data(), ck.data(), st2.data())) return st;
+    for (size_t j = 0; j < k; j++) {
+      const size_t i = i2[j];
+      status[i] = st2[j]; dst_len[i] = ol[j];
+      if (found) found[i] = ck[j];
+      if (st2[j] == ZIPC_OK && ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
+    }
+  }
+  return extract_stored(ctx, ms, i1, s1, d1, dst_len, found, status);
 }
 
 int zipc_b200_zip_deflate_archive(zipc_b200_ctx *ctx, int level, size_t n, const char *const *paths,
