@@ -282,6 +282,70 @@ def test_inflate_progressive_download_and_split_upload(ctx):
         L.zipc_b200_host_free(hsrc); L.zipc_b200_host_free(hdst)
 
 
+def test_zip_extract_progressive_download_with_mixed_members(ctx):
+    """zipc_b200_zip_extract_batch of a large archive into a pinned arena: the deflate members are decoded in download order
+    and copied out group by group while the kernel runs, with stored members, directories and a deflate member whose
+    directory CRC-32 is wrong between them.  The arena holds the deflate members by ascending output size, then the others
+    in member order; every member's bytes, status and found are those of zipfile / zlib, and a second call on the same
+    context gives the same results."""
+    import ctypes as C
+    L = ctx.L
+    n = 1200
+    buf = io.BytesIO()
+    with zipfile.ZipFile(buf, "w", zipfile.ZIP_DEFLATED) as zw:   # (paths in member order: the parser returns members by path)
+        for i in range(n):
+            if i % 97 == 40:
+                zw.mkdir("%04d-d" % i)
+            elif i % 13 == 6:
+                zw.writestr("%04d-s.bin" % i, synth.rand_v1(20_000 + i, 1 + (i * 7919) % 70_000).tobytes(), compress_type=zipfile.ZIP_STORED)
+            else:
+                zw.writestr("%04d-m.txt" % i, synth.text_v1(20_000 + i, 40_000 + (i * 6151) % 60_000).tobytes())
+    arch = np.frombuffer(buf.getvalue(), dtype=np.uint8)
+    zf = zipfile.ZipFile(io.BytesIO(buf.getvalue()))
+    p, cnt = C.POINTER(_lib.Member)(), C.c_size_t()
+    assert L.zipc_b200_zip_parse_ex(arch.ctypes.data, arch.size, zipc.ZIP_REFERENCE, C.byref(p), C.byref(cnt)) == _lib.OK
+    hdst = C.c_void_p()
+    try:
+        assert cnt.value == n
+        names = [C.string_at(p[i].path, p[i].path_len).decode() for i in range(n)]
+        assert all(name.startswith("%04d-" % i) for i, name in enumerate(names))
+        kind = ["dir" if p[i].is_dir else "stored" if p[i].compression == 0 else "deflate" for i in range(n)]
+        want = [b"" if k == "dir" else zf.read(name) for k, name in zip(kind, names)]
+        deflated = [i for i in range(n) if kind[i] == "deflate"]
+        bad = deflated[len(deflated) // 2]
+        p[bad].crc32 ^= 0x1
+        # the arena the progressive download lays out: deflate members by (output size, index), then the rest in member order
+        exp_off, t = np.zeros(n, dtype=np.uint64), 0
+        for i in sorted(deflated, key=lambda i: (len(want[i]), i)) + [i for i in range(n) if kind[i] != "deflate"]:
+            exp_off[i] = t
+            t += (len(want[i]) + 15) & ~15
+        assert len(deflated) >= 1024 and t >= (64 << 20) and {"dir", "stored"} <= set(kind)
+        cap = t + 4096
+        assert L.zipc_b200_host_alloc(cap, C.byref(hdst)) == 0
+        dst = np.ctypeslib.as_array(C.cast(hdst, C.POINTER(C.c_uint8)), shape=(cap,))
+        P = lambda a, ty: a.ctypes.data_as(C.POINTER(ty))
+        runs = []
+        for fill in (0xEE, 0x11):
+            dst[:] = fill
+            need = C.c_size_t()
+            off, ln = np.zeros(n, dtype=np.uint64), np.zeros(n, dtype=np.uint64)
+            fo, st = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.int32)
+            rc = L.zipc_b200_zip_extract_batch(ctx.h, p, n, hdst, cap, C.byref(need), P(off, C.c_size_t), P(ln, C.c_size_t),
+                                               P(fo, C.c_uint32), P(st, C.c_int))
+            assert rc == _lib.OK and need.value == t
+            assert (off == exp_off).all() and not (np.diff(off[deflated].astype(np.int64)) > 0).all()
+            for i in range(n):
+                assert st[i] == (_lib.ERR_CHECKSUM if i == bad else _lib.OK), (i, kind[i], st[i])
+                assert ln[i] == len(want[i]) and fo[i] == (zlib.crc32(want[i]) if kind[i] != "dir" else 0), (i, kind[i])
+                assert dst[int(off[i]):int(off[i]) + int(ln[i])].tobytes() == want[i], (i, kind[i])
+            runs.append((off, ln, fo, st))
+        assert all((a == b).all() for a, b in zip(*runs))
+    finally:
+        L.zipc_b200_free(C.cast(p, C.c_void_p))
+        if hdst.value:
+            L.zipc_b200_host_free(hdst)
+
+
 def test_large_archive_pipelined_equals_plain(ctx):
     """zipc_b200_zip_deflate_archive of a large member set given in path order goes through the pipeline (every group's
     payloads copied to their archive offsets while later groups are compressed); given in reverse order it takes the plain

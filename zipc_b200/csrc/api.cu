@@ -345,22 +345,40 @@ static __global__ void xor_ffffffff_kernel(uint32_t *v, uint32_t n) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) v[i] ^= 0xFFFFFFFFu;
 }
-// one thread per zlib stream in device memory: header status, method and trailer (byte loads: any offset)
+// one thread per zlib stream in device memory (byte loads: any offset)
 static __global__ void zlib_frames_kernel(ZlibFrame *f, uint32_t n) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   ZlibFrame z = f[i];
-  z.method = 0;
-  z.status = (uint32_t)zlib_header_status(z.src, z.len, &z.method);
-  z.expect = z.status == ZIPC_OK ? zlib_trailer(z.src, z.len) : 0u;
+  zlib_check_frame(z);
   f[i] = z;
 }
 
-// One warp per stream (inflate.cu).  All pointers in d_src / d_dst are device addresses.
-static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
-                               const size_t *src_len, const std::vector<uint8_t *> &d_dst, const std::vector<size_t> &cap,
-                               bool count_only, size_t *out_len, uint32_t *checksum, int *status, uint32_t flags,
-                               const DownloadPlan *plan) {
+// The results of both zlib_decompress calls from the frames and the decode of the streams whose header passed (status,
+// dst_len and adler[i], the Adler-32 of the output).  A rejected stream gets its frame's status (found: CM on
+// ZIPC_ERR_ZLIB_METHOD); a decoded one gets expect / found if it decoded, and ZIPC_ERR_CHECKSUM if they differ.
+static void zlib_verdict(size_t n, const ZlibFrame *f, const uint32_t *adler, size_t *dst_len, uint32_t *expect, uint32_t *found,
+                         int *status) {
+  for (size_t i = 0; i < n; i++) {
+    if (f[i].status != ZIPC_OK) {
+      status[i] = (int)f[i].status;
+      dst_len[i] = 0;
+      if (f[i].status == ZIPC_ERR_ZLIB_METHOD && found) found[i] = f[i].method;
+    } else if (status[i] == ZIPC_OK) {
+      if (expect) expect[i] = f[i].expect;
+      if (found) found[i] = adler[i];
+      if (adler[i] != f[i].expect) status[i] = ZIPC_ERR_CHECKSUM;
+    }
+  }
+}
+
+// One warp per stream (inflate.cu), for the streams sel (ascending indices into the caller's arrays, which results are
+// written at).  All pointers in d_src / d_dst are device addresses.
+static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, const std::vector<uint32_t> &sel,
+                               const std::vector<const uint8_t *> &d_src, const size_t *src_len, const std::vector<uint8_t *> &d_dst,
+                               const std::vector<size_t> &cap, bool count_only, size_t *out_len, uint32_t *checksum, int *status,
+                               uint32_t flags, const DownloadPlan *plan) {
+  const size_t n = sel.size();
   if (!n) return ZIPC_OK;
   if (n > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
   static const bool call_debug = env_u64("ZIPC_B200_CALL_DEBUG", 0) != 0;   // host-side time stamps of one call on stderr
@@ -370,18 +388,19 @@ static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_
   // longest streams first: the tail of the dynamic queue is made of short ones.  With a progressive download the groups
   // go in download order instead (smallest outputs first), so that the copies start early and never run dry.
   // (a radix sort of packed keys -- group, length, index: this runs while the GPU waits, 0.5 ms with std::sort for 10k streams)
-  std::vector<uint32_t> order(n);
+  std::vector<uint32_t> order(sel);
   {
     bool fits = n <= 0xFFFFFFu;
-    for (size_t i = 0; i < n && fits; i++) fits = src_len[i] < (1ull << 32);
+    for (size_t j = 0; j < n && fits; j++) fits = src_len[sel[j]] < (1ull << 32);
     if (fits) {
       std::vector<uint64_t> key(n), tmp(n);
-      for (size_t i = 0; i < n; i++) {
+      for (size_t j = 0; j < n; j++) {
+        const uint32_t i = sel[j];
         const uint64_t g = grouped ? plan->group_of[i] : 0u;                                          // < 256
         const uint64_t len = grouped ? (uint64_t)src_len[i] : 0xFFFFFFFFull - (uint64_t)src_len[i];   // ascending in a group, else longest first
-        key[i] = (g << 56) | (len << 24) | (uint64_t)i;
+        key[j] = (g << 56) | (len << 24) | (uint64_t)j;
       }
-      // least significant digit first over bits 24..63 (the index below them keeps equal keys in input order)
+      // least significant digit first over bits 24..63 (the position in sel below them keeps equal keys in input order)
       for (int shift = 24; shift < 64; shift += 8) {
         if (shift == 56 && !grouped) break;
         size_t cnt[257] = {0};
@@ -390,9 +409,8 @@ static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_
         for (size_t i = 0; i < n; i++) tmp[cnt[(key[i] >> shift) & 0xFFu]++] = key[i];
         key.swap(tmp);
       }
-      for (size_t i = 0; i < n; i++) order[i] = (uint32_t)(key[i] & 0xFFFFFFu);
+      for (size_t k = 0; k < n; k++) order[k] = sel[key[k] & 0xFFFFFFu];
     } else {
-      std::iota(order.begin(), order.end(), 0u);
       if (grouped)
         std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
           return plan->group_of[a] != plan->group_of[b] ? plan->group_of[a] < plan->group_of[b] : src_len[a] < src_len[b]; });
@@ -424,7 +442,7 @@ static int inflate_serial_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_
   unsigned int *d_gcount = nullptr;
   if (grouped) {
     std::vector<unsigned int> cnt(plan->ngroups, 0u);
-    for (size_t i = 0; i < n; i++) cnt[plan->group_of[i]]++;
+    for (uint32_t i : sel) cnt[plan->group_of[i]]++;
     d_gcount = reinterpret_cast<unsigned int *>(dck + n);  // behind the checksums (the buffer has 1 KiB to spare)
     if (!ctx->h_gflag) ZB_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_gflag), 256 * sizeof(uint32_t), cudaHostAllocMapped));
     if (!ctx->copy_stream) ZB_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
@@ -682,21 +700,27 @@ static int par_resolve(zipc_b200_ctx *ctx, uint8_t *d_dst, bool *ok) {
   return ZIPC_OK;
 }
 
-// Core of every inflate entry point.  All pointers in d_src / d_dst are device addresses.
+// Core of every inflate entry point.  All pointers in d_src / d_dst are device addresses.  subset (null: all n streams) lists,
+// in ascending order, the streams to decode; the results of the others are left as they are.
 // cap[i] == ZIPC_SIZE_UNKNOWN is only accepted in a count-only pass (the callers resolve sizes first).
 // Large streams are decoded in parallel inside the stream where that works out; everything else (and every stream whose
 // parallel decoding does not check out) goes to the warp-per-stream decoder.
 int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
                  const size_t *src_len, const std::vector<uint8_t *> &d_dst, const std::vector<size_t> &cap,
-                 bool count_only, size_t *out_len, uint32_t *checksum, int *status, uint32_t flags, const DownloadPlan *plan) {
+                 bool count_only, size_t *out_len, uint32_t *checksum, int *status, uint32_t flags, const DownloadPlan *plan,
+                 const std::vector<uint32_t> *subset) {
+  std::vector<uint32_t> rest;  // the selected streams the many-warp decoder has not done
+  if (subset) rest = *subset;
+  else { rest.resize(n); std::iota(rest.begin(), rest.end(), 0u); }
   std::vector<char> done(n, 0);
-  size_t ndone = 0;
   if (flags == 0 && par_min_bytes() != 0 && !(plan && plan->ngroups)) {
     const size_t lanes = ctx->is_sub ? 1 : par_lane_count();
+    std::vector<size_t> len(rest.size());
+    for (size_t j = 0; j < rest.size(); j++) len[j] = src_len[rest[j]];
     std::vector<char> take;
-    par_select(n, src_len, take, lanes);
+    par_select(rest.size(), len.data(), take, lanes);
     std::vector<uint32_t> sel;
-    for (size_t i = 0; i < n; i++) if (take[i]) sel.push_back((uint32_t)i);
+    for (size_t j = 0; j < rest.size(); j++) if (take[j]) sel.push_back(rest[j]);
     // one stream through the many-warp decoder, on context c (ctx itself, or one of its lanes)
     auto one = [&](zipc_b200_ctx *c, uint32_t i, uint64_t &streams, uint64_t &fallbacks) -> int {
       bool ok = false;
@@ -789,21 +813,9 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
         if (rc[k]) { ctx->last_error = zipc_b200_last_error(zipc_b200_mctx_ctx(pool, (int)k)); return rc[k]; }
       }
     }
-    for (size_t i = 0; i < n; i++) ndone += done[i] != 0;
+    rest.erase(std::remove_if(rest.begin(), rest.end(), [&](uint32_t i) { return done[i] != 0; }), rest.end());
   }
-  if (ndone == 0) return inflate_serial_core(ctx, ck, adler_mode, n, d_src, src_len, d_dst, cap, count_only, out_len, checksum, status, flags, plan);
-  if (ndone == n) return ZIPC_OK;
-  // the rest through the warp-per-stream decoder
-  const size_t r = n - ndone;
-  std::vector<const uint8_t *> s2(r);
-  std::vector<uint8_t *> d2(r);
-  std::vector<size_t> l2(r), c2(r), ol(r);
-  std::vector<uint32_t> ck2(r), idx(r);
-  std::vector<int> st2(r);
-  for (size_t i = 0, j = 0; i < n; i++) if (!done[i]) { idx[j] = (uint32_t)i; s2[j] = d_src[i]; d2[j] = d_dst[i]; l2[j] = src_len[i]; c2[j] = cap[i]; j++; }
-  if (int st = inflate_serial_core(ctx, ck, adler_mode, r, s2, l2.data(), d2, c2, count_only, ol.data(), checksum ? ck2.data() : nullptr, st2.data(), flags, nullptr)) return st;
-  for (size_t j = 0; j < r; j++) { out_len[idx[j]] = ol[j]; status[idx[j]] = st2[j]; if (checksum) checksum[idx[j]] = ck2[j]; }
-  return ZIPC_OK;
+  return inflate_serial_core(ctx, ck, adler_mode, rest, d_src, src_len, d_dst, cap, count_only, out_len, checksum, status, flags, plan);
 }
 
 // ---- progressive download ---------------------------------------------------------------------------------------------------
@@ -1124,7 +1136,7 @@ int zipc_b200_inflate_batch(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n
   DownloadPlan plan;
   if (int st = plan_arena(ctx, n, cap.data(), src, src_len, all.data(), split, dst, dst_cap, off, total, plan)) return st;
   if (int st = ctx->d_out.reserve(total + 64)) return st;
-  for (size_t i = 0; i < n; i++) d_dst[i] = ctx->d_out.as<uint8_t>() + off[i];
+  d_dst = slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n);
   if (int st = inflate_core(ctx, ck, adler_mode, n, d_src, src_len, d_dst, cap, false, dst_len, checksum, status, 0, &plan)) {
     if (plan.ngroups && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // no copy into the caller's arena outlives the call
     return st;
@@ -1149,16 +1161,10 @@ int zipc_b200_inflate_batch_dev(zipc_b200_ctx *ctx, int ck, int adler_mode, size
   if (!n) return ZIPC_OK;
   DeviceGuard g(ctx->device);
   ctx->epoch++;  // the caller's device bytes may have changed since the last call
-  std::vector<const uint8_t *> d_src(n);
-  std::vector<uint8_t *> d_dst(n);
-  std::vector<size_t> cap(n);
-  for (size_t i = 0; i < n; i++) {
-    if (max_out[i] == ZIPC_SIZE_UNKNOWN) return ZIPC_ERR_INVALID_ARG;
-    d_src[i] = static_cast<const uint8_t *>(d_src_v) + src_off[i];
-    d_dst[i] = static_cast<uint8_t *>(d_dst_v) + dst_off[i];
-    cap[i] = max_out[i];
-  }
-  return inflate_core(ctx, ck, adler_mode, n, d_src, src_len, d_dst, cap, false, dst_len, checksum, status);
+  for (size_t i = 0; i < n; i++) if (max_out[i] == ZIPC_SIZE_UNKNOWN) return ZIPC_ERR_INVALID_ARG;
+  return inflate_core(ctx, ck, adler_mode, n, slot_addrs(static_cast<const uint8_t *>(d_src_v), src_off, n), src_len,
+                      slot_addrs(static_cast<uint8_t *>(d_dst_v), dst_off, n), std::vector<size_t>(max_out, max_out + n), false,
+                      dst_len, checksum, status);
 }
 
 int zipc_b200_zlib_decompress_batch(zipc_b200_ctx *ctx, int adler_mode, size_t n, const void *const *src,
@@ -1169,37 +1175,25 @@ int zipc_b200_zlib_decompress_batch(zipc_b200_ctx *ctx, int adler_mode, size_t n
   if (dst_need) *dst_need = 0;
   if (!n) return ZIPC_OK;
   // header checks in the reference's order (zipc_deflate.ml:722-731); bad streams become empty tasks
+  std::vector<ZlibFrame> f(n);
   std::vector<const void *> body(n);
-  std::vector<size_t> blen(n);
-  std::vector<int> pre(n, ZIPC_OK);
-  std::vector<uint32_t> exp(n, 0);
+  std::vector<size_t> blen(n, 0), mo(n, 0);
   for (size_t i = 0; i < n; i++) {
     const uint8_t *s = static_cast<const uint8_t *>(src[i]);
-    size_t len = src_len[i];
-    body[i] = s; blen[i] = 0;
-    if (len && !s) return ZIPC_ERR_INVALID_ARG;
-    uint32_t method = 0;
-    pre[i] = zlib_header_status(s, len, &method);
-    if (pre[i] == ZIPC_ERR_ZLIB_METHOD && found) found[i] = method;
-    if (pre[i]) continue;
-    exp[i] = zlib_trailer(s, len);
+    if (src_len[i] && !s) return ZIPC_ERR_INVALID_ARG;
+    f[i] = ZlibFrame{s, src_len[i], 0, 0, 0, 0};
+    zlib_check_frame(f[i]);
+    body[i] = s;
+    if (f[i].status != ZIPC_OK) continue;
     body[i] = s + 2;
-    blen[i] = len - 4;  // as the reference: two bytes into the trailer (zipc_deflate.ml:732)
+    blen[i] = src_len[i] - 4;  // as the reference: two bytes into the trailer (zipc_deflate.ml:732)
+    mo[i] = max_out ? max_out[i] : ZIPC_SIZE_UNKNOWN;
   }
   std::vector<uint32_t> ad(n);
-  std::vector<size_t> mo(n);
-  for (size_t i = 0; i < n; i++) mo[i] = pre[i] ? 0 : (max_out ? max_out[i] : ZIPC_SIZE_UNKNOWN);
   int rc = zipc_b200_inflate_batch(ctx, ZIPC_CK_ADLER32, adler_mode, n, body.data(), blen.data(), mo.data(), dst, dst_cap,
                                    dst_need, dst_off, dst_len, ad.data(), status);
   if (rc != ZIPC_OK && rc != ZIPC_ERR_DST_TOO_SMALL) return rc;
-  for (size_t i = 0; i < n; i++) {
-    if (pre[i]) { status[i] = pre[i]; dst_len[i] = 0; continue; }
-    if (status[i] == ZIPC_OK) {
-      if (expect) expect[i] = exp[i];
-      if (found) found[i] = ad[i];
-      if (ad[i] != exp[i]) status[i] = ZIPC_ERR_CHECKSUM;
-    }
-  }
+  zlib_verdict(n, f.data(), ad.data(), dst_len, expect, found, status);
   return rc;
 }
 
@@ -1225,42 +1219,23 @@ int zipc_b200_zlib_decompress_batch_dev(zipc_b200_ctx *ctx, int adler_mode, size
   ZB_CUDA(ctx, cudaGetLastError());
   ZB_CUDA(ctx, cudaMemcpyAsync(hf, df, n * sizeof(ZlibFrame), cudaMemcpyDeviceToHost, ctx->stream));
   ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
-  // streams with a bad header get their status here and are not decoded (their slots stay untouched); the others' bodies are
-  // [2, len - 2), as in the reference (zipc_deflate.ml:732)
-  std::vector<uint32_t> idx, exp;
-  std::vector<const uint8_t *> body;
-  std::vector<uint8_t *> d_dst;
-  std::vector<size_t> blen, cap;
+  // streams with a bad header are not decoded (their slots stay untouched); the others' bodies are [2, len - 2), as in the
+  // reference (zipc_deflate.ml:732)
+  const std::vector<ZlibFrame> f(hf, hf + n);  // (h_res is the inflate core's too)
+  std::vector<uint32_t> sel;
+  std::vector<const uint8_t *> body(n);
+  std::vector<size_t> blen(n, 0);
   for (size_t i = 0; i < n; i++) {
-    const ZlibFrame &f = hf[i];
-    if (f.status != ZIPC_OK) {
-      status[i] = (int)f.status;
-      dst_len[i] = 0;
-      if (f.status == ZIPC_ERR_ZLIB_METHOD && found) found[i] = f.method;
-      continue;
-    }
-    idx.push_back((uint32_t)i);
-    exp.push_back(f.expect);
-    body.push_back(f.src + 2);
-    blen.push_back((size_t)f.len - 4);
-    d_dst.push_back(static_cast<uint8_t *>(d_dst_v) + dst_off[i]);
-    cap.push_back(max_out[i]);
+    if (f[i].status != ZIPC_OK) continue;
+    sel.push_back((uint32_t)i);
+    body[i] = f[i].src + 2;
+    blen[i] = (size_t)f[i].len - 4;
   }
-  const size_t k = idx.size();
-  std::vector<size_t> ol(k);
-  std::vector<uint32_t> ad(k);
-  std::vector<int> st(k);
-  if (int rc = inflate_core(ctx, ZIPC_CK_ADLER32, adler_mode, k, body, blen.data(), d_dst, cap, false, ol.data(), ad.data(), st.data()))
+  std::vector<uint32_t> ad(n);
+  if (int rc = inflate_core(ctx, ZIPC_CK_ADLER32, adler_mode, n, body, blen.data(), slot_addrs(static_cast<uint8_t *>(d_dst_v), dst_off, n),
+                            std::vector<size_t>(max_out, max_out + n), false, dst_len, ad.data(), status, 0, nullptr, &sel))
     return rc;
-  for (size_t j = 0; j < k; j++) {
-    const uint32_t i = idx[j];
-    status[i] = st[j];
-    dst_len[i] = ol[j];
-    if (st[j] != ZIPC_OK) continue;
-    if (expect) expect[i] = exp[j];
-    if (found) found[i] = ad[j];
-    if (ad[j] != exp[j]) status[i] = ZIPC_ERR_CHECKSUM;
-  }
+  zlib_verdict(n, f.data(), ad.data(), dst_len, expect, found, status);
   return ZIPC_OK;
 }
 

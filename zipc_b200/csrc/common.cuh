@@ -163,7 +163,7 @@ __host__ __device__ inline int zlib_header_status(const uint8_t *s, uint64_t len
 __host__ __device__ inline uint32_t zlib_trailer(const uint8_t *s, uint64_t len) {
   return (uint32_t)s[len - 4] << 24 | (uint32_t)s[len - 3] << 16 | (uint32_t)s[len - 2] << 8 | s[len - 1];
 }
-struct ZlibFrame {    // one stream of zipc_b200_zlib_decompress_batch_dev: the host fills src / len, zlib_frames_kernel the rest
+struct ZlibFrame {    // one stream of zipc_b200_zlib_decompress_batch(_dev): src / len, and what zlib_check_frame finds there
   const uint8_t *src;
   uint64_t len;
   uint32_t status;    // zlib_header_status
@@ -171,6 +171,12 @@ struct ZlibFrame {    // one stream of zipc_b200_zlib_decompress_batch_dev: the 
   uint32_t expect;    // the trailer when status is ZIPC_OK
   uint32_t _pad;
 };
+// fills status, method and expect of f from its src / len (host or device memory)
+__host__ __device__ inline void zlib_check_frame(ZlibFrame &f) {
+  f.method = 0;
+  f.status = (uint32_t)zlib_header_status(f.src, f.len, &f.method);
+  f.expect = f.status == ZIPC_OK ? zlib_trailer(f.src, f.len) : 0u;
+}
 
 // ---- ZIP archives ------------------------------------------------------------------------------
 // The four fields of a local file header (APPNOTE 4.3.7) the parser checks; off comes from the central directory.
@@ -339,16 +345,22 @@ int upload_ranges(zipc_b200_ctx *ctx, size_t n, const void *const *src, const si
 // complete, and the host starts that range's copy while the kernel works on the larger streams.
 struct DownloadPlan {
   uint32_t ngroups = 0;                 // 0: not used, the arena is in member order and comes back with one copy
-  std::vector<uint32_t> group_of;       // per stream handed to inflate_core
+  std::vector<uint32_t> group_of;       // per stream of the batch (inflate_core's index; 0 for streams it does not decode)
   std::vector<size_t> goff, gbytes;     // arena range of each group
   uint8_t *dst = nullptr;               // the caller's (pinned) arena
   size_t tail_off = 0, tail_bytes = 0;  // arena range of everything that is not a grouped stream (copied at the end)
-  std::vector<char> late;               // per stream handed to inflate_core: 1 if the second part of a split upload carries its input
+  std::vector<char> late;               // per stream of the batch: 1 if the second part of a split upload carries its input
 };
 int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
                  const size_t *src_len, const std::vector<uint8_t *> &d_dst, const std::vector<size_t> &cap,
                  bool count_only, size_t *out_len, uint32_t *checksum, int *status, uint32_t flags = 0,
-                 const DownloadPlan *plan = nullptr);
+                 const DownloadPlan *plan = nullptr, const std::vector<uint32_t> *subset = nullptr);
+// the device addresses base + off[i] of n slots
+template <class T> std::vector<T *> slot_addrs(T *base, const size_t *off, size_t n) {
+  std::vector<T *> p(n);
+  for (size_t i = 0; i < n; i++) p[i] = base + off[i];
+  return p;
+}
 // Lay out the output arena of n members (cap[i] bytes each, 16-byte aligned slots).  grouped[i] != 0 marks the streams that
 // go through the inflate kernel.  Fills off / total, and plan when the batch qualifies for a progressive download.
 // The streams whose input the second part of a split upload carries (src: their host addresses) form the later groups.

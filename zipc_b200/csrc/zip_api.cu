@@ -74,21 +74,39 @@ int member_kind(const zipc_b200_member &m, int *status) {
   return m.compression == 0 ? 1 : 2;
 }
 
-// Stored members idx[j]: payload src[j] (device) to dst[j], CRC-32 compared with the directory's (one kernel, stored_copy_crc)
-int extract_stored(zipc_b200_ctx *ctx, const zipc_b200_member *ms, const std::vector<uint32_t> &idx,
-                   const std::vector<const uint8_t *> &src, const std::vector<uint8_t *> &dst, size_t *dst_len, uint32_t *found,
-                   int *status) {
-  const size_t k = idx.size();
-  if (!k) return ZIPC_OK;
-  std::vector<uint64_t> len(k);
-  std::vector<uint32_t> ck(k);
-  for (size_t j = 0; j < k; j++) len[j] = ms[idx[j]].compressed_size;
-  if (int st = stored_copy_crc(ctx, k, src.data(), dst.data(), len.data(), ck.data())) return st;
-  for (size_t j = 0; j < k; j++) {
-    const size_t i = idx[j];
-    dst_len[i] = (size_t)len[j];
-    if (found) found[i] = ck[j];
-    if (ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
+// File.to_binary_string over n members (zipc.ml:205-225) whose payloads are at d_src[i] (device), into d_dst[i]: sets every
+// member's status, dst_len and found.  Deflate members go through the inflate core with CRC-32 (plan: the progressive
+// download of zipc_b200_zip_extract_batch, or null), then stored members through stored_copy_crc, which copies and checksums
+// in one pass; both are checked against the directory's CRC-32.
+int extract_members(zipc_b200_ctx *ctx, const zipc_b200_member *ms, size_t n, const std::vector<const uint8_t *> &d_src,
+                    const std::vector<uint8_t *> &d_dst, const DownloadPlan *plan, size_t *dst_len, uint32_t *found, int *status) {
+  std::vector<uint32_t> inflated, stored;
+  std::vector<size_t> slen(n, 0), cap(n, 0);
+  std::vector<const uint8_t *> s1;
+  std::vector<uint8_t *> d1;
+  std::vector<uint64_t> l1;
+  for (size_t i = 0; i < n; i++) {
+    const zipc_b200_member &m = ms[i];
+    dst_len[i] = 0;
+    if (found) found[i] = 0;
+    const int kind = member_kind(m, &status[i]);
+    if (kind == 1) { stored.push_back((uint32_t)i); s1.push_back(d_src[i]); d1.push_back(d_dst[i]); l1.push_back(m.compressed_size); }
+    if (kind == 2) { inflated.push_back((uint32_t)i); slen[i] = (size_t)m.compressed_size; cap[i] = (size_t)m.decompressed_size; }
+  }
+  std::vector<uint32_t> ck(n);
+  if (int st = inflate_core(ctx, ZIPC_CK_CRC32, 0, n, d_src, slen.data(), d_dst, cap, false, dst_len, ck.data(), status, 0, plan, &inflated))
+    return st;
+  for (uint32_t i : inflated) {
+    if (found) found[i] = ck[i];
+    if (status[i] == ZIPC_OK && ck[i] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
+  }
+  std::vector<uint32_t> c1(stored.size());
+  if (int st = stored_copy_crc(ctx, stored.size(), s1.data(), d1.data(), l1.data(), c1.data())) return st;
+  for (size_t j = 0; j < stored.size(); j++) {
+    const uint32_t i = stored[j];
+    dst_len[i] = (size_t)l1[j];
+    if (found) found[i] = c1[j];
+    if (c1[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
   }
   return ZIPC_OK;
 }
@@ -432,16 +450,10 @@ int zipc_b200_deflate_batch_dev(zipc_b200_ctx *ctx, int level, int ck, int adler
     return ZIPC_ERR_INVALID_ARG;
   if (!n) return ZIPC_OK;
   DeviceGuard g(ctx->device);
-  std::vector<const uint8_t *> d_src(n);
-  std::vector<uint8_t *> d_slot(n);
-  std::vector<size_t> cap(n);
-  for (size_t i = 0; i < n; i++) {
-    d_src[i] = static_cast<const uint8_t *>(d_src_v) + src_off[i];
-    d_slot[i] = static_cast<uint8_t *>(d_dst_v) + dst_off[i];
-    if ((uintptr_t)d_slot[i] & 3) return ZIPC_ERR_INVALID_ARG;  // output slots are written as 32-bit words
-    cap[i] = dst_cap_each[i];
-  }
-  return deflate_run(ctx, level, ck, adler_mode, n, d_src, src_len, d_slot, cap, dst_len, checksum, status);
+  const std::vector<uint8_t *> d_slot = slot_addrs(static_cast<uint8_t *>(d_dst_v), dst_off, n);
+  for (uint8_t *p : d_slot) if ((uintptr_t)p & 3) return ZIPC_ERR_INVALID_ARG;  // output slots are written as 32-bit words
+  return deflate_run(ctx, level, ck, adler_mode, n, slot_addrs(static_cast<const uint8_t *>(d_src_v), src_off, n), src_len, d_slot,
+                     std::vector<size_t>(dst_cap_each, dst_cap_each + n), dst_len, checksum, status);
 }
 
 int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode, size_t n, const void *const *src,
@@ -462,9 +474,7 @@ int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode,
   size_t total = 0;
   for (size_t i = 0; i < n; i++) { off[i] = total; flen[i] = dst_len[i] + 6; total += align_up(flen[i], 16); }
   if (int st = ctx->d_out.reserve(total + 64)) return st;
-  std::vector<uint8_t *> to(n);
-  for (size_t i = 0; i < n; i++) to[i] = ctx->d_out.as<uint8_t>() + off[i];
-  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), to)) return st;
+  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n))) return st;
   for (size_t i = 0; i < n; i++) { dst_len[i] = flen[i]; if (adler) adler[i] = ad[i]; }
   return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
 }
@@ -477,11 +487,10 @@ int zipc_b200_zlib_compress_batch_dev(zipc_b200_ctx *ctx, int level, int adler_m
     return ZIPC_ERR_INVALID_ARG;
   if (!n) return ZIPC_OK;
   DeviceGuard g(ctx->device);
-  std::vector<const uint8_t *> d_src(n);
-  for (size_t i = 0; i < n; i++) d_src[i] = static_cast<const uint8_t *>(d_src_v) + src_off[i];
   std::vector<uint32_t> ad(n);
   Pieces pc;  // compressed into the library's slots as by zipc_b200_zlib_compress_batch: same pieces, same bytes
-  if (int st = deflate_members(ctx, level, ZIPC_CK_ADLER32, adler_mode, n, d_src, src_len, dst_len, ad.data(), status, pc)) return st;
+  if (int st = deflate_members(ctx, level, ZIPC_CK_ADLER32, adler_mode, n, slot_addrs(static_cast<const uint8_t *>(d_src_v), src_off, n),
+                               src_len, dst_len, ad.data(), status, pc)) return st;
   // a stream goes to its slot only if all of it fits: a slot too small is not written at all
   std::vector<uint8_t *> to(n, nullptr);
   for (size_t i = 0; i < n; i++) {
@@ -605,24 +614,23 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
   if (dst_need) *dst_need = 0;
   if (!n) return ZIPC_OK;
   DeviceGuard g(ctx->device);
-  // classify (reference zipc.ml:205-217): encrypted -> error; Stored / Deflate handled; anything else -> error
+  // the payloads and output slots of the members that are extracted (member_kind); the deflate ones may form download groups
   std::vector<const void *> src(n, nullptr);
   std::vector<size_t> slen(n, 0), cap(n, 0);
-  std::vector<int> kind(n, 0);  // 0 skip, 1 stored, 2 deflate
+  std::vector<char> grouped(n, 0);
+  bool all_deflate = true;   // (stored members are copied by a kernel that does not wait for a late half)
   for (size_t i = 0; i < n; i++) {
     const zipc_b200_member &m = ms[i];
-    dst_len[i] = 0;
-    if (found) found[i] = 0;
-    kind[i] = member_kind(m, &status[i]);
-    if (!kind[i]) continue;
+    int kind_status;
+    const int kind = member_kind(m, &kind_status);
+    if (!kind) continue;
     if (m.compressed_size && !m.compressed_bytes) return ZIPC_ERR_INVALID_ARG;
     src[i] = m.compressed_bytes + m.start;
     slen[i] = (size_t)m.compressed_size;
-    cap[i] = kind[i] == 1 ? (size_t)m.compressed_size : (size_t)m.decompressed_size;
+    cap[i] = kind == 1 ? (size_t)m.compressed_size : (size_t)m.decompressed_size;
+    grouped[i] = kind == 2;
+    all_deflate &= kind != 1;
   }
-  std::vector<char> grouped(n);
-  bool all_deflate = true;   // (stored members are copied by a kernel that does not wait for a late half)
-  for (size_t i = 0; i < n; i++) { grouped[i] = kind[i] == 2; all_deflate &= kind[i] != 1; }
   UploadSplit split;
   split.want = all_deflate && progressive_ok(ctx, n, cap.data(), slen.data(), grouped.data(), dst, dst_cap);
   std::vector<const uint8_t *> d_src;
@@ -638,38 +646,8 @@ int zipc_b200_zip_extract_batch(zipc_b200_ctx *ctx, const zipc_b200_member *ms, 
     ~CopyFence() { if (on && c->copy_stream) cudaStreamSynchronize(c->copy_stream); }
   } fence{ctx, plan.ngroups != 0};
   if (int st = ctx->d_out.reserve(total + 64)) return st;
-  // deflate members through the inflate kernel (with CRC-32 of the output)
-  std::vector<uint32_t> idx;
-  for (size_t i = 0; i < n; i++) if (kind[i] == 2) idx.push_back((uint32_t)i);
-  if (!idx.empty()) {
-    size_t k = idx.size();
-    std::vector<const uint8_t *> s2(k);
-    std::vector<uint8_t *> d2(k);
-    std::vector<size_t> l2(k), c2(k), ol(k);
-    std::vector<uint32_t> ck(k);
-    std::vector<int> st2(k);
-    for (size_t j = 0; j < k; j++) { s2[j] = d_src[idx[j]]; d2[j] = ctx->d_out.as<uint8_t>() + off[idx[j]]; l2[j] = slen[idx[j]]; c2[j] = cap[idx[j]]; }
-    DownloadPlan plan2 = plan;  // the same groups, indexed like the arrays handed to inflate_core
-    if (plan.ngroups) {
-      plan2.group_of.resize(k);
-      for (size_t j = 0; j < k; j++) plan2.group_of[j] = plan.group_of[idx[j]];
-      if (!plan.late.empty()) { plan2.late.resize(k); for (size_t j = 0; j < k; j++) plan2.late[j] = plan.late[idx[j]]; }
-    }
-    if (int st = inflate_core(ctx, ZIPC_CK_CRC32, 0, k, s2, l2.data(), d2, c2, false, ol.data(), ck.data(), st2.data(), 0, &plan2)) return st;
-    for (size_t j = 0; j < k; j++) {
-      size_t i = idx[j];
-      status[i] = st2[j]; dst_len[i] = ol[j];
-      if (found) found[i] = ck[j];
-      if (st2[j] == ZIPC_OK && ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
-    }
-  }
-  // stored members: one pass that copies and checksums
-  idx.clear();
-  std::vector<const uint8_t *> s1;
-  std::vector<uint8_t *> d1;
-  for (size_t i = 0; i < n; i++)
-    if (kind[i] == 1) { idx.push_back((uint32_t)i); s1.push_back(d_src[i]); d1.push_back(ctx->d_out.as<uint8_t>() + off[i]); }
-  if (int st = extract_stored(ctx, ms, idx, s1, d1, dst_len, found, status)) return st;
+  if (int st = extract_members(ctx, ms, n, d_src, slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n), &plan, dst_len, found, status))
+    return st;
   return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need, &plan);
 }
 
@@ -736,11 +714,12 @@ int zipc_b200_zip_extract_batch_dev(zipc_b200_ctx *ctx, const zipc_b200_member *
   DeviceGuard g(ctx->device);
   // every payload pointer must be device memory of this ctx's device: host members (zipc_b200_zip_parse_ex) passed here by
   // mistake are refused before anything runs.  One query per distinct pointer.
-  std::vector<const uint8_t *> seen;
+  std::vector<const uint8_t *> seen, d_src(n, nullptr);
   for (size_t i = 0; i < n; i++) {
     const zipc_b200_member &m = ms[i];
     int st_i;
     if (!member_kind(m, &st_i)) continue;
+    d_src[i] = m.compressed_bytes + m.start;
     if (!m.compressed_bytes) {
       if (m.compressed_size) return ZIPC_ERR_INVALID_ARG;
       continue;
@@ -752,36 +731,7 @@ int zipc_b200_zip_extract_batch_dev(zipc_b200_ctx *ctx, const zipc_b200_member *
     seen.push_back(m.compressed_bytes);
   }
   ctx->epoch++;  // the caller's device bytes may have changed since the last call
-  uint8_t *d_dst = static_cast<uint8_t *>(d_dst_v);
-  std::vector<uint32_t> i2, i1;
-  std::vector<const uint8_t *> s2, s1;
-  std::vector<uint8_t *> d2, d1;
-  std::vector<size_t> l2, c2;
-  for (size_t i = 0; i < n; i++) {
-    const zipc_b200_member &m = ms[i];
-    dst_len[i] = 0;
-    if (found) found[i] = 0;
-    const int kind = member_kind(m, &status[i]);
-    if (kind == 1) { i1.push_back((uint32_t)i); s1.push_back(m.compressed_bytes + m.start); d1.push_back(d_dst + dst_off[i]); }
-    if (kind == 2) {
-      i2.push_back((uint32_t)i); s2.push_back(m.compressed_bytes + m.start); d2.push_back(d_dst + dst_off[i]);
-      l2.push_back((size_t)m.compressed_size); c2.push_back((size_t)m.decompressed_size);
-    }
-  }
-  if (!i2.empty()) {
-    const size_t k = i2.size();
-    std::vector<size_t> ol(k);
-    std::vector<uint32_t> ck(k);
-    std::vector<int> st2(k);
-    if (int st = inflate_core(ctx, ZIPC_CK_CRC32, 0, k, s2, l2.data(), d2, c2, false, ol.data(), ck.data(), st2.data())) return st;
-    for (size_t j = 0; j < k; j++) {
-      const size_t i = i2[j];
-      status[i] = st2[j]; dst_len[i] = ol[j];
-      if (found) found[i] = ck[j];
-      if (st2[j] == ZIPC_OK && ck[j] != ms[i].crc32) status[i] = ZIPC_ERR_CHECKSUM;
-    }
-  }
-  return extract_stored(ctx, ms, i1, s1, d1, dst_len, found, status);
+  return extract_members(ctx, ms, n, d_src, slot_addrs(static_cast<uint8_t *>(d_dst_v), dst_off, n), nullptr, dst_len, found, status);
 }
 
 int zipc_b200_zip_deflate_archive(zipc_b200_ctx *ctx, int level, size_t n, const char *const *paths,
