@@ -360,6 +360,38 @@ int zipc_b200_zip_deflate_archive_ex(zipc_b200_ctx *ctx, int level, size_t n,
                                      const void *const *src, const size_t *src_len,
                                      const int32_t *mode, const int64_t *mtime, const char *first, unsigned flags,
                                      void *out, size_t out_cap, size_t *out_len);
+/* Device-resident File.deflate_of_binary_string / File.stored_of_binary_string + Member.make + Zipc.add +
+ * Zipc.to_binary_string (zipc.ml:171-185, 244-255, 308, 570-588): the archive of n payloads in device memory, written into
+ * device memory.
+ *   - Payload i is [src_off[i], src_off[i] + src_len[i]) of d_src, any alignment.  paths, path_len, mode, mtime, first and
+ *     flags are host values and mean what they mean for zipc_b200_zip_deflate_archive_ex: backslashes become slashes,
+ *     mode / mtime may be NULL, mtime is clamped to the DOS epoch, and the ZIPC_ZIP_* flags apply.
+ *   - compression[i] is 0 (stored, CRC-32 of the payload) or 8 (deflate at `level`); NULL deflates every member, as the
+ *     host call does.  Any other value: ZIPC_ERR_INVALID_ARG.
+ *   - d_src (when n > 0) and d_out must be device memory of the ctx's device; otherwise the call returns
+ *     ZIPC_ERR_INVALID_ARG before anything runs.
+ *   - The archive is [0, *out_len) of d_out, any alignment.  Every byte of that range is written once, nothing outside it
+ *     is written, and d_src is not modified.  If out_cap < *out_len the call returns ZIPC_ERR_DST_TOO_SMALL with *out_len
+ *     set to the size needed, and nothing of d_out is written.  zipc_b200_zip_archive_bound always suffices.
+ *   - Layout and bytes are those of the host call: `first` (default "mimetype") leads, then bytewise path order, a later
+ *     duplicate path shadowing an earlier one; header fields as File.make writes them (zipc.ml:138-143).  With all members
+ *     deflated the archive is byte for byte the one zipc_b200_zip_deflate_archive_ex returns; large deflate members are
+ *     cut into primed segments by the same rule.
+ *   - ZIPC_ERR_ZIP_COUNT, _PATH_LEN, _SIZE, _CD_OFFSET and _CD_SIZE come back under the host call's conditions, before
+ *     anything of d_out is written.  A deflate member must be smaller than 4 GiB; a stored member of 4 GiB or more is
+ *     accepted when ZIP64 is allowed (64-bit sizes in ZIP64 extra fields).
+ *   - n = 0 writes the 22-byte empty archive.  The call returns once the archive is complete in d_out. */
+int zipc_b200_zip_deflate_archive_dev(zipc_b200_ctx *ctx, int level, size_t n,
+                                      const char *const *paths, const uint32_t *path_len,
+                                      const void *d_src, const size_t *src_off, const size_t *src_len,
+                                      const int32_t *compression, const int32_t *mode, const int64_t *mtime,
+                                      const char *first, unsigned flags,
+                                      void *d_out, size_t out_cap, size_t *out_len);
+/* Upper bound of the archive zipc_b200_zip_deflate_archive_dev writes for these members, whatever segments the library cuts
+ * them into: per member its payload (src_len for a stored member, zipc_b200_zlib_bound(src_len) - 6 for a deflate one) and
+ * 30 + 20 + 46 + 28 + 2 path_len bytes of headers, ZIP64 extra fields included; then 56 + 20 + 22 bytes of end records.
+ * compression as above (NULL: all deflated).  0 if path_len or src_len is NULL and n > 0. */
+size_t zipc_b200_zip_archive_bound(size_t n, const uint32_t *path_len, const size_t *src_len, const int32_t *compression);
 
 /* ---- box-wide entry points (SURVEY.md 8b "device_mask", 8e) -------------------------------------------------------- */
 /* One call drives every selected GPU of the node: a multi-context owns one zipc_b200_ctx (stream, arenas) and one

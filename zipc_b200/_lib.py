@@ -36,7 +36,8 @@ EXPORTS = [
     "zipc_b200_zlib_bound", "zipc_b200_deflate_segmented", "zipc_b200_deflate_primed", "zipc_b200_inflate_segmented", "zipc_b200_ptime_to_dos", "zipc_b200_ptime_of_dos", "zipc_b200_zip_parse",
     "zipc_b200_zip_encoding_size", "zipc_b200_zip_assemble", "zipc_b200_zip_extract_batch",
     "zipc_b200_zip_parse_ex", "zipc_b200_zip_encoding_size_ex", "zipc_b200_zip_assemble_ex", "zipc_b200_inflate_plan", "zipc_b200_zip_deflate_archive_ex",
-    "zipc_b200_zip_deflate_archive", "zipc_b200_zip_parse_dev", "zipc_b200_zip_extract_batch_dev", "zipc_b200_free", "zipc_b200_synth_text", "zipc_b200_synth_rand",
+    "zipc_b200_zip_deflate_archive", "zipc_b200_zip_parse_dev", "zipc_b200_zip_extract_batch_dev", "zipc_b200_zip_deflate_archive_dev",
+    "zipc_b200_zip_archive_bound", "zipc_b200_free", "zipc_b200_synth_text", "zipc_b200_synth_rand",
     "zipc_b200_mctx_create", "zipc_b200_mctx_destroy", "zipc_b200_mctx_device_count", "zipc_b200_mctx_ctx",
     "zipc_b200_mctx_last_error", "zipc_b200_multi_crc32", "zipc_b200_multi_inflate_batch",
     "zipc_b200_multi_deflate_batch", "zipc_b200_multi_fetch",
@@ -113,6 +114,9 @@ def _declare(L):
                                                    C.c_char_p, C.c_uint, vp, sz, szp]),
         "zipc_b200_zip_parse_dev": (i32, [vp, vp, sz, C.c_uint, P(P(Member)), szp]),
         "zipc_b200_zip_extract_batch_dev": (i32, [vp, P(Member), sz, vp, szp, szp, u32p, ip]),
+        "zipc_b200_zip_deflate_archive_dev": (i32, [vp, i32, sz, vpp, u32p, vp, szp, szp, P(C.c_int32), P(C.c_int32),
+                                                    P(C.c_int64), C.c_char_p, C.c_uint, vp, sz, szp]),
+        "zipc_b200_zip_archive_bound": (sz, [sz, u32p, szp, P(C.c_int32)]),
         "zipc_b200_free": (None, [vp]),
         "zipc_b200_synth_text": (None, [u64, vp, sz]),
         "zipc_b200_synth_rand": (None, [u64, vp, sz]),

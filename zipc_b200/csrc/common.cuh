@@ -199,6 +199,85 @@ struct ZipEnd {       // what the end records say
 // locator in front of it (20)
 constexpr uint64_t kZipTailWindow = 65535 + 22 + 20;
 
+// ---- ZIP archive writing: the header bytes, for the host assembler (host_util.cc) and zip_headers_kernel (zip_api.cu) ----
+// One member's header fields, resolved (zip_hdr, host_util.cc).  big: bit 0 its sizes need 64 bits (a ZIP64 extra field in
+// both headers), bit 1 its local header offset does (in the directory entry's extra field).
+struct ZipHdr {
+  uint64_t lfh_at, cd_at;   // archive offsets of its local header and of its central directory entry
+  uint64_t csize, usize;
+  uint64_t name;            // zip_headers_kernel: offset of its path in the name blob
+  uint32_t crc, path_len;
+  uint32_t ext_attr;        // external attributes: MS-DOS bits in the low half, Unix mode and type in the high half
+  uint16_t made_by, needed, flags, method, time, date;
+  uint32_t big;
+};
+// the archive's end: member count and central directory, whether the ZIP64 end record and locator precede the EOCD
+struct ZipTail {
+  uint64_t count, cd_start, cd_size;
+  uint32_t eocd64, _pad;
+};
+__host__ __device__ inline void zip_put(uint8_t *b, uint64_t v, int bytes) {  // little endian, byte stores (any alignment)
+  for (int k = 0; k < bytes; k++) b[k] = (uint8_t)(v >> (8 * k));
+}
+__host__ __device__ inline uint64_t zip_lfh_size(uint32_t path_len, uint32_t big) { return 30 + path_len + ((big & 1) ? 20 : 0); }
+__host__ __device__ inline uint32_t zip_cd_extra_len(uint32_t big) { return big ? 4 + ((big & 1) ? 16 : 0) + ((big & 2) ? 8 : 0) : 0; }
+__host__ __device__ inline uint64_t zip_cdfh_size(uint32_t path_len, uint32_t big) { return 46 + path_len + zip_cd_extra_len(big); }
+// The local file header of h at b, its name read from `name` (zipc.ml:457-496; ZIP64 extra: APPNOTE 4.5.3).
+__host__ __device__ inline void zip_write_lfh(uint8_t *b, const ZipHdr &h, const char *name) {
+  const bool big = (h.big & 1) != 0;
+  zip_put(b, 0x04034b50u, 4);
+  zip_put(b + 4, big && h.needed < 45 ? 45 : h.needed, 2); zip_put(b + 6, h.flags, 2); zip_put(b + 8, h.method, 2);
+  zip_put(b + 10, h.time, 2); zip_put(b + 12, h.date, 2);
+  zip_put(b + 14, h.crc, 4); zip_put(b + 18, big ? 0xFFFFFFFFull : h.csize, 4); zip_put(b + 22, big ? 0xFFFFFFFFull : h.usize, 4);
+  zip_put(b + 26, h.path_len, 2); zip_put(b + 28, big ? 20 : 0, 2);
+  for (uint32_t k = 0; k < h.path_len; k++) b[30 + k] = (uint8_t)name[k];
+  if (big) {
+    uint8_t *x = b + 30 + h.path_len;
+    zip_put(x, 1, 2); zip_put(x + 2, 16, 2); zip_put(x + 4, h.usize, 8); zip_put(x + 12, h.csize, 8);
+  }
+}
+// The central directory entry of h at b (zipc.ml:498-545): the ZIP64 extra field holds exactly the overflowing values.
+__host__ __device__ inline void zip_write_cdfh(uint8_t *b, const ZipHdr &h, const char *name) {
+  const uint32_t bg = h.big, xlen = zip_cd_extra_len(bg);
+  zip_put(b, 0x02014b50u, 4);
+  zip_put(b + 4, h.made_by, 2); zip_put(b + 6, bg && h.needed < 45 ? 45 : h.needed, 2); zip_put(b + 8, h.flags, 2);
+  zip_put(b + 10, h.method, 2); zip_put(b + 12, h.time, 2); zip_put(b + 14, h.date, 2);
+  zip_put(b + 16, h.crc, 4); zip_put(b + 20, (bg & 1) ? 0xFFFFFFFFull : h.csize, 4); zip_put(b + 24, (bg & 1) ? 0xFFFFFFFFull : h.usize, 4);
+  zip_put(b + 28, h.path_len, 2);
+  zip_put(b + 30, xlen, 2); zip_put(b + 32, 0, 2); zip_put(b + 34, 0, 2); zip_put(b + 36, 0, 2);
+  zip_put(b + 38, h.ext_attr, 4);
+  zip_put(b + 42, (bg & 2) ? 0xFFFFFFFFull : h.lfh_at, 4);
+  for (uint32_t k = 0; k < h.path_len; k++) b[46 + k] = (uint8_t)name[k];
+  if (bg) {
+    uint8_t *x = b + 46 + h.path_len, *q = x + 4;
+    zip_put(x, 1, 2); zip_put(x + 2, xlen - 4, 2);
+    if (bg & 1) { zip_put(q, h.usize, 8); zip_put(q + 8, h.csize, 8); q += 16; }
+    if (bg & 2) zip_put(q, h.lfh_at, 8);
+  }
+}
+// bytes zip_write_end writes
+__host__ __device__ inline uint64_t zip_end_size(const ZipTail &t) { return (t.eocd64 ? 56 + 20 : 0) + 22; }
+// The end records at b = archive offset cd_start + cd_size: the ZIP64 end of central directory record and its locator
+// (APPNOTE 4.3.14, 4.3.15) when t.eocd64, then the EOCD (zipc.ml:553-566).
+__host__ __device__ inline void zip_write_end(uint8_t *b, const ZipTail &t) {
+  if (t.eocd64) {
+    zip_put(b, 0x06064b50u, 4); zip_put(b + 4, 44, 8);
+    zip_put(b + 12, 0x314 | 45, 2); zip_put(b + 14, 45, 2);
+    zip_put(b + 16, 0, 4); zip_put(b + 20, 0, 4);
+    zip_put(b + 24, t.count, 8); zip_put(b + 32, t.count, 8);
+    zip_put(b + 40, t.cd_size, 8); zip_put(b + 48, t.cd_start, 8);
+    zip_put(b + 56, 0x07064b50u, 4); zip_put(b + 60, 0, 4); zip_put(b + 64, t.cd_start + t.cd_size, 8); zip_put(b + 72, 1, 4);
+    b += 76;
+  }
+  const uint64_t c16 = t.count < 0xFFFF ? t.count : 0xFFFF;
+  zip_put(b, 0x06054b50u, 4);
+  zip_put(b + 4, 0, 2); zip_put(b + 6, 0, 2);
+  zip_put(b + 8, c16, 2); zip_put(b + 10, c16, 2);
+  zip_put(b + 12, t.cd_size < 0xFFFFFFFFull ? t.cd_size : 0xFFFFFFFFull, 4);
+  zip_put(b + 16, t.cd_start < 0xFFFFFFFFull ? t.cd_start : 0xFFFFFFFFull, 4);
+  zip_put(b + 20, 0, 2);
+}
+
 }  // namespace zb
 
 // ---- the context -------------------------------------------------------------------------------
@@ -393,7 +472,24 @@ int zip_walk_cd(const uint8_t *cd, uint64_t len, unsigned flags, const ZipEnd &e
 int zip_parse_finish(std::vector<zipc_b200_member> &ms, const std::vector<ZipLfh> &lfh, int cd_status, uint64_t len,
                      const uint8_t *bytes, const uint8_t *cd, uint64_t cd_size, bool cd_copy, zipc_b200_member **members,
                      size_t *n_out);
-// host_util.cc
+// host_util.cc: where everything of an archive goes (Zipc.to_binary_string, zipc.ml:447-455, 570-588).  Members in the
+// reference's order: `first` (default "mimetype") leads, then bytewise path order, a later duplicate path shadowing an
+// earlier one.  With ZIP64 allowed, a member whose sizes do not fit 32 bits gets a 20-byte ZIP64 extra field in its local
+// header (both sizes: APPNOTE 4.5.3) and its directory entry one that holds exactly the overflowing values (sizes, local
+// header offset).
+struct Layout {
+  std::vector<size_t> ord;       // members in archive order
+  std::vector<uint64_t> lfh_at;  // per ord index
+  std::vector<uint64_t> cd_at;   // per ord index: its central directory entry
+  std::vector<uint8_t> big;      // per ord index: ZipHdr::big
+  uint64_t cd_start = 0, cd_size = 0, total = 0;
+  bool eocd64 = false;
+};
+int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigned flags, Layout &L);
+// the header fields of member m, archive position j of L (File.make's values for a file, zipc.ml:138-143; directories as
+// zipc.ml:458-465, 499-507); name stays 0
+ZipHdr zip_hdr(const zipc_b200_member &m, const Layout &L, size_t j);
+inline ZipTail zip_tail(const Layout &L) { return ZipTail{L.ord.size(), L.cd_start, L.cd_size, L.eocd64, 0}; }
 int zip_assemble_impl(const zipc_b200_member *ms, size_t n, const char *first, void *out_v, size_t out_cap,
                       size_t *out_len, bool copy_payload, uint64_t *payload_off, unsigned flags = 0 /* ZIPC_ZIP_* */);
 // inflate.cu

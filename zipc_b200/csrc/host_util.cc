@@ -106,8 +106,6 @@ int64_t zipc_b200_ptime_of_dos(int dos_date, int dos_time) {  // zipc.ml:96-113
 // ---- little-endian field access --------------------------------------------------------------------
 static inline unsigned rd16(const uint8_t *b, size_t o) { return b[o] | (unsigned)b[o + 1] << 8; }
 static inline uint32_t rd32(const uint8_t *b, size_t o) { return rd16(b, o) | (uint32_t)rd16(b, o + 2) << 16; }
-static inline void wr16(uint8_t *b, size_t o, unsigned v) { b[o] = (uint8_t)v; b[o + 1] = (uint8_t)(v >> 8); }
-static inline void wr32(uint8_t *b, size_t o, uint32_t v) { wr16(b, o, v & 0xffff); wr16(b, o + 2, v >> 16); }
 
 static inline bool path_less(const zipc_b200_member &a, const zipc_b200_member &b) {  // String.compare
   size_t n = std::min(a.path_len, b.path_len);
@@ -130,7 +128,6 @@ static std::vector<size_t> map_order(const zipc_b200_member *ms, size_t n) {
 }
 
 static inline uint64_t rd64(const uint8_t *b, size_t o) { return rd32(b, o) | (uint64_t)rd32(b, o + 4) << 32; }
-static inline void wr64(uint8_t *b, size_t o, uint64_t v) { wr32(b, o, (uint32_t)v); wr32(b, o + 4, (uint32_t)(v >> 32)); }
 
 // ZIP64 extended information extra field (header id 0x0001, APPNOTE 4.5.3) of a central directory entry: the 64-bit
 // values stand in the fixed order uncompressed size, compressed size, local header offset, and only those whose 32-bit
@@ -334,42 +331,35 @@ uint64_t zipc_b200_zip_encoding_size(const zipc_b200_member *ms, size_t n) {
   return acc;
 }
 
-namespace {
-struct Hdr {  // the fields LFH and CDFH share, resolved for directories (zipc.ml:458-465, 499-507)
-  unsigned made_by, needed, flags, method, date, time;
-  uint32_t crc;
-  uint64_t csize, usize;
-};
-Hdr header_fields(const zipc_b200_member &m) {
-  Hdr h;
+}  // extern "C"
+
+namespace zb {
+ZipHdr zip_hdr(const zipc_b200_member &m, const Layout &L, size_t j) {
+  ZipHdr h;
+  std::memset(&h, 0, sizeof h);
   int date, time;
   zipc_b200_ptime_to_dos(m.mtime, &date, &time);
-  h.date = (unsigned)date;
-  h.time = (unsigned)time;
+  h.date = (uint16_t)date;
+  h.time = (uint16_t)time;
   if (m.is_dir) { h.made_by = 0x314; h.needed = 20; h.flags = 0x800; h.method = 0; h.crc = 0; h.csize = h.usize = 0; }
   else {
-    h.made_by = (unsigned)m.version_made_by;
-    h.needed = (unsigned)m.version_needed;
-    h.flags = (unsigned)m.gp_flags & ~8u;  // data-descriptor bit is never written (zipc.ml:442-445)
-    h.method = (unsigned)m.compression;
+    h.made_by = (uint16_t)m.version_made_by;
+    h.needed = (uint16_t)m.version_needed;
+    h.flags = (uint16_t)(m.gp_flags & ~8);  // data-descriptor bit is never written (zipc.ml:442-445)
+    h.method = (uint16_t)m.compression;
     h.crc = m.crc32;
     h.csize = m.compressed_size;
     h.usize = m.decompressed_size;
   }
+  h.ext_attr = (m.is_dir ? 0x10u : 0u) | ((m.is_dir ? 040000u : 0100000u) | ((unsigned)m.mode & 07777u)) << 16;
+  h.path_len = m.path_len;
+  h.lfh_at = L.lfh_at[j];
+  h.cd_at = L.cd_at[j];
+  h.big = L.big[j];
   return h;
 }
 
-// Where everything goes.  Classic format: zipc.ml:447-455.  With ZIP64 allowed, a member whose sizes do not fit 32 bits
-// gets a 20-byte ZIP64 extra field in its local header (both sizes: APPNOTE 4.5.3) and its directory entry one that holds
-// exactly the overflowing values (sizes, local header offset).
 constexpr uint64_t k32 = 0xFFFFFFFFull;
-struct Layout {
-  std::vector<size_t> ord;       // members in archive order
-  std::vector<uint64_t> lfh_at;  // per ord index
-  std::vector<uint8_t> big;      // per ord index: bit 0 sizes need 64 bits, bit 1 local header offset does
-  uint64_t cd_start = 0, cd_size = 0, total = 0;
-  bool eocd64 = false;
-};
 int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigned flags, Layout &L) {
   if (!first) first = "mimetype";
   const size_t flen = std::strlen(first);
@@ -386,6 +376,7 @@ int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigne
     }
   }
   L.lfh_at.resize(L.ord.size());
+  L.cd_at.resize(L.ord.size());
   L.big.assign(L.ord.size(), 0);
   uint64_t pos = 0;
   for (size_t j = 0; j < L.ord.size(); j++) {
@@ -399,12 +390,12 @@ int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigne
     if (force) L.big[j] |= 3;
     if (pos >= k32) L.big[j] |= 2;  // (only reachable with ZIP64 allowed: without it the directory offset check fails below)
     L.lfh_at[j] = pos;
-    pos += 30 + m.path_len + ((L.big[j] & 1) ? 20 : 0) + cs;
+    pos += zip_lfh_size(m.path_len, L.big[j]) + cs;
   }
   L.cd_start = pos;
   for (size_t j = 0; j < L.ord.size(); j++) {
-    const unsigned b = L.big[j];
-    pos += 46 + ms[L.ord[j]].path_len + (b ? 4 + ((b & 1) ? 16 : 0) + ((b & 2) ? 8 : 0) : 0);
+    L.cd_at[j] = pos;
+    pos += zip_cdfh_size(ms[L.ord[j]].path_len, L.big[j]);
   }
   L.cd_size = pos - L.cd_start;
   if (L.ord.empty()) L.cd_start = L.cd_size = 0;                       // zipc.ml:571-572
@@ -414,14 +405,10 @@ int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigne
     if (L.cd_size > k32) return ZIPC_ERR_ZIP_CD_SIZE;                  // zipc.ml:551
     L.eocd64 = false;
   }
-  L.total = pos + (L.eocd64 ? 56 + 20 : 0) + 22;
+  L.total = pos + zip_end_size(zip_tail(L));
   return ZIPC_OK;
 }
-}  // namespace
 
-}  // extern "C"
-
-namespace zb {
 // Archive layout engine behind zipc_b200_zip_assemble.  out_v == nullptr: compute *out_len and the
 // payload offsets only.  copy_payload == false: payloads are already in place (the GPU gathered them).
 // payload_off[i] (optional) receives the archive offset of member i's payload (members in caller order).
@@ -433,70 +420,20 @@ int zip_assemble_impl(const zipc_b200_member *ms, size_t n, const char *first, v
   const std::vector<size_t> &ord = L.ord;
   if (payload_off)
     for (size_t j = 0; j < ord.size(); j++)
-      payload_off[ord[j]] = L.lfh_at[j] + 30 + ms[ord[j]].path_len + ((L.big[j] & 1) ? 20 : 0);
+      payload_off[ord[j]] = L.lfh_at[j] + zip_lfh_size(ms[ord[j]].path_len, L.big[j]);
   if (!out_v) { *out_len = (size_t)L.total; return ZIPC_OK; }
   if (L.total > out_cap) { *out_len = (size_t)L.total; return ZIPC_ERR_DST_TOO_SMALL; }
   uint8_t *b = static_cast<uint8_t *>(out_v);
-  uint64_t pos = 0;
-  for (size_t j = 0; j < ord.size(); j++) {  // local headers + payloads (zipc.ml:457-496)
+  for (size_t j = 0; j < ord.size(); j++) {  // headers (common.cuh: the same writers as zip_headers_kernel) and payloads
     const zipc_b200_member &m = ms[ord[j]];
-    const Hdr h = header_fields(m);
-    const bool big = (L.big[j] & 1) != 0;
-    wr32(b, pos, 0x04034b50u);
-    wr16(b, pos + 4, big ? std::max(h.needed, 45u) : h.needed); wr16(b, pos + 6, h.flags); wr16(b, pos + 8, h.method);
-    wr16(b, pos + 10, h.time); wr16(b, pos + 12, h.date);
-    wr32(b, pos + 14, h.crc); wr32(b, pos + 18, big ? (uint32_t)k32 : (uint32_t)h.csize); wr32(b, pos + 22, big ? (uint32_t)k32 : (uint32_t)h.usize);
-    wr16(b, pos + 26, m.path_len); wr16(b, pos + 28, big ? 20 : 0);
-    std::memcpy(b + pos + 30, m.path, m.path_len);
-    pos += 30 + m.path_len;
-    if (big) { wr16(b, pos, 1); wr16(b, pos + 2, 16); wr64(b, pos + 4, h.usize); wr64(b, pos + 12, h.csize); pos += 20; }
-    if (!m.is_dir && m.compressed_size) {
-      if (copy_payload) std::memcpy(b + pos, m.compressed_bytes + m.start, m.compressed_size);
-      pos += m.compressed_size;
-    }
+    const ZipHdr h = zip_hdr(m, L, j);
+    zip_write_lfh(b + h.lfh_at, h, m.path);
+    zip_write_cdfh(b + h.cd_at, h, m.path);
+    if (copy_payload && !m.is_dir && m.compressed_size)
+      std::memcpy(b + h.lfh_at + zip_lfh_size(h.path_len, h.big), m.compressed_bytes + m.start, m.compressed_size);
   }
-  for (size_t j = 0; j < ord.size(); j++) {  // central directory (zipc.ml:498-545)
-    const zipc_b200_member &m = ms[ord[j]];
-    const Hdr h = header_fields(m);
-    const unsigned bg = L.big[j];
-    const unsigned xlen = bg ? 4 + ((bg & 1) ? 16 : 0) + ((bg & 2) ? 8 : 0) : 0;
-    wr32(b, pos, 0x02014b50u);
-    wr16(b, pos + 4, h.made_by); wr16(b, pos + 6, bg ? std::max(h.needed, 45u) : h.needed); wr16(b, pos + 8, h.flags); wr16(b, pos + 10, h.method);
-    wr16(b, pos + 12, h.time); wr16(b, pos + 14, h.date);
-    wr32(b, pos + 16, h.crc); wr32(b, pos + 20, (bg & 1) ? (uint32_t)k32 : (uint32_t)h.csize); wr32(b, pos + 24, (bg & 1) ? (uint32_t)k32 : (uint32_t)h.usize);
-    wr16(b, pos + 28, m.path_len);
-    wr16(b, pos + 30, xlen); wr16(b, pos + 32, 0); wr16(b, pos + 34, 0); wr16(b, pos + 36, 0);
-    wr16(b, pos + 38, m.is_dir ? 0x10 : 0);
-    wr16(b, pos + 40, (m.is_dir ? 040000u : 0100000u) | ((unsigned)m.mode & 07777u));
-    wr32(b, pos + 42, (bg & 2) ? (uint32_t)k32 : (uint32_t)L.lfh_at[j]);
-    std::memcpy(b + pos + 46, m.path, m.path_len);
-    pos += 46 + m.path_len;
-    if (bg) {
-      wr16(b, pos, 1); wr16(b, pos + 2, xlen - 4);
-      size_t q = pos + 4;
-      if (bg & 1) { wr64(b, q, h.usize); wr64(b, q + 8, h.csize); q += 16; }
-      if (bg & 2) wr64(b, q, L.lfh_at[j]);
-      pos += xlen;
-    }
-  }
-  if (L.eocd64) {  // ZIP64 end of central directory record + locator (APPNOTE 4.3.14, 4.3.15)
-    const uint64_t at = pos;
-    wr32(b, pos, 0x06064b50u); wr64(b, pos + 4, 44);
-    wr16(b, pos + 12, 0x314 | 45); wr16(b, pos + 14, 45);
-    wr32(b, pos + 16, 0); wr32(b, pos + 20, 0);
-    wr64(b, pos + 24, ord.size()); wr64(b, pos + 32, ord.size());
-    wr64(b, pos + 40, L.cd_size); wr64(b, pos + 48, L.cd_start);
-    pos += 56;
-    wr32(b, pos, 0x07064b50u); wr32(b, pos + 4, 0); wr64(b, pos + 8, at); wr32(b, pos + 16, 1);
-    pos += 20;
-  }
-  wr32(b, pos, 0x06054b50u);                                           // zipc.ml:553-566
-  wr16(b, pos + 4, 0); wr16(b, pos + 6, 0);
-  const unsigned c16 = (unsigned)std::min<uint64_t>(ord.size(), 0xFFFF);
-  wr16(b, pos + 8, c16); wr16(b, pos + 10, c16);
-  wr32(b, pos + 12, (uint32_t)std::min(L.cd_size, k32)); wr32(b, pos + 16, (uint32_t)std::min(L.cd_start, k32));
-  wr16(b, pos + 20, 0);
-  *out_len = (size_t)(pos + 22);
+  zip_write_end(b + L.cd_start + L.cd_size, zip_tail(L));
+  *out_len = (size_t)L.total;
   return ZIPC_OK;
 }
 }  // namespace zb

@@ -64,6 +64,27 @@ __global__ void zip_lfh_kernel(const uint8_t *__restrict__ archive, ZipLfh *f, u
   f[i] = h;
 }
 
+// One thread per member of an archive being written: its local header at lfh_at and its central directory entry at cd_at,
+// byte stores at any alignment of out; thread n writes the end records.  The writers are the host assembler's (common.cuh).
+__global__ void zip_headers_kernel(const ZipHdr *__restrict__ hdr, uint32_t n, const char *__restrict__ names, ZipTail tail,
+                                   uint8_t *__restrict__ out) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) {
+    const ZipHdr h = hdr[i];
+    zip_write_lfh(out + h.lfh_at, h, names + h.name);
+    zip_write_cdfh(out + h.cd_at, h, names + h.name);
+  } else if (i == n) {
+    zip_write_end(out + tail.cd_start + tail.cd_size, tail);
+  }
+}
+
+// p is device memory of the ctx's device (a host pointer handed to a _dev call by mistake is refused before anything runs)
+bool on_device(const zipc_b200_ctx *ctx, const void *p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return a.type == cudaMemoryTypeDevice && a.device == ctx->device;
+}
+
 // File.to_binary_string's dispatch (zipc.ml:205-217): 1 stored, 2 deflate, 0 nothing to extract (a directory, or a member
 // whose status this sets: encrypted, unsupported method)
 int member_kind(const zipc_b200_member &m, int *status) {
@@ -383,6 +404,38 @@ int place_zlib(zipc_b200_ctx *ctx, int level, size_t n, const Pieces &pc, const 
   return gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)nd);
 }
 
+// The paths of an archive's n members as Member.make keeps them (zipc.ml:244-255): backslashes become slashes.  Checked in
+// member order: the path's length, then the size of a member that is deflated (compression NULL: every member; the encoder
+// takes inputs below 4 GiB).
+int archive_paths(size_t n, const char *const *paths, const uint32_t *path_len, const size_t *src_len, const int32_t *compression,
+                  std::vector<std::string> &norm) {
+  norm.resize(n);
+  for (size_t i = 0; i < n; i++) {
+    if (path_len[i] > 0xFFFF) return ZIPC_ERR_ZIP_PATH_LEN;
+    if ((!compression || compression[i] == 8) && src_len[i] > 0xFFFFFFFFull) return ZIPC_ERR_ZIP_SIZE;
+    norm[i].assign(paths[i], path_len[i]);
+    for (char &c : norm[i]) if (c == '\\') c = '/';
+  }
+  return ZIPC_OK;
+}
+// File.make + Member.make over the n payloads (zipc.ml:138-143, 244-255): compression[i] (NULL: 8), clen[i] bytes of payload
+// for src_len[i] bytes of data, CRC-32 crc[i]; mode / mtime may be NULL
+void archive_members(size_t n, const std::vector<std::string> &norm, const int32_t *compression, const int32_t *mode,
+                     const int64_t *mtime, const size_t *src_len, const size_t *clen, const uint32_t *crc,
+                     std::vector<zipc_b200_member> &ms) {
+  ms.resize(n);
+  for (size_t i = 0; i < n; i++) {
+    zipc_b200_member &m = ms[i];
+    std::memset(&m, 0, sizeof m);
+    m.path = norm[i].data(); m.path_len = (uint32_t)norm[i].size();
+    m.mode = mode ? mode[i] : 0644;
+    m.mtime = mtime ? std::max<int64_t>(mtime[i], 315532800) : 315532800;
+    m.version_made_by = 0x314; m.version_needed = 20; m.gp_flags = 0x800;  // File.make defaults (zipc.ml:138-143)
+    m.compression = compression ? compression[i] : 8;
+    m.compressed_size = clen[i]; m.decompressed_size = src_len[i]; m.crc32 = crc[i];
+  }
+}
+
 }  // namespace
 
 int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaStream_t stream) {
@@ -515,6 +568,17 @@ int zipc_b200_zlib_compress_batch_dev(zipc_b200_ctx *ctx, int level, int adler_m
 //   L + 6 (L / 61440 + 2 nseg) + 1  <=  L + 6 (L / 61440 + 2) + 12 (L / 65536) + 1  <=  deflate_bound(L) + 12 (L / 65536)
 // bytes, 2 + 4 framing bytes around it.  (Level none is never split: stored blocks of 65534 bytes, within deflate_bound.)
 size_t zipc_b200_zlib_bound(size_t src_len) { return zipc_b200_deflate_bound(src_len) + 12 * (src_len / kSplitSegmentMin) + 6; }
+
+// Per member: its payload (a deflate body is a zlib stream without its 6 framing bytes), the local header with a ZIP64
+// extra field (30 + 20 + path), the directory entry with the longest one (46 + 28 + path); then the ZIP64 end record, its
+// locator and the EOCD.
+size_t zipc_b200_zip_archive_bound(size_t n, const uint32_t *path_len, const size_t *src_len, const int32_t *compression) {
+  if (n && (!path_len || !src_len)) return 0;
+  size_t b = 56 + 20 + 22;
+  for (size_t i = 0; i < n; i++)
+    b += (compression && compression[i] == 0 ? src_len[i] : zipc_b200_zlib_bound(src_len[i]) - 6) + 30 + 20 + 46 + 28 + 2 * (size_t)path_len[i];
+  return b;
+}
 
 // ---- segmented single stream -----------------------------------------------------------------------------
 static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size_t len, size_t segment_size,
@@ -725,9 +789,7 @@ int zipc_b200_zip_extract_batch_dev(zipc_b200_ctx *ctx, const zipc_b200_member *
       continue;
     }
     if (std::find(seen.begin(), seen.end(), m.compressed_bytes) != seen.end()) continue;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, m.compressed_bytes) != cudaSuccess) { cudaGetLastError(); return ZIPC_ERR_INVALID_ARG; }
-    if (a.type != cudaMemoryTypeDevice || a.device != ctx->device) return ZIPC_ERR_INVALID_ARG;
+    if (!on_device(ctx, m.compressed_bytes)) return ZIPC_ERR_INVALID_ARG;
     seen.push_back(m.compressed_bytes);
   }
   ctx->epoch++;  // the caller's device bytes may have changed since the last call
@@ -752,28 +814,13 @@ int zipc_b200_zip_deflate_archive_ex(zipc_b200_ctx *ctx, int level, size_t n, co
   DeviceGuard g(ctx->device);
   const bool zip64 = (flags & (ZIPC_ZIP_ALLOW_ZIP64 | ZIPC_ZIP_FORCE_ZIP64)) != 0;
   if (n > 0xFFFF && !zip64) return ZIPC_ERR_ZIP_COUNT;  // zipc.ml:574
-  // Member.make path rules (zipc.ml:244-255): backslashes become slashes; sizes are checked by File.make
-  std::vector<std::string> norm(n);
-  for (size_t i = 0; i < n; i++) {
-    if (path_len[i] > 0xFFFF) return ZIPC_ERR_ZIP_PATH_LEN;
-    if (src_len[i] > 0xFFFFFFFFull) return ZIPC_ERR_ZIP_SIZE;
-    norm[i].assign(paths[i], path_len[i]);
-    for (char &c : norm[i]) if (c == '\\') c = '/';
-  }
+  std::vector<std::string> norm;
+  if (int st = archive_paths(n, paths, path_len, src_len, nullptr, norm)) return st;
   std::vector<size_t> clen(n);
   std::vector<uint32_t> crc(n);
   std::vector<int> st_m(n);
   auto fill_members = [&](std::vector<zipc_b200_member> &ms) {
-    for (size_t i = 0; i < n; i++) {
-      zipc_b200_member &m = ms[i];
-      std::memset(&m, 0, sizeof m);
-      m.path = norm[i].data(); m.path_len = (uint32_t)norm[i].size();
-      m.mode = mode ? mode[i] : 0644;
-      m.mtime = mtime ? std::max<int64_t>(mtime[i], 315532800) : 315532800;
-      m.version_made_by = 0x314; m.version_needed = 20; m.gp_flags = 0x800;  // File.make defaults (zipc.ml:138-143)
-      m.compression = 8;
-      m.compressed_size = clen[i]; m.decompressed_size = src_len[i]; m.crc32 = crc[i];
-    }
+    archive_members(n, norm, nullptr, mode, mtime, src_len, clen.data(), crc.data(), ms);
   };
   // A large archive whose members come in path order (the order Zipc.to_binary_string writes them in, none of them the
   // `first` member unless it is the first anyway): through the pipeline, every group's payloads copied straight to their
@@ -830,6 +877,103 @@ int zipc_b200_zip_deflate_archive_ex(zipc_b200_ctx *ctx, int level, size_t n, co
   if (int st = compact_pieces(ctx, pc, off, total)) return st;
   if (int st = d2h(ctx, out, ctx->d_out.p, total)) return st;
   return zip_assemble_impl(ms.data(), n, first, out, out_cap, out_len, false, nullptr, flags);
+}
+
+// The archive of zipc_b200_zip_deflate_archive_ex written into device memory from device payloads, stored members allowed.
+// The deflate members are compressed as the host call compresses them, the layout is the host assembler's (make_layout), and
+// the GPU places everything: deflate pieces by one gather, stored members by stored_copy_crc (copy and CRC-32 in one pass),
+// headers and end records by zip_headers_kernel.
+int zipc_b200_zip_deflate_archive_dev(zipc_b200_ctx *ctx, int level, size_t n, const char *const *paths, const uint32_t *path_len,
+                                      const void *d_src_v, const size_t *src_off, const size_t *src_len, const int32_t *compression,
+                                      const int32_t *mode, const int64_t *mtime, const char *first, unsigned flags,
+                                      void *d_out_v, size_t out_cap, size_t *out_len) {
+  if (!ctx || level < 0 || level > 3 || !out_len || !d_out_v || (n && (!paths || !path_len || !d_src_v || !src_off || !src_len)))
+    return ZIPC_ERR_INVALID_ARG;
+  if (n > 0xFFFFFFF0ull) return ZIPC_ERR_INVALID_ARG;
+  for (size_t i = 0; compression && i < n; i++)
+    if (compression[i] != 0 && compression[i] != 8) return ZIPC_ERR_INVALID_ARG;
+  DeviceGuard g(ctx->device);
+  if (!on_device(ctx, d_out_v) || (n && !on_device(ctx, d_src_v))) return ZIPC_ERR_INVALID_ARG;
+  const bool zip64 = (flags & (ZIPC_ZIP_ALLOW_ZIP64 | ZIPC_ZIP_FORCE_ZIP64)) != 0;
+  if (n > 0xFFFF && !zip64) return ZIPC_ERR_ZIP_COUNT;  // zipc.ml:574
+  std::vector<std::string> norm;
+  if (int st = archive_paths(n, paths, path_len, src_len, compression, norm)) return st;
+  const uint8_t *base = static_cast<const uint8_t *>(d_src_v);
+  uint8_t *out = static_cast<uint8_t *>(d_out_v);
+  // 1. the deflate members, in member order, through the host call's path: the same pieces and bytes
+  std::vector<uint32_t> defl;
+  std::vector<const uint8_t *> d_src;
+  std::vector<size_t> dlen;
+  for (size_t i = 0; i < n; i++)
+    if (!compression || compression[i] == 8) { defl.push_back((uint32_t)i); d_src.push_back(base + src_off[i]); dlen.push_back(src_len[i]); }
+  const size_t nd = defl.size();
+  std::vector<size_t> dclen(nd);
+  std::vector<uint32_t> dcrc(nd);
+  std::vector<int> dst_m(nd);
+  Pieces pc;
+  if (int st = deflate_members(ctx, level, ZIPC_CK_CRC32, 0, nd, d_src, dlen.data(), dclen.data(), dcrc.data(), dst_m.data(), pc)) return st;
+  for (int s : dst_m) if (s) return s;
+  // 2. the host call's layout; a stored member's payload is its data, its CRC-32 comes with the copy (3)
+  std::vector<size_t> clen(src_len, src_len + n);
+  std::vector<uint32_t> crc(n, 0);
+  for (size_t k = 0; k < nd; k++) { clen[defl[k]] = dclen[k]; crc[defl[k]] = dcrc[k]; }
+  std::vector<zipc_b200_member> ms;
+  archive_members(n, norm, compression, mode, mtime, src_len, clen.data(), crc.data(), ms);
+  Layout L;
+  if (int st = make_layout(ms.data(), n, first, flags, L)) return st;
+  *out_len = (size_t)L.total;
+  if (out_cap < L.total) return ZIPC_ERR_DST_TOO_SMALL;
+  std::vector<uint64_t> poff(n, ~0ull);  // members shadowed by a later duplicate path keep ~0 and are not written
+  for (size_t j = 0; j < L.ord.size(); j++) poff[L.ord[j]] = L.lfh_at[j] + zip_lfh_size(ms[L.ord[j]].path_len, L.big[j]);
+  // 3. payloads: the deflate pieces by one gather, then the stored members
+  const size_t np = pc.member.size();
+  if (int st = ctx->h_desc.reserve(np * sizeof(CopyDesc))) return st;
+  if (int st = ctx->d_desc2.reserve(np * sizeof(CopyDesc))) return st;
+  CopyDesc *hc = ctx->h_desc.as<CopyDesc>();
+  size_t nc = 0;
+  for (size_t k = 0; k < np; k++) {
+    const uint64_t o = poff[defl[pc.member[k]]];
+    if (o != ~0ull && pc.len[k]) hc[nc++] = CopyDesc{pc.d_slot[k], out + o + pc.rel[k], pc.len[k]};
+  }
+  if (nc) {
+    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, hc, nc * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
+    if (int st = gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)nc)) return st;
+    ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (stored_copy_crc and the headers refill h_desc / d_desc2)
+  }
+  std::vector<uint32_t> stored;
+  std::vector<const uint8_t *> s_src;
+  std::vector<uint8_t *> s_dst;
+  std::vector<uint64_t> s_len;
+  for (size_t i = 0; compression && i < n; i++)
+    if (compression[i] == 0 && poff[i] != ~0ull) { stored.push_back((uint32_t)i); s_src.push_back(base + src_off[i]); s_dst.push_back(out + poff[i]); s_len.push_back(src_len[i]); }
+  std::vector<uint32_t> s_crc(stored.size());
+  if (int st = stored_copy_crc(ctx, stored.size(), s_src.data(), s_dst.data(), s_len.data(), s_crc.data())) return st;  // (synchronises)
+  for (size_t k = 0; k < stored.size(); k++) ms[stored[k]].crc32 = s_crc[k];
+  // 4. headers and end records: one record per member and the names behind them, one upload, one kernel
+  const size_t m = L.ord.size();
+  size_t name_bytes = 0;
+  for (size_t i : L.ord) name_bytes += ms[i].path_len;
+  const size_t rec_bytes = m * sizeof(ZipHdr);
+  if (int st = ctx->h_desc.reserve(rec_bytes + name_bytes)) return st;
+  if (int st = ctx->d_desc2.reserve(rec_bytes + name_bytes)) return st;
+  ZipHdr *hh = ctx->h_desc.as<ZipHdr>();
+  char *hn = reinterpret_cast<char *>(hh + m);
+  for (size_t j = 0, at = 0; j < m; j++) {
+    const zipc_b200_member &mb = ms[L.ord[j]];
+    hh[j] = zip_hdr(mb, L, j);
+    hh[j].name = at;
+    std::memcpy(hn + at, mb.path, mb.path_len);
+    at += mb.path_len;
+  }
+  if (rec_bytes + name_bytes)
+    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, hh, rec_bytes + name_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  const ZipHdr *dh = ctx->d_desc2.as<ZipHdr>();
+  zip_headers_kernel<<<(unsigned)((m + 1 + 255) / 256), 256, 0, ctx->stream>>>(dh, (uint32_t)m, reinterpret_cast<const char *>(dh + m),
+                                                                             zip_tail(L), out);
+  ctx->launches++;
+  ZB_CUDA(ctx, cudaGetLastError());
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
+  return ZIPC_OK;
 }
 
 }  // extern "C"
