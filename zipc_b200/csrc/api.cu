@@ -574,6 +574,9 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
   *ok = false;
   zipc_b200_ctx::ParPlan &plan = ctx->par_plan;
   if (plan.src == d_src && plan.src_len == src_len && plan.epoch == ctx->epoch && !plan.len.empty()) { *ok = true; return ZIPC_OK; }
+  // The key goes with the chunks: a speculation that stops part way (a pass that accepts nothing, no room for the symbols of
+  // a re-cut) returns with the chunks of its earlier passes in the plan, which must not pass for the previous stream's.
+  plan.src = nullptr; plan.src_len = 0; plan.epoch = 0;
   plan.len.clear(); plan.spec_off.clear(); plan.blocks.clear(); plan.total = 0;
   const uint64_t cb = par_chunk_bytes();
   const uint32_t nch0 = (uint32_t)((src_len + cb - 1) / cb);
