@@ -299,7 +299,7 @@ struct zipc_b200_ctx {
   zb::PinBuf h_stage, h_res, h_desc;
   cudaStream_t copy_stream = nullptr;  // progressive downloads (api.cu)
   cudaStream_t upload_stream = nullptr;  // late half of a split upload
-  cudaStream_t hi_stream = nullptr;      // high priority: compaction of a pipelined group (zip_api.cu compact)
+  cudaStream_t hi_stream = nullptr;      // high priority: placement gather of a pipelined group (zip_api.cu place_pieces)
   uint32_t *d_upflag = nullptr;        // device word: serial number of the last completed late half
   uint32_t upload_serial = 0;
   cudaEvent_t ev_block = nullptr;      // stream_sync of a sub-context
@@ -392,8 +392,6 @@ int deflate_launch(zipc_b200_ctx *ctx, const DeflateTask *d_tasks, uint32_t n, D
 // upper bound of the number of deflate blocks the encoder emits for an input of src_len bytes
 inline uint32_t deflate_max_blocks(uint64_t src_len) { return (uint32_t)(src_len / 61440) + 2; }
 constexpr uint32_t kStoredBlock = 65534;  // source bytes per block at level `None (reference :747-750, :1106-1116)
-// zip_api.cu: n independent copies on the device (compaction of per-member output slots)
-int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaStream_t stream = nullptr);
 // api.cu helpers shared with zip_api.cu
 int h2d(zipc_b200_ctx *ctx, void *d, const void *h, size_t bytes);
 int d2h(zipc_b200_ctx *ctx, void *h, const void *d, size_t bytes);
@@ -486,12 +484,14 @@ struct Layout {
   bool eocd64 = false;
 };
 int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigned flags, Layout &L);
+// the archive offset of every member's payload under L (members in caller order; ~0 for one shadowed by a later duplicate path)
+std::vector<uint64_t> payload_offsets(const std::vector<zipc_b200_member> &ms, const Layout &L);
 // the header fields of member m, archive position j of L (File.make's values for a file, zipc.ml:138-143; directories as
 // zipc.ml:458-465, 499-507); name stays 0
 ZipHdr zip_hdr(const zipc_b200_member &m, const Layout &L, size_t j);
 inline ZipTail zip_tail(const Layout &L) { return ZipTail{L.ord.size(), L.cd_start, L.cd_size, L.eocd64, 0}; }
 int zip_assemble_impl(const zipc_b200_member *ms, size_t n, const char *first, void *out_v, size_t out_cap,
-                      size_t *out_len, bool copy_payload, uint64_t *payload_off, unsigned flags = 0 /* ZIPC_ZIP_* */);
+                      size_t *out_len, bool copy_payload, unsigned flags = 0 /* ZIPC_ZIP_* */);
 // inflate.cu
 int inflate_launch(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, InflateResult *d_results,
                    bool count_only, int adler_mode /* -1: none */, unsigned int *d_group_count = nullptr,

@@ -409,18 +409,20 @@ int make_layout(const zipc_b200_member *ms, size_t n, const char *first, unsigne
   return ZIPC_OK;
 }
 
-// Archive layout engine behind zipc_b200_zip_assemble.  out_v == nullptr: compute *out_len and the
-// payload offsets only.  copy_payload == false: payloads are already in place (the GPU gathered them).
-// payload_off[i] (optional) receives the archive offset of member i's payload (members in caller order).
+std::vector<uint64_t> payload_offsets(const std::vector<zipc_b200_member> &ms, const Layout &L) {
+  std::vector<uint64_t> off(ms.size(), ~0ull);
+  for (size_t j = 0; j < L.ord.size(); j++) off[L.ord[j]] = L.lfh_at[j] + zip_lfh_size(ms[L.ord[j]].path_len, L.big[j]);
+  return off;
+}
+
+// Archive layout engine behind zipc_b200_zip_assemble.  out_v == nullptr: compute *out_len only.
+// copy_payload == false: payloads are already in place (the pipelined archive call put them there).
 int zip_assemble_impl(const zipc_b200_member *ms, size_t n, const char *first, void *out_v, size_t out_cap,
-                      size_t *out_len, bool copy_payload, uint64_t *payload_off, unsigned flags) {
+                      size_t *out_len, bool copy_payload, unsigned flags) {
   if (!out_len || (!ms && n)) return ZIPC_ERR_INVALID_ARG;
   Layout L;
   if (int st = make_layout(ms, n, first, flags, L)) return st;
   const std::vector<size_t> &ord = L.ord;
-  if (payload_off)
-    for (size_t j = 0; j < ord.size(); j++)
-      payload_off[ord[j]] = L.lfh_at[j] + zip_lfh_size(ms[ord[j]].path_len, L.big[j]);
   if (!out_v) { *out_len = (size_t)L.total; return ZIPC_OK; }
   if (L.total > out_cap) { *out_len = (size_t)L.total; return ZIPC_ERR_DST_TOO_SMALL; }
   uint8_t *b = static_cast<uint8_t *>(out_v);
@@ -443,20 +445,20 @@ extern "C" {
 int zipc_b200_zip_assemble(const zipc_b200_member *ms, size_t n, const char *first, void *out_v, size_t out_cap,
                            size_t *out_len) {
   if (!out_v) return ZIPC_ERR_INVALID_ARG;
-  return zb::zip_assemble_impl(ms, n, first, out_v, out_cap, out_len, true, nullptr, ZIPC_ZIP_REFERENCE);
+  return zb::zip_assemble_impl(ms, n, first, out_v, out_cap, out_len, true, ZIPC_ZIP_REFERENCE);
 }
 
 int zipc_b200_zip_assemble_ex(const zipc_b200_member *ms, size_t n, const char *first, unsigned flags, void *out_v,
                               size_t out_cap, size_t *out_len) {
   if (!out_v) return ZIPC_ERR_INVALID_ARG;
-  return zb::zip_assemble_impl(ms, n, first, out_v, out_cap, out_len, true, nullptr, flags);
+  return zb::zip_assemble_impl(ms, n, first, out_v, out_cap, out_len, true, flags);
 }
 
 // Zipc.encoding_size for an archive that may need ZIP64 structures (their presence depends on the offsets, hence `first`).
 // 0 if the members cannot be encoded under `flags`.
 uint64_t zipc_b200_zip_encoding_size_ex(const zipc_b200_member *ms, size_t n, const char *first, unsigned flags) {
   size_t total = 0;
-  if (zb::zip_assemble_impl(ms, n, first, nullptr, 0, &total, false, nullptr, flags)) return 0;
+  if (zb::zip_assemble_impl(ms, n, first, nullptr, 0, &total, false, flags)) return 0;
   return total;
 }
 

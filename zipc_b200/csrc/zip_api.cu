@@ -1,5 +1,5 @@
 // zip_api.cu -- deflate / zlib-compress / archive entry points of the C ABI (host orchestration) and the
-// device gather that compacts per-member output slots.
+// device gather that places the encoder's pieces (place_pieces: every compress call's output goes through it).
 //
 //   zipc_b200_deflate_batch        <- Zipc_deflate.deflate / crc_32_and_deflate / adler_32_and_deflate
 //                                     (reference src/zipc_deflate.ml:1247-1259)
@@ -8,7 +8,9 @@
 //                                     and outputs in device memory
 //   zipc_b200_zip_parse_dev        <- Zipc.of_binary_string (src/zipc.ml:400-438) of an archive in device memory
 //   zipc_b200_zip_deflate_archive  <- Zipc.File.deflate_of_binary_string + Zipc.to_binary_string
-//                                     (src/zipc.ml:179-185, 570-588)
+//                                     (src/zipc.ml:179-185, 570-588); _dev: payloads and archive in device memory.  Both
+//                                     write through plan_archive + write_archive; the host call uploads before and
+//                                     downloads after (a large batch in path order is pipelined instead)
 #include <algorithm>
 #include <cstring>
 #include <numeric>
@@ -133,7 +135,7 @@ int extract_members(zipc_b200_ctx *ctx, const zipc_b200_member *ms, size_t n, co
 }
 
 // Runs the encoder over n device-resident inputs.  Output of member i lands in a private slot
-// (d_slot[i], capacity slot_cap[i]); the caller compacts.  Checksums are of the INPUT (crc_op); Adler-32 is folded
+// (d_slot[i], capacity slot_cap[i]); the caller places it (place_pieces).  Checksums are of the INPUT (crc_op); Adler-32 is folded
 // per emitted block, which is what the reference's own zlib_decompress recomputes from the stream.
 int deflate_run(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n,
                 const std::vector<const uint8_t *> &d_src, const size_t *src_len,
@@ -257,32 +259,6 @@ int make_slots(zipc_b200_ctx *ctx, size_t n, const size_t *src_len, std::vector<
   return ZIPC_OK;
 }
 
-// Compacts slot outputs into ctx->d_out at the given offsets.
-int compact(zipc_b200_ctx *ctx, size_t n, const std::vector<uint8_t *> &d_slot, const size_t *len,
-            const std::vector<size_t> &off, size_t total) {
-  if (int st = ctx->d_out.reserve(total + 64)) return st;
-  if (int st = ctx->h_desc.reserve(n * sizeof(CopyDesc))) return st;
-  if (int st = ctx->d_desc2.reserve(n * sizeof(CopyDesc))) return st;
-  CopyDesc *h = ctx->h_desc.as<CopyDesc>();
-  for (size_t i = 0; i < n; i++) { h[i].src = d_slot[i]; h[i].dst = ctx->d_out.as<uint8_t>() + off[i]; h[i].len = len[i]; }
-  // A group of a pipelined batch compacts on a high-priority stream: its few CTAs then get the first SMs the running deflate
-  // kernel (of a later group) gives up, ahead of the deflate kernels already queued behind that one.  (The host has seen
-  // this group's results, so nothing on the context's stream is pending.)
-  cudaStream_t s = ctx->stream;
-  if (ctx->is_sub) {
-    if (!ctx->hi_stream) {
-      int lo = 0, hi = 0;
-      ZB_CUDA(ctx, cudaDeviceGetStreamPriorityRange(&lo, &hi));
-      ZB_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->hi_stream, cudaStreamNonBlocking, hi));
-    }
-    s = ctx->hi_stream;
-  }
-  ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, h, n * sizeof(CopyDesc), cudaMemcpyHostToDevice, s));
-  if (int st = gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)n, s)) return st;
-  if (s != ctx->stream) ZB_CUDA(ctx, stream_sync(ctx, s));
-  return ZIPC_OK;
-}
-
 // ---- large members over several CTAs -------------------------------------------------------------------------------------
 // A member of ZIPC_B200_SPLIT_MIN bytes or more (default 2 MiB, 320 KiB in a thin batch; 0 = never) is compressed as primed segments of 64 - 256 KiB, one
 // CTA each: every segment but the last ends with a byte-aligning empty stored block, every segment but the first sees the
@@ -295,6 +271,22 @@ struct Pieces {
   std::vector<uint8_t *> d_slot;         // piece -> where the kernel wrote it
   std::vector<size_t> len, rel;          // piece -> compressed length, offset inside its member's output
 };
+// The encoder inputs of one stream of len bytes at src cut into segments of seg bytes (one empty segment when len is 0),
+// appended to e_src / e_len / e_flags; returns their number.  Every segment but the last ends with a byte-aligning empty stored
+// block, the last one too unless last_final.  Primed, every segment but the first sees the (at most 32 KiB of) input before
+// it, in whole tiles.
+size_t cut_segments(const uint8_t *src, size_t len, size_t seg, bool primed, bool last_final, std::vector<const uint8_t *> &e_src,
+                    std::vector<size_t> &e_len, std::vector<uint32_t> &e_flags) {
+  const size_t nseg = len ? (len + seg - 1) / seg : 1;
+  for (size_t k = 0; k < nseg; k++) {
+    e_src.push_back(src + k * seg);
+    e_len.push_back(std::min(seg, len - k * seg));
+    uint32_t f = k + 1 < nseg || !last_final ? kDeflateNotFinal : 0u;
+    if (primed && k) f |= (uint32_t)(std::min<size_t>(k * seg, 32768) / kDeflatePrimeTile) << kDeflatePrimeShift;
+    e_flags.push_back(f);
+  }
+  return nseg;
+}
 int deflate_members(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n, const std::vector<const uint8_t *> &d_src,
                     const size_t *src_len, size_t *out_len, uint32_t *checksum, int *status, Pieces &pc) {
   // smallest member that is split: 2 MiB in a batch that fills the GPU with whole members anyway, 320 KiB in a thin one (fewer
@@ -324,15 +316,14 @@ int deflate_members(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_
     seg_bytes = (size_t)std::min<uint64_t>(kSplitSegment, std::max<uint64_t>(kSplitSegmentMin, (even + 4095) & ~4095ull));
   }
   for (size_t i = 0; i < n; i++) {
-    if (!may_split || src_len[i] < split_min) { e_src.push_back(d_src[i]); e_len.push_back(src_len[i]); e_flags.push_back(0u); pc.member.push_back((uint32_t)i); continue; }
-    any_split = true;
-    const size_t nseg = (src_len[i] + seg_bytes - 1) / seg_bytes;
-    for (size_t k = 0; k < nseg; k++) {
-      e_src.push_back(d_src[i] + k * seg_bytes);
-      e_len.push_back(std::min(seg_bytes, src_len[i] - k * seg_bytes));
-      e_flags.push_back((k + 1 < nseg ? kDeflateNotFinal : 0u) | (k ? (uint32_t)(32768 / kDeflatePrimeTile) << kDeflatePrimeShift : 0u));
-      pc.member.push_back((uint32_t)i);
+    size_t nseg = 1;
+    if (may_split && src_len[i] >= split_min) {
+      any_split = true;
+      nseg = cut_segments(d_src[i], src_len[i], seg_bytes, true, true, e_src, e_len, e_flags);
+    } else {
+      e_src.push_back(d_src[i]); e_len.push_back(src_len[i]); e_flags.push_back(0u);
     }
+    pc.member.insert(pc.member.end(), nseg, (uint32_t)i);
   }
   const size_t m = e_src.size();
   std::vector<size_t> cap, e_out(m);
@@ -367,41 +358,62 @@ int deflate_members(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_
     if (status[pc.member[k]] != ZIPC_OK) { pc.len[k] = 0; out_len[pc.member[k]] = 0; }
   return ZIPC_OK;
 }
-// the pieces to their places: member i's output starts at off[i] of ctx->d_out
-int compact_pieces(zipc_b200_ctx *ctx, const Pieces &pc, const std::vector<size_t> &off, size_t total) {
-  std::vector<size_t> poff(pc.member.size());
-  for (size_t k = 0; k < poff.size(); k++) poff[k] = off[pc.member[k]] + pc.rel[k];
-  return compact(ctx, poff.size(), pc.d_slot, pc.len.data(), poff, total);
+int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaStream_t stream) {
+  uint32_t grid = std::min<uint32_t>(n, (uint32_t)ctx->sm_count * 8);
+  gather_kernel<<<grid, 256, 0, stream>>>(d_descs, n);
+  ctx->launches++;
+  ZB_CUDA(ctx, cudaGetLastError());
+  return ZIPC_OK;
 }
 
-// zlib framing of the members deflate_members compressed into pc (reference :1264-1277): 2 header bytes at to[i], the body's
-// pieces behind them, the big-endian Adler-32 behind the body_len[i] bytes of body.  Header, pieces and trailer are placed
-// by one device gather (one descriptor table, one launch) at any alignment of to[i]; a member whose to[i] is null is left out.
-int place_zlib(zipc_b200_ctx *ctx, int level, size_t n, const Pieces &pc, const size_t *body_len, const uint32_t *adler,
-               const std::vector<uint8_t *> &to) {
-  const size_t np = pc.member.size();
-  const unsigned cmf = 0x78, hdr = (cmf << 8) | ((unsigned)level << 6), flg = (hdr + 31 - hdr % 31) & 0xFF;
-  if (int st = ctx->h_res.reserve(n * 8)) return st;
-  if (int st = ctx->d_res.reserve(n * 8)) return st;
-  if (int st = ctx->h_desc.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
-  if (int st = ctx->d_desc2.reserve((2 * n + np) * sizeof(CopyDesc))) return st;
-  uint8_t *hb = ctx->h_res.as<uint8_t>();
-  uint8_t *db = ctx->d_res.as<uint8_t>();
-  CopyDesc *h = ctx->h_desc.as<CopyDesc>();
+// The pieces of pc to their places: piece k of member i = pc.member[k] goes to to[i] + pc.rel[k], at any alignment.  A member
+// whose to[i] is null is left out (it failed, is shadowed, or its slot is too small).  With adler, each member is framed as a
+// zlib stream of that level (reference :1264-1277): 2 header bytes at to[i], the body 2 bytes further, the big-endian adler[i]
+// behind the body.  One descriptor table (framing bytes in front of it), one upload, one gather_kernel launch.  The copies are
+// left queued on the context's stream (a wait here would cost every small call its time): the caller waits for that stream
+// before the pinned table (ctx->h_desc) is refilled or the output is read.
+int place_pieces(zipc_b200_ctx *ctx, const Pieces &pc, const std::vector<uint8_t *> &to, const uint32_t *adler = nullptr,
+                 int level = 0) {
+  const size_t n = to.size(), np = pc.member.size(), nf = adler ? n : 0;
+  const size_t frame_bytes = 8 * nf, table_bytes = frame_bytes + (2 * nf + np) * sizeof(CopyDesc);
+  if (int st = ctx->h_desc.reserve(table_bytes)) return st;
+  if (int st = ctx->d_desc2.reserve(table_bytes)) return st;
+  uint8_t *hb = ctx->h_desc.as<uint8_t>(), *db = ctx->d_desc2.as<uint8_t>();
+  CopyDesc *h = reinterpret_cast<CopyDesc *>(hb + frame_bytes);
   size_t nd = 0;
-  for (size_t i = 0; i < n; i++) {
-    if (!to[i]) continue;
-    hb[8 * i] = (uint8_t)cmf; hb[8 * i + 1] = (uint8_t)flg;
-    hb[8 * i + 2] = (uint8_t)(adler[i] >> 24); hb[8 * i + 3] = (uint8_t)(adler[i] >> 16);
-    hb[8 * i + 4] = (uint8_t)(adler[i] >> 8); hb[8 * i + 5] = (uint8_t)adler[i];
-    h[nd++] = CopyDesc{db + 8 * i, to[i], 2};
-    h[nd++] = CopyDesc{db + 8 * i + 2, to[i] + 2 + body_len[i], 4};
+  if (adler) {
+    std::vector<size_t> body(n, 0);
+    for (size_t k = 0; k < np; k++) body[pc.member[k]] += pc.len[k];
+    const unsigned cmf = 0x78, hdr = (cmf << 8) | ((unsigned)level << 6), flg = (hdr + 31 - hdr % 31) & 0xFF;
+    for (size_t i = 0; i < n; i++) {
+      if (!to[i]) continue;
+      uint8_t *f = hb + 8 * i;
+      f[0] = (uint8_t)cmf; f[1] = (uint8_t)flg;
+      f[2] = (uint8_t)(adler[i] >> 24); f[3] = (uint8_t)(adler[i] >> 16); f[4] = (uint8_t)(adler[i] >> 8); f[5] = (uint8_t)adler[i];
+      h[nd++] = CopyDesc{db + 8 * i, to[i], 2};
+      h[nd++] = CopyDesc{db + 8 * i + 2, to[i] + 2 + body[i], 4};
+    }
   }
+  const size_t skip = adler ? 2 : 0;
   for (size_t k = 0; k < np; k++)
-    if (to[pc.member[k]]) h[nd++] = CopyDesc{pc.d_slot[k], to[pc.member[k]] + 2 + pc.rel[k], pc.len[k]};
-  ZB_CUDA(ctx, cudaMemcpyAsync(db, hb, n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, h, nd * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
-  return gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)nd);
+    if (to[pc.member[k]] && pc.len[k]) h[nd++] = CopyDesc{pc.d_slot[k], to[pc.member[k]] + skip + pc.rel[k], pc.len[k]};
+  if (!nd) return ZIPC_OK;
+  // A group of a pipelined batch places its pieces on a high-priority stream: its few CTAs then get the first SMs the running
+  // deflate kernel (of a later group) gives up, ahead of the deflate kernels already queued behind that one.  (The host has
+  // seen this group's results, so nothing on the context's stream is pending.)
+  cudaStream_t s = ctx->stream;
+  if (ctx->is_sub) {
+    if (!ctx->hi_stream) {
+      int lo = 0, hi = 0;
+      ZB_CUDA(ctx, cudaDeviceGetStreamPriorityRange(&lo, &hi));
+      ZB_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->hi_stream, cudaStreamNonBlocking, hi));
+    }
+    s = ctx->hi_stream;
+  }
+  ZB_CUDA(ctx, cudaMemcpyAsync(db, hb, frame_bytes + nd * sizeof(CopyDesc), cudaMemcpyHostToDevice, s));
+  if (int st = gather_launch(ctx, reinterpret_cast<const CopyDesc *>(db + frame_bytes), (uint32_t)nd, s)) return st;
+  if (s != ctx->stream) ZB_CUDA(ctx, stream_sync(ctx, s));
+  return ZIPC_OK;
 }
 
 // The paths of an archive's n members as Member.make keeps them (zipc.ml:244-255): backslashes become slashes.  Checked in
@@ -436,16 +448,89 @@ void archive_members(size_t n, const std::vector<std::string> &norm, const int32
   }
 }
 
-}  // namespace
-
-int gather_launch(zipc_b200_ctx *ctx, const CopyDesc *d_descs, uint32_t n, cudaStream_t stream) {
-  if (!n) return ZIPC_OK;
-  uint32_t grid = std::min<uint32_t>(n, (uint32_t)ctx->sm_count * 8);
-  gather_kernel<<<grid, 256, 0, stream ? stream : ctx->stream>>>(d_descs, n);
-  ctx->launches++;
-  ZB_CUDA(ctx, cudaGetLastError());
+// An archive of n members whose data are at d_src[i] (device memory), planned: compressed, described, laid out.  pc's pieces
+// name their archive member; poff: payload_offsets.
+struct ArchivePlan {
+  Pieces pc;
+  std::vector<zipc_b200_member> ms;
+  Layout L;
+  std::vector<uint64_t> poff;
+};
+// The deflate members (compression NULL: every member) go through deflate_members with CRC-32, in member order.  Returns the
+// first member's deflate status, then make_layout's; *out_len is set once the layout stands.  A stored member's CRC-32 comes
+// with its copy (write_archive).
+int plan_archive(zipc_b200_ctx *ctx, int level, size_t n, const std::vector<std::string> &norm, const std::vector<const uint8_t *> &d_src,
+                 const size_t *src_len, const int32_t *compression, const int32_t *mode, const int64_t *mtime, const char *first,
+                 unsigned flags, size_t *out_len, ArchivePlan &a) {
+  std::vector<uint32_t> defl;
+  std::vector<const uint8_t *> ds;
+  std::vector<size_t> dlen;
+  for (size_t i = 0; i < n; i++)
+    if (!compression || compression[i] == 8) { defl.push_back((uint32_t)i); ds.push_back(d_src[i]); dlen.push_back(src_len[i]); }
+  const size_t nd = defl.size();
+  std::vector<size_t> dclen(nd);
+  std::vector<uint32_t> dcrc(nd);
+  std::vector<int> dst_m(nd);
+  if (int st = deflate_members(ctx, level, ZIPC_CK_CRC32, 0, nd, ds, dlen.data(), dclen.data(), dcrc.data(), dst_m.data(), a.pc)) return st;
+  for (int s : dst_m) if (s) return s;
+  for (uint32_t &i : a.pc.member) i = defl[i];
+  std::vector<size_t> clen(src_len, src_len + n);
+  std::vector<uint32_t> crc(n, 0);
+  for (size_t k = 0; k < nd; k++) { clen[defl[k]] = dclen[k]; crc[defl[k]] = dcrc[k]; }
+  archive_members(n, norm, compression, mode, mtime, src_len, clen.data(), crc.data(), a.ms);
+  if (int st = make_layout(a.ms.data(), n, first, flags, a.L)) return st;
+  a.poff = payload_offsets(a.ms, a.L);
+  *out_len = (size_t)a.L.total;
   return ZIPC_OK;
 }
+// The planned archive into device memory at out (a.L.total bytes): the deflate pieces by place_pieces, the stored members
+// from d_src by stored_copy_crc (copy and CRC-32 in one pass), then the headers and end records by zip_headers_kernel from one
+// record per member and the names behind them, one upload.  Shadowed members are not written.  The stream is through on return.
+int write_archive(zipc_b200_ctx *ctx, ArchivePlan &a, const std::vector<const uint8_t *> &d_src, uint8_t *out) {
+  const size_t n = a.ms.size();
+  std::vector<uint8_t *> to(n, nullptr);
+  std::vector<uint32_t> stored;
+  std::vector<const uint8_t *> s_src;
+  std::vector<uint8_t *> s_dst;
+  std::vector<uint64_t> s_len;
+  for (size_t i = 0; i < n; i++) {
+    if (a.poff[i] == ~0ull) continue;
+    if (a.ms[i].compression == 8) to[i] = out + a.poff[i];
+    else { stored.push_back((uint32_t)i); s_src.push_back(d_src[i]); s_dst.push_back(out + a.poff[i]); s_len.push_back(a.ms[i].compressed_size); }
+  }
+  if (int st = place_pieces(ctx, a.pc, to)) return st;
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (place_pieces)
+  std::vector<uint32_t> s_crc(stored.size());
+  if (int st = stored_copy_crc(ctx, stored.size(), s_src.data(), s_dst.data(), s_len.data(), s_crc.data())) return st;
+  for (size_t k = 0; k < stored.size(); k++) a.ms[stored[k]].crc32 = s_crc[k];
+  const Layout &L = a.L;
+  const size_t m = L.ord.size();
+  size_t name_bytes = 0;
+  for (size_t i : L.ord) name_bytes += a.ms[i].path_len;
+  const size_t rec_bytes = m * sizeof(ZipHdr);
+  if (int st = ctx->h_desc.reserve(rec_bytes + name_bytes)) return st;
+  if (int st = ctx->d_desc2.reserve(rec_bytes + name_bytes)) return st;
+  ZipHdr *hh = ctx->h_desc.as<ZipHdr>();
+  char *hn = reinterpret_cast<char *>(hh + m);
+  for (size_t j = 0, at = 0; j < m; j++) {
+    const zipc_b200_member &mb = a.ms[L.ord[j]];
+    hh[j] = zip_hdr(mb, L, j);
+    hh[j].name = at;
+    std::memcpy(hn + at, mb.path, mb.path_len);
+    at += mb.path_len;
+  }
+  if (rec_bytes + name_bytes)
+    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, hh, rec_bytes + name_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  const ZipHdr *dh = ctx->d_desc2.as<ZipHdr>();
+  zip_headers_kernel<<<(unsigned)((m + 1 + 255) / 256), 256, 0, ctx->stream>>>(dh, (uint32_t)m, reinterpret_cast<const char *>(dh + m),
+                                                                             zip_tail(L), out);
+  ctx->launches++;
+  ZB_CUDA(ctx, cudaGetLastError());
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
+  return ZIPC_OK;
+}
+
+}  // namespace
 
 // One context's worth of zipc_b200_deflate_batch with a caller-defined layout of the outputs: `gap[i]` bytes (may be null)
 // are left free in front of output i and every output's length is rounded up to `align` -- (nullptr, 16) is the public
@@ -464,7 +549,8 @@ int deflate_batch_layout(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, 
   std::vector<size_t> off(n);
   size_t total = 0;
   for (size_t i = 0; i < n; i++) { off[i] = total + (gap ? gap[i] : 0); total = off[i] + align_up(dst_len[i], align); }
-  if (int st = compact_pieces(ctx, pc, off, total)) return st;
+  if (int st = ctx->d_out.reserve(total + 64)) return st;
+  if (int st = place_pieces(ctx, pc, slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n))) return st;
   const int rc = finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
   pipe_mark(ctx, "compacted");
   return rc;
@@ -527,7 +613,7 @@ int zipc_b200_zlib_compress_batch(zipc_b200_ctx *ctx, int level, int adler_mode,
   size_t total = 0;
   for (size_t i = 0; i < n; i++) { off[i] = total; flen[i] = dst_len[i] + 6; total += align_up(flen[i], 16); }
   if (int st = ctx->d_out.reserve(total + 64)) return st;
-  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n))) return st;
+  if (int st = place_pieces(ctx, pc, slot_addrs(ctx->d_out.as<uint8_t>(), off.data(), n), ad.data(), level)) return st;
   for (size_t i = 0; i < n; i++) { dst_len[i] = flen[i]; if (adler) adler[i] = ad[i]; }
   return finish_to_host(ctx, off, total, dst, dst_cap, dst_off, dst_need);
 }
@@ -550,8 +636,8 @@ int zipc_b200_zlib_compress_batch_dev(zipc_b200_ctx *ctx, int level, int adler_m
     if (status[i] == ZIPC_OK && (dst_cap_each[i] < 6 || dst_len[i] > dst_cap_each[i] - 6)) status[i] = ZIPC_ERR_DST_TOO_SMALL;
     if (status[i] == ZIPC_OK) to[i] = static_cast<uint8_t *>(d_dst_v) + dst_off[i];
   }
-  if (int st = place_zlib(ctx, level, n, pc, dst_len, ad.data(), to)) return st;
-  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (the gather reads the pinned descriptor table: it must be through before the next call)
+  if (int st = place_pieces(ctx, pc, to, ad.data(), level)) return st;
+  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (place_pieces)
   for (size_t i = 0; i < n; i++) {
     dst_len[i] = to[i] ? dst_len[i] + 6 : 0;
     if (adler) adler[i] = to[i] ? ad[i] : 0u;
@@ -594,34 +680,30 @@ static int deflate_segments(zipc_b200_ctx *ctx, int level, const void *src, size
   // input to the device (one copy), segments are slices of it
   const uint8_t *d_base;
   if (int st = upload_buffer(ctx, src, len, &d_base)) return st;
-  std::vector<const uint8_t *> d_src(nseg);
-  std::vector<size_t> slen(nseg);
-  std::vector<uint32_t> flags(nseg, kDeflateNotFinal);
-  for (size_t i = 0; i < nseg; i++) { d_src[i] = d_base + i * segment_size; slen[i] = std::min(segment_size, len - i * segment_size); }
-  if (last_piece) flags[nseg - 1] = 0;
-  if (primed)  // every segment but the first sees the 32 KiB of input before it (whole tiles of it)
-    for (size_t i = 1; i < nseg; i++) {
-      const size_t before = std::min<size_t>(i * segment_size, 32768) / kDeflatePrimeTile;
-      flags[i] |= (uint32_t)before << kDeflatePrimeShift;
-    }
-  std::vector<uint8_t *> d_slot;
-  std::vector<size_t> cap, clen(nseg);
+  std::vector<const uint8_t *> d_src;
+  std::vector<size_t> slen, cap;
+  std::vector<uint32_t> flags;
+  cut_segments(d_base, len, segment_size, primed, last_piece != 0, d_src, slen, flags);
+  Pieces pc;  // the pieces of one member, stream 0
+  pc.member.assign(nseg, 0);
+  pc.len.resize(nseg);
   std::vector<int> st_m(nseg);
-  if (int st = make_slots(ctx, nseg, slen.data(), d_slot, cap)) return st;
-  if (int st = deflate_run(ctx, level, ZIPC_CK_NONE, 0, nseg, d_src, slen.data(), d_slot, cap, clen.data(), nullptr, st_m.data(), &flags)) return st;
+  if (int st = make_slots(ctx, nseg, slen.data(), pc.d_slot, cap)) return st;
+  if (int st = deflate_run(ctx, level, ZIPC_CK_NONE, 0, nseg, d_src, slen.data(), pc.d_slot, cap, pc.len.data(), nullptr, st_m.data(), &flags)) return st;
   for (size_t i = 0; i < nseg; i++) if (st_m[i]) return st_m[i];
   if (crc32)
     if (int st = crc32_to_host_word(ctx, d_base, len)) return st;
   // the pieces are byte aligned: concatenate without gaps
-  std::vector<size_t> off(nseg);
+  pc.rel.resize(nseg);
   size_t total = 0;
-  for (size_t i = 0; i < nseg; i++) { off[i] = total; total += clen[i]; }
+  for (size_t i = 0; i < nseg; i++) { pc.rel[i] = total; total += pc.len[i]; }
   if (index) {
-    for (size_t i = 0; i < nseg; i++) { index[2 * i] = off[i]; index[2 * i + 1] = (uint64_t)i * segment_size; }
+    for (size_t i = 0; i < nseg; i++) { index[2 * i] = pc.rel[i]; index[2 * i + 1] = (uint64_t)i * segment_size; }
     index[2 * nseg] = total; index[2 * nseg + 1] = len;
   }
-  if (int st = compact(ctx, nseg, d_slot, clen.data(), off, total)) return st;
-  const int rc = finish_to_host(ctx, off, total, dst, dst_cap, nullptr, dst_len);
+  if (int st = ctx->d_out.reserve(total + 64)) return st;
+  if (int st = place_pieces(ctx, pc, {ctx->d_out.as<uint8_t>()})) return st;
+  const int rc = finish_to_host(ctx, {}, total, dst, dst_cap, nullptr, dst_len);
   if (crc32 && (rc == ZIPC_OK || rc == ZIPC_ERR_DST_TOO_SMALL)) *crc32 = host_word_crc32(ctx);
   return rc;
 }
@@ -816,12 +898,6 @@ int zipc_b200_zip_deflate_archive_ex(zipc_b200_ctx *ctx, int level, size_t n, co
   if (n > 0xFFFF && !zip64) return ZIPC_ERR_ZIP_COUNT;  // zipc.ml:574
   std::vector<std::string> norm;
   if (int st = archive_paths(n, paths, path_len, src_len, nullptr, norm)) return st;
-  std::vector<size_t> clen(n);
-  std::vector<uint32_t> crc(n);
-  std::vector<int> st_m(n);
-  auto fill_members = [&](std::vector<zipc_b200_member> &ms) {
-    archive_members(n, norm, nullptr, mode, mtime, src_len, clen.data(), crc.data(), ms);
-  };
   // A large archive whose members come in path order (the order Zipc.to_binary_string writes them in, none of them the
   // `first` member unless it is the first anyway): through the pipeline, every group's payloads copied straight to their
   // place in `out` while the later groups are compressed; the headers are written around them afterwards.
@@ -837,52 +913,41 @@ int zipc_b200_zip_deflate_archive_ex(zipc_b200_ctx *ctx, int level, size_t n, co
     if (pipe) {
       std::vector<uint32_t> gap(n);
       for (size_t i = 0; i < n; i++) gap[i] = 30u + (uint32_t)norm[i].size();
-      std::vector<size_t> poff(n);
+      std::vector<size_t> poff(n), clen(n);
+      std::vector<uint32_t> crc(n);
+      std::vector<int> st_m(n);
       size_t need = 0;
       const uint64_t l0 = pipeline_launches(pipe);
       const int rc = pipeline_deflate_gapped(pipe, level, n, src, src_len, gap.data(), out, out_cap, &need, poff.data(), clen.data(), crc.data(), st_m.data());
       ctx->launches += pipeline_launches(pipe) - l0;
       if (rc == ZIPC_OK) {
         for (size_t i = 0; i < n; i++) if (st_m[i]) return st_m[i];
-        std::vector<zipc_b200_member> ms(n);
-        fill_members(ms);
-        std::vector<uint64_t> want(n, ~0ull);
-        size_t total = 0;
-        if (int st = zip_assemble_impl(ms.data(), n, first, nullptr, 0, &total, false, want.data(), flags)) return st;
-        bool placed = true;
-        for (size_t i = 0; i < n && placed; i++) placed = want[i] == poff[i];
-        if (placed) return zip_assemble_impl(ms.data(), n, first, out, out_cap, out_len, false, nullptr, flags);
+        std::vector<zipc_b200_member> ms;
+        archive_members(n, norm, nullptr, mode, mtime, src_len, clen.data(), crc.data(), ms);
+        Layout L;
+        if (int st = make_layout(ms.data(), n, first, flags, L)) return st;
+        const std::vector<uint64_t> want = payload_offsets(ms, L);
+        if (std::equal(want.begin(), want.end(), poff.begin())) return zip_assemble_impl(ms.data(), n, first, out, out_cap, out_len, false, flags);
       } else if (rc != ZIPC_ERR_DST_TOO_SMALL) {
         return rc;
       }
       // (too small for the payloads, or not where the layout wants them: the plain path below reports / redoes it)
     }
   }
+  // the device call's steps between an upload and a download
   std::vector<const uint8_t *> d_src;
   if (int st = upload_ranges(ctx, n, src, src_len, d_src)) return st;
-  Pieces pc;
-  if (int st = deflate_members(ctx, level, ZIPC_CK_CRC32, 0, n, d_src, src_len, clen.data(), crc.data(), st_m.data(), pc)) return st;
-  for (size_t i = 0; i < n; i++) if (st_m[i]) return st_m[i];
-  std::vector<zipc_b200_member> ms(n);
-  fill_members(ms);
-  // layout first, then the GPU gathers every payload to its archive offset, then headers on the host
-  std::vector<uint64_t> poff(n, ~0ull);  // members shadowed by a later duplicate path keep ~0
-  size_t total = 0;
-  if (int st = zip_assemble_impl(ms.data(), n, first, nullptr, 0, &total, false, poff.data(), flags)) return st;
-  *out_len = total;
-  if (!out || out_cap < total) return ZIPC_ERR_DST_TOO_SMALL;
-  std::vector<size_t> off(n);
-  for (size_t i = 0; i < n; i++) off[i] = poff[i] != ~0ull ? (size_t)poff[i] : 0;
-  for (size_t k = 0; k < pc.member.size(); k++) if (poff[pc.member[k]] == ~0ull) pc.len[k] = 0;  // shadowed by a later duplicate path
-  if (int st = compact_pieces(ctx, pc, off, total)) return st;
-  if (int st = d2h(ctx, out, ctx->d_out.p, total)) return st;
-  return zip_assemble_impl(ms.data(), n, first, out, out_cap, out_len, false, nullptr, flags);
+  ArchivePlan a;
+  if (int st = plan_archive(ctx, level, n, norm, d_src, src_len, nullptr, mode, mtime, first, flags, out_len, a)) return st;
+  if (!out || out_cap < a.L.total) return ZIPC_ERR_DST_TOO_SMALL;
+  if (int st = ctx->d_out.reserve(a.L.total + 64)) return st;
+  if (int st = write_archive(ctx, a, d_src, ctx->d_out.as<uint8_t>())) return st;
+  return d2h(ctx, out, ctx->d_out.p, a.L.total);
 }
 
-// The archive of zipc_b200_zip_deflate_archive_ex written into device memory from device payloads, stored members allowed.
-// The deflate members are compressed as the host call compresses them, the layout is the host assembler's (make_layout), and
-// the GPU places everything: deflate pieces by one gather, stored members by stored_copy_crc (copy and CRC-32 in one pass),
-// headers and end records by zip_headers_kernel.
+// The archive of zipc_b200_zip_deflate_archive_ex written into device memory from device payloads, stored members allowed:
+// plan_archive, then write_archive into the caller's buffer.  The deflate members are compressed as the host call compresses
+// them, the layout is the host assembler's (make_layout), and the GPU places everything.
 int zipc_b200_zip_deflate_archive_dev(zipc_b200_ctx *ctx, int level, size_t n, const char *const *paths, const uint32_t *path_len,
                                       const void *d_src_v, const size_t *src_off, const size_t *src_len, const int32_t *compression,
                                       const int32_t *mode, const int64_t *mtime, const char *first, unsigned flags,
@@ -898,82 +963,11 @@ int zipc_b200_zip_deflate_archive_dev(zipc_b200_ctx *ctx, int level, size_t n, c
   if (n > 0xFFFF && !zip64) return ZIPC_ERR_ZIP_COUNT;  // zipc.ml:574
   std::vector<std::string> norm;
   if (int st = archive_paths(n, paths, path_len, src_len, compression, norm)) return st;
-  const uint8_t *base = static_cast<const uint8_t *>(d_src_v);
-  uint8_t *out = static_cast<uint8_t *>(d_out_v);
-  // 1. the deflate members, in member order, through the host call's path: the same pieces and bytes
-  std::vector<uint32_t> defl;
-  std::vector<const uint8_t *> d_src;
-  std::vector<size_t> dlen;
-  for (size_t i = 0; i < n; i++)
-    if (!compression || compression[i] == 8) { defl.push_back((uint32_t)i); d_src.push_back(base + src_off[i]); dlen.push_back(src_len[i]); }
-  const size_t nd = defl.size();
-  std::vector<size_t> dclen(nd);
-  std::vector<uint32_t> dcrc(nd);
-  std::vector<int> dst_m(nd);
-  Pieces pc;
-  if (int st = deflate_members(ctx, level, ZIPC_CK_CRC32, 0, nd, d_src, dlen.data(), dclen.data(), dcrc.data(), dst_m.data(), pc)) return st;
-  for (int s : dst_m) if (s) return s;
-  // 2. the host call's layout; a stored member's payload is its data, its CRC-32 comes with the copy (3)
-  std::vector<size_t> clen(src_len, src_len + n);
-  std::vector<uint32_t> crc(n, 0);
-  for (size_t k = 0; k < nd; k++) { clen[defl[k]] = dclen[k]; crc[defl[k]] = dcrc[k]; }
-  std::vector<zipc_b200_member> ms;
-  archive_members(n, norm, compression, mode, mtime, src_len, clen.data(), crc.data(), ms);
-  Layout L;
-  if (int st = make_layout(ms.data(), n, first, flags, L)) return st;
-  *out_len = (size_t)L.total;
-  if (out_cap < L.total) return ZIPC_ERR_DST_TOO_SMALL;
-  std::vector<uint64_t> poff(n, ~0ull);  // members shadowed by a later duplicate path keep ~0 and are not written
-  for (size_t j = 0; j < L.ord.size(); j++) poff[L.ord[j]] = L.lfh_at[j] + zip_lfh_size(ms[L.ord[j]].path_len, L.big[j]);
-  // 3. payloads: the deflate pieces by one gather, then the stored members
-  const size_t np = pc.member.size();
-  if (int st = ctx->h_desc.reserve(np * sizeof(CopyDesc))) return st;
-  if (int st = ctx->d_desc2.reserve(np * sizeof(CopyDesc))) return st;
-  CopyDesc *hc = ctx->h_desc.as<CopyDesc>();
-  size_t nc = 0;
-  for (size_t k = 0; k < np; k++) {
-    const uint64_t o = poff[defl[pc.member[k]]];
-    if (o != ~0ull && pc.len[k]) hc[nc++] = CopyDesc{pc.d_slot[k], out + o + pc.rel[k], pc.len[k]};
-  }
-  if (nc) {
-    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, hc, nc * sizeof(CopyDesc), cudaMemcpyHostToDevice, ctx->stream));
-    if (int st = gather_launch(ctx, ctx->d_desc2.as<CopyDesc>(), (uint32_t)nc)) return st;
-    ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));  // (stored_copy_crc and the headers refill h_desc / d_desc2)
-  }
-  std::vector<uint32_t> stored;
-  std::vector<const uint8_t *> s_src;
-  std::vector<uint8_t *> s_dst;
-  std::vector<uint64_t> s_len;
-  for (size_t i = 0; compression && i < n; i++)
-    if (compression[i] == 0 && poff[i] != ~0ull) { stored.push_back((uint32_t)i); s_src.push_back(base + src_off[i]); s_dst.push_back(out + poff[i]); s_len.push_back(src_len[i]); }
-  std::vector<uint32_t> s_crc(stored.size());
-  if (int st = stored_copy_crc(ctx, stored.size(), s_src.data(), s_dst.data(), s_len.data(), s_crc.data())) return st;  // (synchronises)
-  for (size_t k = 0; k < stored.size(); k++) ms[stored[k]].crc32 = s_crc[k];
-  // 4. headers and end records: one record per member and the names behind them, one upload, one kernel
-  const size_t m = L.ord.size();
-  size_t name_bytes = 0;
-  for (size_t i : L.ord) name_bytes += ms[i].path_len;
-  const size_t rec_bytes = m * sizeof(ZipHdr);
-  if (int st = ctx->h_desc.reserve(rec_bytes + name_bytes)) return st;
-  if (int st = ctx->d_desc2.reserve(rec_bytes + name_bytes)) return st;
-  ZipHdr *hh = ctx->h_desc.as<ZipHdr>();
-  char *hn = reinterpret_cast<char *>(hh + m);
-  for (size_t j = 0, at = 0; j < m; j++) {
-    const zipc_b200_member &mb = ms[L.ord[j]];
-    hh[j] = zip_hdr(mb, L, j);
-    hh[j].name = at;
-    std::memcpy(hn + at, mb.path, mb.path_len);
-    at += mb.path_len;
-  }
-  if (rec_bytes + name_bytes)
-    ZB_CUDA(ctx, cudaMemcpyAsync(ctx->d_desc2.p, hh, rec_bytes + name_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  const ZipHdr *dh = ctx->d_desc2.as<ZipHdr>();
-  zip_headers_kernel<<<(unsigned)((m + 1 + 255) / 256), 256, 0, ctx->stream>>>(dh, (uint32_t)m, reinterpret_cast<const char *>(dh + m),
-                                                                             zip_tail(L), out);
-  ctx->launches++;
-  ZB_CUDA(ctx, cudaGetLastError());
-  ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
-  return ZIPC_OK;
+  const std::vector<const uint8_t *> d_src = slot_addrs(static_cast<const uint8_t *>(d_src_v), src_off, n);
+  ArchivePlan a;
+  if (int st = plan_archive(ctx, level, n, norm, d_src, src_len, compression, mode, mtime, first, flags, out_len, a)) return st;
+  if (out_cap < a.L.total) return ZIPC_ERR_DST_TOO_SMALL;
+  return write_archive(ctx, a, d_src, static_cast<uint8_t *>(d_out_v));
 }
 
 }  // extern "C"
