@@ -135,8 +135,14 @@ extern "C" {
 // Order of the phases per tile t, as in the kernel (it matters: chain links of positions 32 KiB back are overwritten
 // by the insertion of the next tile, so that happens after the deep walks of this one): rounds of { P0(t) parse,
 // D(t) deep walks }, P1(t) final parse, I(t+1) insertion, S(t+1) shallow walks.
-int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **out_p, uint64_t *out_len) {
-  const uint32_t n = (uint32_t)n64;
+// One segment of a larger stream, as encode_member (deflate.cu) writes it: src[0, prime) is the input right before the
+// segment (a multiple of the tile), hashed and inserted into the chains but not searched, parsed or emitted; the parse
+// starts at `prime` with nothing pending and blocks count tiles from there.  A not_final segment keeps BFINAL off and ends
+// with a byte-aligning empty stored block.  prime = 0, not_final = 0 is a whole member (zipc_model_deflate).
+int zipc_model_deflate_ex(int level, const uint8_t *src, uint64_t n64, uint64_t prime64, int not_final, uint8_t **out_p,
+                          uint64_t *out_len) {
+  const uint32_t n = (uint32_t)n64, prime = (uint32_t)prime64;
+  if (prime % kTile || prime > n || (prime && prime == n)) return 1;
   LevelParams lp = level_params(level);
   Ring ring;
   Prev prev;
@@ -147,8 +153,8 @@ int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **ou
   std::vector<uint8_t> obuf((size_t)n + n / 8 + 1024);
   BitSink sink{obuf.data(), 0, 0, 0};
   Block blk;
-  blk.reset(0);
-  uint32_t pos = 0, kind = 0, loaded = 0;
+  blk.reset(prime);
+  uint32_t pos = prime, kind = 0, loaded = 0;
   int tiles_in_block = 0;
 
   auto insert = [&](uint32_t ts, int g) {
@@ -167,7 +173,7 @@ int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **ou
     mlen[g][0] = (uint16_t)carry_len; mdist[g][0] = (uint16_t)carry_dist;  // slot 0 holds position ts-1, slot 1+i holds ts+i
     for (uint32_t p = ts; p < te; p++) {
       uint32_t i = p - ts, l = 0, d = 0, rt = p & 0xFFFFu;
-      if (p + 4 <= n) {
+      if (p + 4 <= n && p >= prime) {
         MatchState m;
         match_begin(m, ring, p, n, tok[g][i], lp.shallow);
         while (!m.done) match_step(m, ring, prev, lp.shallow_nice);
@@ -182,6 +188,10 @@ int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **ou
   for (uint32_t ts = 0; ts < n; ts += kTile, g ^= 1) {
     const uint32_t te = std::min(ts + (uint32_t)kTile, n);
     std::vector<uint16_t> &ML = mlen[g], &MD = mdist[g], &TK = tok[g];
+    if (te <= prime) {  // a priming tile: nothing is parsed or emitted
+      insert(te, g ^ 1); shallow(te, g ^ 1, 0, 0);
+      continue;
+    }
     // D: visited positions continue their chain walk to the full depth; so do the positions a match taken there would land on
     // and their lazy look-ahead (inside this tile), up to lp.hops landings away (breadth first).  A position is deepened at
     // most once.
@@ -241,17 +251,28 @@ int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **ou
     bool last = te == n;
     if (tiles_in_block == kTilesPerBlock || last) {
       uint64_t next_start = blk.src_start + blk.src_len;
-      finalize_block(blk, src, last, sink);
+      finalize_block(blk, src, last && !not_final, sink);
       blk.reset(next_start);
       tiles_in_block = 0;
     }
   }
-  if (n == 0) finalize_block(blk, src, true, sink);
+  if (n == 0) finalize_block(blk, src, !not_final, sink);
+  if (not_final) {  // 000, pad to the byte, LEN 0, NLEN ffff
+    sink.put(0, 3);
+    sink.put(0, (8 - (sink.bits() & 7)) & 7);
+    sink.put(0, 16);
+    sink.put(0xFFFFu, 16);
+  }
   sink.flush();
   uint8_t *o = (uint8_t *)malloc(sink.pos ? sink.pos : 1);
   memcpy(o, obuf.data(), sink.pos);
   *out_p = o; *out_len = sink.pos;
   return 0;
 }
+int zipc_model_deflate(int level, const uint8_t *src, uint64_t n64, uint8_t **out_p, uint64_t *out_len) {
+  return zipc_model_deflate_ex(level, src, n64, 0, 0, out_p, out_len);
+}
+// The encoder's code length builder on its own: freq[nsym] (each < 2^23) -> out[nsym], at most max_bits.
+void zipc_model_huff_lengths(const uint32_t *freq, int nsym, int max_bits, uint8_t *out) { lengths_for(freq, nsym, max_bits, out); }
 void zipc_model_free(void *p) { free(p); }
 }

@@ -32,7 +32,8 @@ constexpr int kWindow = 32768;
 constexpr int kMinMatch = 4;
 constexpr int kMaxMatch = 258;
 constexpr int kTile = 2048;            // positions matched / parsed per step
-constexpr int kTilesPerBlock = 30;     // 61440 source bytes per deflate block (+ <= 257 of overhang)
+constexpr int kTilesPerBlock = 30;     // 61440 source bytes per deflate block (+ <= 257 of overhang, or one byte less when the
+                                       // lazy parse decides the token at a block's last position only in the next tile)
 constexpr int kHashBits = 14;
 constexpr int kRing = 65536;           // input ring in shared memory (power of two)
 constexpr int kNumLit = 286, kNumDist = 30, kNumClen = 19;
