@@ -89,7 +89,10 @@ void *zipc_b200_ctx_stream(zipc_b200_ctx *ctx);
 /* Number of kernels this ctx has launched so far (bench.py's gpu_launches). */
 uint64_t zipc_b200_ctx_launches(const zipc_b200_ctx *ctx);
 /* Diagnostics counters: 0 = kernels launched, 1 = large streams inflated in parallel inside the stream, 2 = large streams
- * whose parallel decoding did not check out and that were decoded by the serial path instead. */
+ * whose parallel decoding did not check out and that were decoded by the serial path instead, 3 = speculation passes of
+ * the parallel decoder (block-start search and speculative decode over what is left of a stream; a plan kept from the
+ * sizing pass of the same call runs none), 4 = chunks resolved by the parallel decoder.  A call without output sizes
+ * counts its large streams in 1 / 2 twice, once for the sizing pass and once for the real pass. */
 uint64_t zipc_b200_ctx_counter(const zipc_b200_ctx *ctx, int which);
 /* Diagnostics: when enabled, every call brackets its dominant kernel (CRC tiles / Adler chunks / inflate /
  * deflate) with CUDA events on the ctx stream; zipc_b200_ctx_kernel_ms returns the duration of the last

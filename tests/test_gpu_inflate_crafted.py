@@ -17,6 +17,7 @@ import pytest
 import deflate_writer as dw
 from oracle import zipc_oracle as zo
 from test_gpu_device_entry_points import _check_inflate_dev, dev, oracle_inflate  # noqa: F401  (dev: the fixture)
+from test_gpu_inflate_spec_plan import decode_pinned
 from zipc_b200 import _lib, synth
 from zipc_b200 import zipc_deflate as zd
 
@@ -287,13 +288,14 @@ def test_large_stream_match_before_the_start_in_a_later_chunk(ctx, monkeypatch):
 
 def test_large_stream_with_stored_deflate_streams_inside(ctx, monkeypatch):
     """stored blocks whose payload is itself a deflate stream (what storing a .gz or .png member gives), between text blocks:
-    the block-start search finds valid headers inside the payloads and the re-cut has to recover"""
+    the block-start search finds valid headers inside the payloads and the re-cut has to recover -- one re-cut per payload,
+    so twelve payloads take 13 of the 16 passes (24 of them used the passes up and fell back)"""
     monkeypatch.setenv("ZIPC_B200_PAR_MIN", "20000")
     monkeypatch.setenv("ZIPC_B200_PAR_CHUNK", "4096")
     rng = random.Random(4)
     text = synth.text_v1(4, 1 << 20).tobytes()
     w = dw.Writer()
-    for k in range(24):
+    for k in range(12):
         _block(w, rng, text, SHAPES[k % len(SHAPES)])
         inner = zlib.compressobj(6, zlib.DEFLATED, -15, 1)
         at = rng.randrange(len(text) - 70000)
@@ -304,15 +306,15 @@ def test_large_stream_with_stored_deflate_streams_inside(ctx, monkeypatch):
     s = w.finish()
     want = zo.inflate(s)
     assert want == bytes(w.out)
-    for ck, mode in ((_lib.CK_CRC32, 0), (_lib.CK_ADLER32, _lib.ADLER_REF_COMPAT)):
-        st, p0, p1 = _decode_like_oracle(ctx, s, [len(want), None], ck, mode)
-        assert st == [_lib.OK, _lib.OK]
-        print("stored deflate payloads: (parallel, fallback) %s -> %s" % (p0, p1))
+    plan = decode_pinned(ctx, s, [len(want), None], ((_lib.CK_CRC32, 0), (_lib.CK_ADLER32, _lib.ADLER_REF_COMPAT)))
+    assert plan.outcome == "parallel" and plan.recuts == 12, plan.describe()
 
 
-def test_more_spec_blocks_in_a_chunk_than_the_list_holds(ctx, monkeypatch):
+def test_sync_flushed_stream_over_the_block_list_falls_back(ctx, monkeypatch):
     """a text stream Z_SYNC_FLUSHed every ~30 bytes in its second half: far more than 256 non-empty blocks in one chunk, with
-    Adler-32 (the chunks report the lengths of their blocks for the fold): the oracle's output and fold"""
+    Adler-32 (the chunks report the lengths of their blocks for the fold).  The chunk's list overflows, on the re-cut too,
+    and the one-warp decoder gives the oracle's output and fold; block_list_256 of tests/par_inflate_inputs.py is a chunk of
+    256 blocks that the many-warp decoder takes."""
     monkeypatch.setenv("ZIPC_B200_PAR_MIN", "20000")
     monkeypatch.setenv("ZIPC_B200_PAR_CHUNK", "16384")
     data = synth.text_v1(5, 3 << 20).tobytes()
@@ -323,10 +325,9 @@ def test_more_spec_blocks_in_a_chunk_than_the_list_holds(ctx, monkeypatch):
         parts.append(c.compress(data[i:i + 30]) + c.flush(zlib.Z_SYNC_FLUSH))
     parts.append(c.compress(data[half + 600_000:]) + c.flush())
     s = b"".join(parts)
-    for mode in (_lib.ADLER_REF_COMPAT, _lib.ADLER_RFC1950):
-        st, p0, p1 = _decode_like_oracle(ctx, s, [len(data), None], _lib.CK_ADLER32, mode)
-        assert st == [_lib.OK, _lib.OK]
-        print("sync-flushed stream: (parallel, fallback) %s -> %s" % (p0, p1))
+    plan = decode_pinned(ctx, s, [len(data), None], ((_lib.CK_ADLER32, _lib.ADLER_REF_COMPAT), (_lib.CK_ADLER32, _lib.ADLER_RFC1950)),
+                         chunk=16384)
+    assert plan.outcome == "block_list", plan.describe()
 
 
 # ==== the plan cache of the many-warp decoder ==============================================================================

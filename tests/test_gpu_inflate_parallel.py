@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 from oracle import zipc_oracle as zo
+from test_gpu_inflate_spec_plan import decode_pinned
 from zipc_b200 import _lib, synth
 from zipc_b200 import zipc_deflate as zd
 
@@ -56,16 +57,19 @@ def test_large_zlib_streams(ctx, level):
 
 def test_mixed_content_and_block_kinds(ctx):
     """text, incompressible stretches (stored blocks), runs (long matches, distance 1), binary structure; also streams made
-    with Z_FIXED (no dynamic block anywhere: nothing to find, serial path) and Z_HUFFMAN_ONLY / Z_RLE"""
+    with Z_FIXED (no dynamic block anywhere: nothing to find, serial path) and Z_HUFFMAN_ONLY / Z_RLE.  Each takes the path
+    and the passes and chunks of tests/par_inflate_model.py's plan: under Z_RLE and Z_FILTERED the 500,000 zero bytes come
+    out of a chunk at more than 24 times its compressed size, and the one-warp decoder takes the stream."""
     rnd = random.Random(9)
     t = synth.text_v1(77, 3 << 20).tobytes()
     parts = [t[:900000], rnd.randbytes(300000), bytes(500000), t[900000:2000000], bytes(range(256)) * 2000, rnd.randbytes(70000), t[2000000:]]
     data = b"".join(parts)
     for level, strategy in ((6, zlib.Z_DEFAULT_STRATEGY), (1, zlib.Z_DEFAULT_STRATEGY), (6, zlib.Z_RLE), (6, zlib.Z_HUFFMAN_ONLY), (6, zlib.Z_FILTERED)):
         stream = _raw(data, level, strategy)
-        _check(ctx, stream, data)
-    stream = _raw(t, 6, zlib.Z_FIXED)
-    _check(ctx, stream, t, expect_parallel=False)
+        plan = decode_pinned(ctx, stream, [len(data), None], chunk=8192, par_min=None)
+        assert plan.outcome == ("symbol_budget" if strategy in (zlib.Z_RLE, zlib.Z_FILTERED) else "parallel"), plan.describe()
+    plan = decode_pinned(ctx, _raw(t, 6, zlib.Z_FIXED), [len(t), None], chunk=8192, par_min=None)
+    assert plan.outcome == "no_start"
 
 
 def test_stream_made_by_the_oracle_and_by_us(ctx):
@@ -84,10 +88,12 @@ def test_small_chunks_and_thresholds(ctx, monkeypatch):
         for level in (1, 6):
             c = zlib.compressobj(level, zlib.DEFLATED, -15, 1)  # memLevel 1: small blocks
             stream = c.compress(data) + c.flush()
-            _check(ctx, stream, data)
-    # one single dynamic block (the reference's own fixture shape): nothing to split, the serial path answers
+            plan = decode_pinned(ctx, stream, [len(data), None], chunk=4096, par_min=20000)
+            assert plan.outcome == "parallel" and len(plan.chunks) > 4, plan.describe()
+    # the reference's own fixture size at level 9: zlib writes it in two dynamic blocks, and the second is found
     data = synth.text_v1(9, 174_585).tobytes()
-    _check(ctx, _raw(data, 9), data)
+    plan = decode_pinned(ctx, _raw(data, 9), [len(data), None], chunk=4096, par_min=20000)
+    assert plan.outcome == "parallel" and len(plan.chunks) == 2, plan.describe()
 
 
 def test_corrupt_large_streams_have_the_reference_status(ctx):

@@ -570,7 +570,7 @@ static zipc_b200_mctx *par_lanes(zipc_b200_ctx *ctx, size_t lanes) {
 
 static bool par_debug() { static const bool v = env_u64("ZIPC_B200_PAR_DEBUG", 0) != 0; return v; }
 
-static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_len, bool *ok) {
+static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_len, bool *ok, uint64_t *passes) {
   *ok = false;
   zipc_b200_ctx::ParPlan &plan = ctx->par_plan;
   if (plan.src == d_src && plan.src_len == src_len && plan.epoch == ctx->epoch && !plan.len.empty()) { *ok = true; return ZIPC_OK; }
@@ -600,6 +600,7 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
   uint64_t spec_used = 0;     // symbols of d_spec taken by accepted chunks
   uint64_t spec_cap = 0;      // symbols d_spec holds (fixed by the first pass: later passes must not move the buffer)
   for (int pass = 0; pass < 16; pass++) {
+    ++*passes;
     const double t_begin = par_debug() ? (cudaStreamSynchronize(ctx->stream), now_ms()) : 0;
     const uint64_t left_bits = 8ull * src_len - from_bit;
     const uint32_t nch = (uint32_t)std::min<uint64_t>(nch0, (left_bits + 8 * cb - 1) / (8 * cb));
@@ -680,9 +681,10 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
   return ZIPC_OK;
 }
 
-static int par_resolve(zipc_b200_ctx *ctx, uint8_t *d_dst, bool *ok) {
+static int par_resolve(zipc_b200_ctx *ctx, uint8_t *d_dst, bool *ok, uint64_t *chunks) {
   const zipc_b200_ctx::ParPlan &plan = ctx->par_plan;
   const uint32_t m = (uint32_t)plan.len.size();
+  *chunks += m;
   *ok = false;
   const double t_begin = par_debug() ? (cudaStreamSynchronize(ctx->stream), now_ms()) : 0;
   std::vector<uint64_t> tab(3 * (size_t)m);
@@ -725,16 +727,16 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
     std::vector<uint32_t> sel;
     for (size_t j = 0; j < rest.size(); j++) if (take[j]) sel.push_back(rest[j]);
     // one stream through the many-warp decoder, on context c (ctx itself, or one of its lanes)
-    auto one = [&](zipc_b200_ctx *c, uint32_t i, uint64_t &streams, uint64_t &fallbacks) -> int {
+    auto one = [&](zipc_b200_ctx *c, uint32_t i, zipc_b200_ctx::ParCounts &count) -> int {
       bool ok = false;
-      if (int st = par_speculate(c, d_src[i], src_len[i], &ok)) {
+      if (int st = par_speculate(c, d_src[i], src_len[i], &ok, &count.passes)) {
         if (st != ZIPC_ERR_NOMEM) return st;
         ok = false;  // no room for this stream's symbols (24 x its compressed size): the one-warp decoder needs none
       }
       const uint64_t total = c->par_plan.total;
       if (ok && cap[i] != ZIPC_SIZE_UNKNOWN && total > cap[i]) ok = false;  // the serial decoder reports the exact error
       if (ok && !count_only) {
-        if (int st = par_resolve(c, d_dst[i], &ok)) { if (st != ZIPC_ERR_NOMEM) return st; ok = false; }
+        if (int st = par_resolve(c, d_dst[i], &ok, &count.chunks)) { if (st != ZIPC_ERR_NOMEM) return st; ok = false; }
         if (ok && checksum) {
           checksum[i] = 0;
           if (ck == ZIPC_CK_CRC32) {
@@ -754,13 +756,13 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
           }
         }
       }
-      if (ok) { done[i] = 1; status[i] = ZIPC_OK; out_len[i] = (size_t)total; streams++; }
-      else fallbacks++;
+      if (ok) { done[i] = 1; status[i] = ZIPC_OK; out_len[i] = (size_t)total; count.streams++; }
+      else count.fallbacks++;
       return ZIPC_OK;
     };
     zipc_b200_mctx *pool = sel.size() >= 2 && lanes >= 2 ? par_lanes(ctx, lanes) : nullptr;
     if (!pool) {
-      for (uint32_t i : sel) if (int st = one(ctx, i, ctx->par_streams, ctx->par_fallbacks)) return st;
+      for (uint32_t i : sel) if (int st = one(ctx, i, ctx->par_counts)) return st;
     } else {
       // Several streams at a time: lane k is a host thread with a sub-context (stream, scratch arenas) of its own.  The streams
       // are dealt out largest first, each to the lane with the least compressed bytes so far (the same deal in the sizing pass and
@@ -794,7 +796,7 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
       for (uint32_t i : sel) sel_bytes += (double)src_len[i];
       const double active_bytes = std::max(1.0, sel_bytes * (double)L / (double)sel.size());  // (L of the sel.size() streams at a time)
       std::vector<int> rc(L, ZIPC_OK);
-      std::vector<uint64_t> ns(L, 0), nf(L, 0);
+      std::vector<zipc_b200_ctx::ParCounts> counts(L);
       std::vector<std::thread> th;
       auto lane = [&](size_t k) {
         zipc_b200_ctx *c = zipc_b200_mctx_ctx(pool, (int)k);
@@ -805,14 +807,15 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
           // this stream's share of the SMs for its speculative decode (a CTA of that kernel owns its SM): by its size among the
           // streams that are under way at the same time
           c->sm_share = (uint32_t)std::min<double>(ctx->sm_count, std::max(2.0, ctx->sm_count * (double)src_len[i] / active_bytes));
-          if ((rc[k] = one(c, i, ns[k], nf[k])) != ZIPC_OK) return;
+          if ((rc[k] = one(c, i, counts[k])) != ZIPC_OK) return;
         }
       };
       for (size_t k = 1; k < L; k++) th.emplace_back(lane, k);
       lane(0);
       for (auto &t : th) t.join();
       for (size_t k = 0; k < L; k++) {
-        ctx->par_streams += ns[k]; ctx->par_fallbacks += nf[k];
+        ctx->par_counts.streams += counts[k].streams; ctx->par_counts.fallbacks += counts[k].fallbacks;
+        ctx->par_counts.passes += counts[k].passes; ctx->par_counts.chunks += counts[k].chunks;
         if (rc[k]) { ctx->last_error = zipc_b200_last_error(zipc_b200_mctx_ctx(pool, (int)k)); return rc[k]; }
       }
     }
@@ -987,7 +990,8 @@ void *zipc_b200_ctx_stream(zipc_b200_ctx *ctx) { return ctx ? (void *)ctx->strea
 uint64_t zipc_b200_ctx_launches(const zipc_b200_ctx *ctx) { return ctx ? ctx->launches + (ctx->par_pool ? pipeline_launches(ctx->par_pool) : 0) : 0; }
 uint64_t zipc_b200_ctx_counter(const zipc_b200_ctx *ctx, int which) {
   if (!ctx) return 0;
-  return which == 0 ? ctx->launches : which == 1 ? ctx->par_streams : which == 2 ? ctx->par_fallbacks : 0;
+  const zipc_b200_ctx::ParCounts &p = ctx->par_counts;
+  return which == 0 ? ctx->launches : which == 1 ? p.streams : which == 2 ? p.fallbacks : which == 3 ? p.passes : which == 4 ? p.chunks : 0;
 }
 void zipc_b200_ctx_profile(zipc_b200_ctx *ctx, int enable) {
   if (!ctx) return;

@@ -324,7 +324,9 @@ struct zipc_b200_ctx {
   zb::DevBuf d_adler_chain;          // adler32.cu: tile counter + the two chains of the REF_COMPAT fold (tagged by adler_epoch)
   uint32_t adler_epoch = 0;
   void *adler_ticket_at = nullptr;   // where the counter was last zeroed (the kernel resets it itself afterwards)
-  uint64_t par_streams = 0, par_fallbacks = 0;   // diagnostics: large streams decoded in parallel / handed back to the serial path
+  // diagnostics of the many-warp decoder: large streams decoded in parallel / handed back to the serial path, speculation
+  // passes run (plans served from the cache run none), chunks resolved
+  struct ParCounts { uint64_t streams = 0, fallbacks = 0, passes = 0, chunks = 0; } par_counts;
 
   // pipelining (multi.cc): a sub-context waits for its turn to upload; the parent owns the sub-contexts
   zb::UploadGate *gate = nullptr;

@@ -140,6 +140,12 @@ class Context:
         """(large streams inflated in parallel inside the stream, large streams handed back to the one-warp decoder)"""
         return self.L.zipc_b200_ctx_counter(self.h, 1), self.L.zipc_b200_ctx_counter(self.h, 2)
 
+    @property
+    def parallel_counters(self) -> tuple[int, int, int, int]:
+        """parallel_streams, then the many-warp decoder's speculation passes (none for a plan kept from the sizing pass of the
+        same call) and the chunks it resolved"""
+        return tuple(self.L.zipc_b200_ctx_counter(self.h, k) for k in (1, 2, 3, 4))
+
     @staticmethod
     def _ptr_arrays(items: Sequence[np.ndarray]):
         n = len(items)
