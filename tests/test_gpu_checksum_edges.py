@@ -11,8 +11,8 @@ checksum_inputs.py (whose layouts test_checksum_inputs_cpu.py holds to their pla
   4. Past 4 GiB: crc32_dev / adler32_dev, and a stored member whose tiles have 2^32 bytes or more after them, through
      zip_extract_batch_dev and zip_deflate_archive_dev.
 
-Not covered: the wrap of the Adler chain's epoch counter (after 2^32 launches on one context); inflate outputs over 4 GiB
-(minutes on the one-warp decoder)."""
+Not covered: the wrap of the Adler chain's epoch counter (after 2^32 launches on one context).  Inflate outputs over 4 GiB
+are in test_gpu_inflate_past_4gib.py."""
 import ctypes as C
 import zlib
 

@@ -458,7 +458,7 @@ int adler32_ranges(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint6
   return ZIPC_OK;
 }
 
-int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint32_t *nblk, const uint32_t *blk_len,
+int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint32_t *nblk, const uint64_t *blk_len,
                     size_t n, int mode, uint32_t *h_out) {
   // every block is chunked on its own grid (first chunk = block length mod 5552), exactly what Adler_32.string_update
   // does when the reference calls it once per block with the packed state of the previous block
@@ -477,11 +477,11 @@ int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint
   for (size_t i = 0; i < n; i++) {
     uint64_t off = 0;
     for (uint32_t b = 0; b < nblk[i]; b++, nb++) {
-      const uint32_t len = blk_len[nb];
+      const uint64_t len = blk_len[nb];
       if (!len) continue;
-      uint32_t m = len % kChunk;
+      uint32_t m = (uint32_t)(len % kChunk);
       if (m == 0) m = kChunk;
-      for (uint32_t done = 0; done < len; done += m, m = kChunk) { h[k].ptr = d_ptrs[i] + off + done; h[k].len = m; h[k]._pad = 0; k++; }
+      for (uint64_t done = 0; done < len; done += m, m = kChunk) { h[k].ptr = d_ptrs[i] + off + done; h[k].len = m; h[k]._pad = 0; k++; }
       off += len;
     }
   }
@@ -500,12 +500,12 @@ int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint
   for (size_t i = 0; i < n; i++) {
     uint32_t state = 1;
     for (uint32_t b = 0; b < nblk[i]; b++, nb++) {
-      const uint32_t len = blk_len[nb];
+      const uint64_t len = blk_len[nb];
       if (!len) continue;
       uint32_t s1 = state & 0xFFFFu, s2 = state >> 16;  // the state is re-packed between blocks (zipc_deflate.ml:178,198)
-      uint32_t m = len % kChunk;
+      uint32_t m = (uint32_t)(len % kChunk);
       if (m == 0) m = kChunk;
-      for (uint32_t done = 0; done < len; done += m, m = kChunk, k++) adler_fold_step(s1, s2, m, h_ab[k].x, h_ab[k].y, mode);
+      for (uint64_t done = 0; done < len; done += m, m = kChunk, k++) adler_fold_step(s1, s2, m, h_ab[k].x, h_ab[k].y, mode);
       state = (s2 << 16) + s1;
     }
     h_out[i] = state;

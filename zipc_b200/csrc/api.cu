@@ -581,17 +581,25 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
   const uint64_t cb = par_chunk_bytes();
   const uint32_t nch0 = (uint32_t)((src_len + cb - 1) / cb);
   if (nch0 < 4 || src_len > (1ull << 40)) return ZIPC_OK;
-  const size_t tab = (size_t)nch0 * (sizeof(uint64_t) * 4 + sizeof(InflateTask) + sizeof(InflateResult) + kSpecBlocks * sizeof(uint32_t)) + 256;
+  // chunk tables: found starts, tasks, results, then the block lists of the chunks of a pass (reserved once their number is
+  // known and the stream has passed the symbol check below: kSpecBlocks 64-bit lengths per chunk)
+  const size_t tab = (size_t)nch0 * (sizeof(uint64_t) * 4 + sizeof(InflateTask) + sizeof(InflateResult)) + 256;
   if (int st = ctx->d_par.reserve(tab)) return st;
   if (int st = ctx->h_res.reserve(tab)) return st;
-  uint64_t *d_found = ctx->d_par.as<uint64_t>();
-  uint64_t *h_found = ctx->h_res.as<uint64_t>();
-  InflateTask *d_tasks = reinterpret_cast<InflateTask *>(ctx->d_par.as<uint64_t>() + 4 * (size_t)nch0);
-  InflateResult *d_results = reinterpret_cast<InflateResult *>(d_tasks + nch0);
-  InflateResult *h_results = reinterpret_cast<InflateResult *>(ctx->h_res.as<uint64_t>() + 4 * (size_t)nch0);
-  // per chunk: the output lengths of its non-empty blocks (the Adler-32 of a zlib stream is folded block by block)
-  unsigned int *d_blk = reinterpret_cast<unsigned int *>(d_results + nch0);
-  const uint32_t *h_blk = reinterpret_cast<const uint32_t *>(h_results + nch0);
+  uint64_t *d_found, *h_found, *d_blk;
+  InflateTask *d_tasks;
+  InflateResult *d_results, *h_results;
+  const uint64_t *h_blk;   // per chunk: the output lengths of its non-empty blocks (the Adler-32 of a zlib stream is folded block by block)
+  auto layout = [&] {      // (again after every reserve: it does not keep the buffer where it was)
+    d_found = ctx->d_par.as<uint64_t>();
+    h_found = ctx->h_res.as<uint64_t>();
+    d_tasks = reinterpret_cast<InflateTask *>(ctx->d_par.as<uint64_t>() + 4 * (size_t)nch0);
+    d_results = reinterpret_cast<InflateResult *>(d_tasks + nch0);
+    h_results = reinterpret_cast<InflateResult *>(ctx->h_res.as<uint64_t>() + 4 * (size_t)nch0);
+    d_blk = reinterpret_cast<uint64_t *>(d_results + nch0);
+    h_blk = reinterpret_cast<const uint64_t *>(h_results + nch0);
+  };
+  layout();
   // Passes over what is left of the stream.  A pass: (1) block starts, (2) speculative decode of the chunks between them,
   // (3) the chunks must chain up exactly -- each one ends, at a block boundary, on the very bit where the next one was found
   // to start.  A found start that is an accident of the bits inside a block (rare) breaks the chain, and may have hidden the
@@ -632,6 +640,9 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
     } else if (need > spec_cap) {
       return ZIPC_OK;
     }
+    if (int st = ctx->d_par.reserve(tab + (size_t)m * kSpecBlocks * sizeof(uint64_t))) return st;
+    if (int st = ctx->h_res.reserve(tab + (size_t)m * kSpecBlocks * sizeof(uint64_t))) return st;
+    layout();
     std::vector<InflateTask> tasks(m);
     for (uint32_t k = 0; k < m; k++) {
       InflateTask &t = tasks[k];
@@ -643,7 +654,7 @@ static int par_speculate(zipc_b200_ctx *ctx, const uint8_t *d_src, size_t src_le
     ZB_CUDA(ctx, cudaMemcpyAsync(d_tasks, tasks.data(), m * sizeof(InflateTask), cudaMemcpyHostToDevice, ctx->stream));
     if (int st = inflate_launch_spec(ctx, d_tasks, m, d_results, d_blk)) return st;
     ZB_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, m * sizeof(InflateResult), cudaMemcpyDeviceToHost, ctx->stream));
-    ZB_CUDA(ctx, cudaMemcpyAsync(const_cast<uint32_t *>(h_blk), d_blk, (size_t)m * kSpecBlocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    ZB_CUDA(ctx, cudaMemcpyAsync(const_cast<uint64_t *>(h_blk), d_blk, (size_t)m * kSpecBlocks * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
     ZB_CUDA(ctx, stream_sync(ctx, ctx->stream));
     if (par_debug())
       std::fprintf(stderr, "[par] pass %d from bit %llu of %zu bytes: %u nominal chunks, %u block starts: find %.2f ms, speculative decode %.2f ms\n",
@@ -750,8 +761,10 @@ int inflate_core(zipc_b200_ctx *ctx, int ck, int adler_mode, size_t n, const std
             const uint8_t *base = d_dst[i];
             const uint32_t nb = (uint32_t)c->par_plan.blocks.size();
             uint64_t sum = 0;
-            for (uint32_t b : c->par_plan.blocks) sum += b;
-            if (sum != total) ok = false;  // (cannot happen; the one-warp decoder folds it then)
+            for (uint64_t b : c->par_plan.blocks) sum += b;
+            // every byte of an accepted chunk lies in one of its non-empty blocks, whose lengths are 64-bit (one block may
+            // output 4 GiB or more), so the lists add up to the output; if they ever did not, the one-warp decoder folds it
+            if (sum != total) ok = false;
             else if (int st = adler32_blocked(c, &base, &nb, c->par_plan.blocks.data(), 1, adler_mode, &checksum[i])) return st;
           }
         }

@@ -316,7 +316,8 @@ struct zipc_b200_ctx {
     size_t src_len = 0;
     uint64_t epoch = 0;
     std::vector<uint64_t> spec_off, len;
-    std::vector<uint32_t> blocks;      // output lengths of the stream's non-empty deflate blocks, in order (Adler-32 is folded per block)
+    std::vector<uint64_t> blocks;      // output lengths of the stream's non-empty deflate blocks, in order (Adler-32 is folded per block;
+                                       // one block may output 4 GiB or more)
     uint64_t total = 0;
   } par_plan;
   uint64_t epoch = 1;
@@ -384,7 +385,7 @@ int adler32_ranges(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint6
 // Adler-32 of n inputs, each folded block by block as the reference does on both codec sides (state re-packed and the
 // 5552-byte chunk grid restarted at every block, :682-690, :1081-1086): member i consists of nblk[i] consecutive
 // blocks whose lengths follow each other in blk_len
-int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint32_t *nblk, const uint32_t *blk_len,
+int adler32_blocked(zipc_b200_ctx *ctx, const uint8_t *const *d_ptrs, const uint32_t *nblk, const uint64_t *blk_len,
                     size_t n, int mode, uint32_t *h_out);
 // deflate.cu
 // d_blk_lens (may be null): receives the source length of every deflate block of member i at
@@ -505,9 +506,10 @@ int inflate_launch(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, I
 int inflate_find_starts(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t src_len, uint64_t first_bit, uint64_t chunk_bytes,
                         uint32_t nchunks, uint64_t *d_found);
 // 2. speculative decode of the chunks (tasks carry start_bit / stop_bit, dst = 16-bit symbols)
-// d_block_lists (may be null): kSpecBlocks entries per task, the output lengths of the non-empty blocks of every chunk (for Adler-32)
+// d_block_lists (may be null): kSpecBlocks entries per task, the output lengths of the non-empty blocks of every chunk (for Adler-32;
+// 64 bits, as one block may output 4 GiB or more)
 constexpr uint32_t kSpecBlocks = 256;
-int inflate_launch_spec(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, InflateResult *d_results, unsigned int *d_block_lists = nullptr);
+int inflate_launch_spec(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, InflateResult *d_results, uint64_t *d_block_lists = nullptr);
 // 3. resolve: windows chunk by chunk, then every symbol to its byte.  d_spec_off / d_out_off / d_len: per chunk (device).
 //    d_windows: 4 * 32768 bytes per chunk of scratch.  *d_bad is set if anything refers to bytes before the stream
 int inflate_resolve(zipc_b200_ctx *ctx, const uint16_t *d_spec, const uint64_t *d_spec_off, const uint64_t *d_out_off,

@@ -537,10 +537,12 @@ __global__ void __launch_bounds__(THREADS, 1)
 inflate_kernel(const InflateTask *__restrict__ tasks, uint32_t ntasks, InflateResult *__restrict__ results,
                unsigned int *__restrict__ queue, uint16_t *__restrict__ g_syms, int adler_mode,
                unsigned int *__restrict__ group_count, uint32_t *__restrict__ group_flag,
-               const uint32_t *__restrict__ upload_flag, uint32_t upload_serial) {
+               const uint32_t *__restrict__ upload_flag, uint32_t upload_serial, uint64_t *__restrict__ block_lens) {
   // adler_mode: -1 = no checksum in this kernel, else ZIPC_ADLER_* (fused per-block Adler-32 of the output)
   // group_count / group_flag (may be null): streams left in each download group; the warp that finishes a group's last
   // stream raises the group's flag (mapped host memory), and the host starts copying that range of the arena
+  // block_lens (SPEC, may be null): kSpecBlocks entries per task, the output lengths of the chunk's non-empty blocks (64 bits:
+  // one block may output 4 GiB or more)
   // upload_flag / upload_serial: a stream whose flags name part p >= 1 of a split upload is opened only once *upload_flag has
   // reached upload_serial + p (its bytes travel on another stream while this kernel already works on the first part)
   extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -952,13 +954,13 @@ inflate_kernel(const InflateTask *__restrict__ tasks, uint32_t ntasks, InflateRe
     // Adler-32 restarts its 5552-byte chunk grid at every block and, as written in the reference, reduces
     // with a signed remainder, so it has to be folded block by block to stay bit-exact.
     if (ad_pending) {
-      if (SPEC && group_count) {
-        // speculative chunk: the output length of every non-empty block goes to the chunk's list (group_count is that array in
-        // this mode, kSpecBlocks entries per task): the host folds the Adler-32 of a large zlib stream over these blocks
+      if (SPEC && block_lens) {
+        // speculative chunk: the output length of every non-empty block goes to the chunk's list: the host folds the Adler-32
+        // of a large zlib stream over these blocks
         if (lane == 0) {
           const uint64_t blen = out_pos - st.ad_from;
           if (blen) {
-            if (st.nblk < kSpecBlocks) group_count[(size_t)task * kSpecBlocks + st.nblk] = (unsigned int)blen;
+            if (st.nblk < kSpecBlocks) block_lens[(size_t)task * kSpecBlocks + st.nblk] = blen;
             st.nblk++;
             st.ad_from = out_pos;
           }
@@ -986,7 +988,7 @@ inflate_kernel(const InflateTask *__restrict__ tasks, uint32_t ntasks, InflateRe
         r.end_bit = in.consumed(wk);
         r.final_seen = final_blk ? 1u : 0u;
         r._pad2 = SPEC ? st.nblk : 0u;              // (speculative chunks) non-empty blocks decoded: their lengths are in the chunk's list
-        if (SPEC && group_count && st.nblk > kSpecBlocks && status == ZIPC_OK) { r.status = ZIPC_ERR_DST_TOO_SMALL; r.out_len = 0; }  // list full: not this way
+        if (SPEC && block_lens && st.nblk > kSpecBlocks && status == ZIPC_OK) { r.status = ZIPC_ERR_DST_TOO_SMALL; r.out_len = 0; }  // list full: not this way
         results[task] = r;
       }
       if (!COUNT_ONLY && !SPEC && group_count) {
@@ -1172,10 +1174,10 @@ int inflate_launch(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, I
   }
   KernelTimer kt(ctx);
   if (count_only)
-    inflate_kernel<true, false><<<grid, THREADS, kSmemBytes, ctx->stream>>>(d_tasks, n, d_results, queue, ctx->d_scratch.as<uint16_t>(), -1, nullptr, nullptr, nullptr, 0);
+    inflate_kernel<true, false><<<grid, THREADS, kSmemBytes, ctx->stream>>>(d_tasks, n, d_results, queue, ctx->d_scratch.as<uint16_t>(), -1, nullptr, nullptr, nullptr, 0, nullptr);
   else
     inflate_kernel<false, false><<<grid, THREADS, kSmemBytes, ctx->stream>>>(d_tasks, n, d_results, queue, ctx->d_scratch.as<uint16_t>(), adler_mode,
-                                                                            d_group_count, group_flag, d_upflag, upload_serial);
+                                                                            d_group_count, group_flag, d_upflag, upload_serial, nullptr);
   ctx->launches++;
   ZB_CUDA(ctx, cudaGetLastError());
   return ZIPC_OK;
@@ -1202,7 +1204,7 @@ int inflate_find_starts(zipc_b200_ctx *ctx, const uint8_t *d_src, uint64_t src_l
   return ZIPC_OK;
 }
 
-int inflate_launch_spec(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, InflateResult *d_results, unsigned int *d_block_lists) {
+int inflate_launch_spec(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t n, InflateResult *d_results, uint64_t *d_block_lists) {
   if (n == 0) return ZIPC_OK;
   // Spread the chunks: a chunk is one block of the stream on one warp, and the call waits for the slowest of them -- a warp with
   // few neighbours on its SM decodes nearly twice as fast as one of 32 (35 against 16-20 MB/s).  About four chunks per CTA, over
@@ -1216,7 +1218,7 @@ int inflate_launch_spec(zipc_b200_ctx *ctx, const InflateTask *d_tasks, uint32_t
   unsigned int start = grid * WARPS;  // tasks [0, start) are assigned statically
   ZB_CUDA(ctx, cudaMemcpyAsync(queue, &start, sizeof start, cudaMemcpyHostToDevice, ctx->stream));
   KernelTimer kt(ctx);
-  inflate_kernel<false, true><<<grid, THREADS, kSmemBytes, ctx->stream>>>(d_tasks, n, d_results, queue, ctx->d_scratch.as<uint16_t>(), -1, d_block_lists, nullptr, nullptr, 0);
+  inflate_kernel<false, true><<<grid, THREADS, kSmemBytes, ctx->stream>>>(d_tasks, n, d_results, queue, ctx->d_scratch.as<uint16_t>(), -1, nullptr, nullptr, nullptr, 0, d_block_lists);
   ctx->launches++;
   ZB_CUDA(ctx, cudaGetLastError());
   return ZIPC_OK;

@@ -141,7 +141,7 @@ int deflate_run(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n,
                 const std::vector<const uint8_t *> &d_src, const size_t *src_len,
                 const std::vector<uint8_t *> &d_slot, const std::vector<size_t> &slot_cap,
                 size_t *out_len, uint32_t *checksum, int *status, const std::vector<uint32_t> *flags = nullptr,
-                std::vector<uint32_t> *blocks_out = nullptr, std::vector<uint32_t> *nblocks_out = nullptr) {
+                std::vector<uint64_t> *blocks_out = nullptr, std::vector<uint32_t> *nblocks_out = nullptr) {
   // blocks_out / nblocks_out (Adler-32 at a compressing level only): the source lengths of the blocks every input was emitted
   // as, input after input, and their number per input, INSTEAD of the checksums -- the caller folds them itself (the pieces of a
   // split member are folded as the one stream they form)
@@ -229,14 +229,14 @@ int deflate_run(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_t n,
       for (size_t i = 0; i < n; i++) checksum[i] = hck[i] ^ 0xFFFFFFFFu;
     } else if (ck == ZIPC_CK_ADLER32) {
       // block lists per member, in member order
-      std::vector<uint32_t> lens;
+      std::vector<uint64_t> lens;
       if (blocks_from_kernel) {
         for (size_t i = 0; i < n; i++) lens.insert(lens.end(), h_blk.begin() + blk_off[i], h_blk.begin() + blk_off[i] + nblk[i]);
         if (blocks_out && nblocks_out) { *blocks_out = std::move(lens); *nblocks_out = nblk; return ZIPC_OK; }
       } else {  // level `None: stored blocks of kStoredBlock source bytes (reference :1106-1116)
         for (size_t i = 0; i < n; i++) {
           nblk[i] = 0;
-          for (uint64_t o = 0; o < src_len[i]; o += kStoredBlock, nblk[i]++) lens.push_back((uint32_t)std::min<uint64_t>(kStoredBlock, src_len[i] - o));
+          for (uint64_t o = 0; o < src_len[i]; o += kStoredBlock, nblk[i]++) lens.push_back(std::min<uint64_t>(kStoredBlock, src_len[i] - o));
         }
       }
       if (int st = adler32_blocked(ctx, d_src.data(), nblk.data(), lens.data(), n, adler_mode, checksum)) return st;
@@ -334,7 +334,8 @@ int deflate_members(zipc_b200_ctx *ctx, int level, int ck, int adler_mode, size_
   // reference's zlib_decompress recomputes from the concatenated stream (the empty stored blocks between the pieces fold
   // nothing; zipc_deflate.ml:682-690, 1081-1086)
   const bool fold_here = any_split && checksum && ck == ZIPC_CK_ADLER32;
-  std::vector<uint32_t> blk, nblk;
+  std::vector<uint64_t> blk;
+  std::vector<uint32_t> nblk;
   if (int st = deflate_run(ctx, level, ck, adler_mode, m, e_src, e_len.data(), pc.d_slot, cap, e_out.data(), checksum ? e_ck.data() : nullptr,
                            e_st.data(), any_split ? &e_flags : nullptr, fold_here ? &blk : nullptr, fold_here ? &nblk : nullptr)) return st;
   pc.len = e_out;
